@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (own arm, B200 kernels)
     python bench.py --impl reference --gpus N ...            (reference arm: CPU port)
+    python bench.py ... --dump-outputs DIR                   (+ the last timed step's outputs as DIR/*.npy)
 
 Workload (BASELINE.json configs[1], "cfg2_sh"): TensoRF-VM 300^3 grid, density 3x16 /
 appearance 3x48 components, app_dim 27, SH shading, 4096-ray batch, S=1000 samples per
@@ -75,7 +76,16 @@ def parse():
     ap.add_argument("--render-chunk", type=int, default=16384, help="rays per forward call of the full-frame render")
     ap.add_argument("--head", default="auto", choices=["auto", "tc", "fp32"],
                     help="shading head: tcgen05 tensor-core kernels (auto/tc) or strict-fp32 SIMT GEMMs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed training step computed (rgb, depth, acc, "
+                         "loss and every gradient, rank 0) as DIR/<name>.npy; arrays over 2^21 elements are replaced by "
+                         "a fixed seeded sample of that many elements (<name>.sample.npy). Same arguments, same inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.mode != "train"):
+        ap.error("--dump-outputs writes the outputs of the training step of --impl b200 --mode train")
+    return a
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -451,6 +461,28 @@ def gemm_flops(name, A, F, ctot, in_dim, H):
     return table.get(name)
 
 
+DUMP_MAX_ELEMS = 1 << 21          # per array: 8 MB of float32
+DUMP_MAX_BYTES = 64 << 20         # per dump
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of `arrays` as out_dir/<name>.npy (float64 stays float64, anything else becomes float32). A
+    tensor of more than DUMP_MAX_ELEMS elements is written as <name>.sample.npy instead: its elements at
+    DUMP_MAX_ELEMS flat indices drawn from a generator seeded with 0, in increasing order -- the same indices for
+    every run and every build, so two dumps compare element for element."""
+    import numpy as np
+    arrays = {k: (v.detach() if v.dtype == torch.float64 else v.detach().float()) for k, v in arrays.items()}
+    size = sum(min(v.numel(), DUMP_MAX_ELEMS) * v.element_size() for v in arrays.values())
+    if size > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {size} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        if v.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            v, name = v.reshape(-1)[idx.to(v.device)], name + ".sample"
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy())
+
+
 def own_arm(args):
     import torch.distributed as dist
 
@@ -524,6 +556,7 @@ def own_arm(args):
                                         split21={"auto": "auto", "on": True, "off": False}[args.sync_split21])
             .attach(model, [se3_refine]) if world > 1 else None)
     inv_world = 1.0 / world
+    last_out = {}              # --dump-outputs: the latest step's forward outputs (static tensors under --cuda-graph)
 
     def make_step(model, opt, params):
         def step(pix, tgt, reduce=True):
@@ -537,6 +570,8 @@ def own_arm(args):
             (loss * inv_world if world > 1 else loss).backward()
             if sync is not None and reduce:
                 sync.finish([se3_refine])
+            if args.dump_outputs:
+                last_out.update(rgb=rgb.detach(), depth=depth.detach(), acc=acc.detach(), loss=loss.detach())
             return loss
         return step
 
@@ -627,6 +662,9 @@ def own_arm(args):
             launches = launches_per_graph * args.steps               # replayed, not re-issued: count what the graph holds
         ms_e2e = timed(step_e2e, args.steps, align=True)
         barrier()
+    if args.dump_outputs and rank == 0:
+        grads = {f"grad.{k}": p.grad for k, p in model.named_parameters() if p.grad is not None}
+        dump_outputs(args.dump_outputs, {**last_out, **grads, "grad.se3_refine": se3_refine.grad})
     t = torch.tensor([ms, ms_e2e], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
