@@ -46,7 +46,7 @@ typedef struct CUstream_st* cudaStream_t;
 
 /* ---- library ----------------------------------------------------------- */
 const char* jt_strerror(int code);
-int jt_version(void);            /* ABI version, bumped on any signature change */
+int jt_version(void);            /* ABI version, bumped on any signature or argument-semantics change (3: NULL gradients) */
 /* number of kernel launches issued through this library since load (for bench.py) */
 long long jt_launch_count(void);
 
@@ -109,7 +109,9 @@ int jt_vm_gather_bwd(int app, const void* const* h_factors, void* const* h_facto
  * kernel running on a second stream; 0 = fill the machine.
  * plane_mask: bit i = walk plane / line pair i in this launch (7 = all three in one launch). The data-parallel
  * backward launches the appearance planes one by one so that each plane's gradients can be all-reduced while the
- * next plane is still being walked. */
+ * next plane is still being walked.
+ * h_factor_grads = NULL (since version 3): coordinate-only walk for a frozen field -- only d_o / d_d are accumulated,
+ * no factor gradient is written; every other argument keeps its meaning. */
 int jt_vm_scatter_rays(int app, const void* const* h_factors, void* const* h_factor_grads, const int* h_dims,
                        const float* samp, const int* slot, const int* sidx, const int* n_dev, int n_max,
                        const void* gin, int gin_bf16, int n_samples, const float* h_inv, float* d_o, float* d_d,
@@ -185,7 +187,9 @@ int jt_head_mlp_fwd_tc(int split, const float* featdir, const float* W1, const f
  * [A][4] (gradient at the head's pre-activation, from jt_render_bwd), feat [A][ldf] and the
  * tiles the forward left in `stage`, computes dcomps [A][144] (for jt_vm_gather_bwd) and ADDS
  * the weight gradients into gWb [27][144], gW1 [64][150], gb1, gW2 [64][64], gb2, gW3 [3][64],
- * gb3. relu masks are the forward's own; nothing is recomputed. */
+ * gb3. relu masks are the forward's own; nothing is recomputed.
+ * All seven weight-gradient pointers NULL (since version 3; frozen head and basis_mat): dcomps alone, bit-identical
+ * to the full call; `stage` is still read (relu masks). A mix of NULL and non-NULL pointers returns JT_ERR_ARG. */
 int jt_head_bwd_tc(const float* dout, const float* feat, int ldf, const float* Wb, const float* W1, const float* W2,
                    const float* W3, const int* n_dev, int n_max, float fea_progress, void* dcomps, int dcomps_bf16, void* stage,
                    float* gWb, float* gW1, float* gb1, float* gW2, float* gb2, float* gW3, float* gb3,
@@ -197,7 +201,9 @@ int jt_head_bwd_tc(const float* dout, const float* feat, int ldf, const float* W
  * featdir [A][32] only receives the view direction (floats 28..30) for the backward.
  * jt_sh_bwd_tc = backward of basis_mat + SHRender: dout [A][4] (gradient at the pre-activation,
  * jt_render_bwd with shade_act 2) -> DF = dout (x) Y (bf16) -> dcomps [A][144] = DF * Wb on
- * tcgen05; ADDS d basis_mat into gWb [27][144] from the component tiles the forward staged. */
+ * tcgen05; ADDS d basis_mat into gWb [27][144] from the component tiles the forward staged.
+ * gWb = NULL (since version 3; frozen basis_mat): dcomps alone, bit-identical to the full call, and `stage` may be
+ * NULL (a forward that staged nothing). */
 int jt_app_basis_sh_fwd_tc(int split, const void* const* h_factors, const int* h_dims, const float* samp,
                            const int* aidx, const int* sidx, const float* rays_d, int n_samples, int normalize_dir,
                            const float* Wb, const int* n_dev, int n_max, float* featdir, float* rgb, void* stage,
@@ -370,7 +376,9 @@ int jt_wv_head_fwd_tc(const float* comps, const int* aidx, const int* sidx, cons
 /* Autograd of the above (bf16-operand GEMMs, fp32 accumulation in TMEM). dout [n][4] = dL/d(pre-sigmoid) as
  * jt_render_bwd writes it; dcomps [n][60] fp32 = gradient w.r.t. the gathered components (input of
  * jt_vm_scatter_rays); the weight gradients are ACCUMULATED into gWb [20][60], gW1 [32][100], gb1 [32],
- * gW2 [32][32], gb2 [32], gW3 [3][44], gb3 [3] (zero-initialised by the caller). */
+ * gW2 [32][32], gb2 [32], gW3 [3][44], gb3 [3] (zero-initialised by the caller).
+ * All seven weight-gradient pointers NULL (since version 3): dcomps alone, bit-identical to the full call; a mix of
+ * NULL and non-NULL pointers returns JT_ERR_ARG. */
 int jt_wv_head_bwd_tc(const float* dout, const float* featdir, const float* Wb, const float* W1, const float* W2,
                       const float* W3, const int* n_dev, int n_max, float fea_progress, float* dcomps, void* stage,
                       float* gWb, float* gW1, float* gb1, float* gW2, float* gb2, float* gW3, float* gb3,

@@ -17,7 +17,9 @@
 //     and writes dcomps (fp32) for the VM scatter kernel. The bf16 operand tiles it
 //     builds on the way (D2, D1, DF, DO = dout) are pushed next to the forward's tiles
 //     (A0 comps, A1 encoded input, A2, A3) in the HBM staging area with bulk async
-//     stores (TMA engine), already in the UMMA canonical layout.
+//     stores (TMA engine), already in the UMMA canonical layout. Only the wgrad kernel
+//     reads them: without weight gradients (WST = false, a frozen head) they stay in
+//     shared memory, and dcomps comes out of the same arithmetic bit for bit.
 //
 //  head_bwd_wgrad_kernel (persistent, one CTA per SM)
 //     a TMA -> tcgen05 pipeline over those staged tiles: weight gradients are
@@ -53,7 +55,7 @@ __device__ __forceinline__ uint32_t chunk_mask(const uint4 q) {
 
 constexpr int NTB = 2 * TM;     // two threads per sample row (column halves), as in the forward kernel
 
-template <bool DC16>
+template <bool DC16, bool WST>
 __global__ void __launch_bounds__(NTB, 2) head_bwd_data_kernel(
     const float* __restrict__ dout, const float* __restrict__ feat_in, int ldf, const float* __restrict__ Wb,
     const float* __restrict__ W1, const float* __restrict__ W2, const float* __restrict__ W3,
@@ -124,7 +126,7 @@ __global__ void __launch_bounds__(NTB, 2) head_bwd_data_kernel(
         const bool live = row < n;
         unsigned char* st = stage + (size_t)tile * STAGE_TILE_BYTES;
         // ---- S0: dh2 = (dout W3) . [h2 > 0] -> D2 (this thread: columns [32 hh, 32 hh + 32)) ; dout -> DO
-        if (hh == 0) {
+        if (WST && hh == 0) {
             const float v[8] = {go[0], go[1], go[2], 0.f, 0.f, 0.f, 0.f, 0.f};
             store_chunk(DO, nullptr, TM, 0, r, v);
         }
@@ -147,9 +149,11 @@ __global__ void __launch_bounds__(NTB, 2) head_bwd_data_kernel(
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem + T_DH1, D2, nullptr, w2t, nullptr, H_, H_, H_);
             mma_commit(&bar);
-            bulk_s2g(st + OFF_D2, D2, SZ_D2);
-            bulk_s2g(st + OFF_DO, DO, SZ_DO);
-            bulk_commit();
+            if (WST) {
+                bulk_s2g(st + OFF_D2, D2, SZ_D2);
+                bulk_s2g(st + OFF_DO, DO, SZ_DO);
+                bulk_commit();
+            }
         }
         mbar_wait(&bar, phase); phase ^= 1;
         tc_fence_after();
@@ -174,8 +178,10 @@ __global__ void __launch_bounds__(NTB, 2) head_bwd_data_kernel(
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem + T_DIN, D1, nullptr, w1t, nullptr, H_, K1, K1);
             mma_commit(&bar);
-            bulk_s2g(st + OFF_D1, D1, SZ_D1);
-            bulk_commit();
+            if (WST) {
+                bulk_s2g(st + OFF_D1, D1, SZ_D1);
+                bulk_commit();
+            }
         }
         mbar_wait(&bar, phase); phase ^= 1;
         tc_fence_after();
@@ -211,18 +217,20 @@ __global__ void __launch_bounds__(NTB, 2) head_bwd_data_kernel(
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem + T_DC, DF, nullptr, wbt, nullptr, NB, CT, CT);
             mma_commit(&bar);
-            bulk_s2g(st + OFF_DF, DF, SZ_DF);
-            bulk_commit();
+            if (WST) {
+                bulk_s2g(st + OFF_DF, DF, SZ_DF);
+                bulk_commit();
+            }
         }
         mbar_wait(&bar, phase); phase ^= 1;
         tc_fence_after();
         // ---- S3: dcomps row -> global (fp32, or bf16 when DC16)
         store_dcomps_row<DC16>(lane_addr + T_DC, hh, live, row, dcomps_out);
-        if (tid == 0) bulk_wait_read0();       // D2 / D1 / DF / DO have left shared memory
+        if (WST && tid == 0) bulk_wait_read0();       // D2 / D1 / DF / DO have left shared memory
         tc_fence_before();
         __syncthreads();
     }
-    if (tid == 0) bulk_wait0();
+    if (WST && tid == 0) bulk_wait0();
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem, 256);
@@ -353,6 +361,7 @@ __global__ void __launch_bounds__(TM) head_bwd_wgrad_kernel(const unsigned char*
 //     DF[128x32] (bf16) = dpre (x) Y     ->  MMA  dcomps[128x144] = DF * Wb   (TMEM)  -> bf16 rows
 // DF is pushed to the staging area next to the forward's component tile A0, and the
 // basis_mat weight gradient is group 3 of the shared TMA -> tcgen05 wgrad pipeline.
+// WST = false (frozen basis_mat): no staging area, DF stays in shared memory.
 struct ShBwdSmem {
     static constexpr int WBT = tile_bytes(CT, NB);
     static constexpr int OUT = TM * CT * 2;                     // dcomps tile, bf16 row-major = its global image
@@ -361,13 +370,12 @@ struct ShBwdSmem {
     static constexpr int total = off_out + 2 * OUT;
 };
 
-__device__ __forceinline__ void bulk_wait_read_2() { asm volatile("cp.async.bulk.wait_group.read 2;" ::: "memory"); }
-
 // dcomps leaves the SM as ONE bulk async store per tile: the 128 rows x 288 B of a tile are contiguous in
 // global memory, the threads only write their TMEM columns into a shared-memory image of it (per-thread
 // 16-byte global stores at a 288-byte row pitch kept the LSU queues full: lg_throttle, 0.33 ms). DF and
 // the output tile are double-buffered; the issuing thread waits for the bulk stores of two tiles ago
 // *before* it signals the MMA barrier, so passing that barrier also means both buffers are free.
+template <bool WST>
 __global__ void __launch_bounds__(NTB, 2) sh_bwd_data_kernel(const float* __restrict__ dout, const float* __restrict__ featdir,
                                                              int ldf, const float* __restrict__ Wb,
                                                              const int* __restrict__ n_dev, int n_fixed,
@@ -407,7 +415,6 @@ __global__ void __launch_bounds__(NTB, 2) sh_bwd_data_kernel(const float* __rest
 
     for (int tile = blockIdx.x; (long long)tile * TM < n; tile += gridDim.x, buf ^= 1) {
         const int rows = min(TM, n - tile * TM);
-        unsigned char* st = stage + (size_t)tile * STAGE_TILE_BYTES;
         unsigned char* DF = smem + L::off_df + buf * SZ_DF;
         unsigned char* OUT = smem + L::off_out + buf * L::OUT;
         // ---- DF row: columns c*9+k = dpre[c] * Y_k, 27..31 = 0; this thread: columns [16 hh, 16 hh + 16)
@@ -434,11 +441,15 @@ __global__ void __launch_bounds__(NTB, 2) sh_bwd_data_kernel(const float* __rest
         if (tid == 0) {
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem, DF, nullptr, wbt, nullptr, NB, CT, CT);
-            bulk_s2g(st + OFF_DF, DF, SZ_DF);
-            bulk_commit();
-            // pending afterwards: at most OUT(t-1) and DF(t) -> DF(t-1) and OUT(t-2), the previous users of the
-            // buffers this tile's successor / this tile's epilogue write, have been read out of shared memory
-            bulk_wait_read_2();
+            if (WST) {
+                bulk_s2g(stage + (size_t)tile * STAGE_TILE_BYTES + OFF_DF, DF, SZ_DF);
+                bulk_commit();
+                // pending afterwards: at most OUT(t-1) and DF(t) -> DF(t-1) and OUT(t-2), the previous users of the
+                // buffers this tile's successor / this tile's epilogue write, have been read out of shared memory
+                bulk_wait_read2();
+            } else {
+                bulk_wait_read1();             // only OUT(t-1) may still be pending: OUT(t-2) has been read
+            }
             mma_commit(&bar);
         }
         mbar_wait(&bar, phase); phase ^= 1;
@@ -492,42 +503,56 @@ extern "C" int jt_head_bwd_tc(const float* dout, const float* feat, int ldf, con
                               int dcomps_bf16, void* stage, float* gWb, float* gW1, float* gb1, float* gW2, float* gb2, float* gW3,
                               float* gb3, cudaStream_t stream) {
     JT_CHECK_ARG(dout && feat && Wb && W1 && W2 && W3 && dcomps && stage && ldf >= 28 && ldf % 4 == 0);
-    JT_CHECK_ARG(gWb && gW1 && gb1 && gW2 && gb2 && gW3 && gb3);
+    const int n_wg = !!gWb + !!gW1 + !!gb1 + !!gW2 + !!gb2 + !!gW3 + !!gb3;
+    JT_CHECK_ARG(n_wg == 0 || n_wg == 7);                // all weight gradients, or none (frozen head + basis_mat)
     JT_CHECK_ARG((reinterpret_cast<uintptr_t>(stage) & 127) == 0);
     if (n_max <= 0) return JT_OK;
+    const bool wg = n_wg == 7;
     long long tiles = ((long long)n_max + TM - 1) / TM;
     int grid_d = (int)(tiles < 2 * kNumSMs ? tiles : 2 * kNumSMs);
     int grid_w = (int)(tiles < kNumSMs ? tiles : kNumSMs);
-    if (int rc = set_smem(head_bwd_data_kernel<false>, BwdSmem::total)) return rc;
-    if (int rc = set_smem(head_bwd_data_kernel<true>, BwdSmem::total)) return rc;
-    if (int rc = set_smem(head_bwd_wgrad_kernel<0, 4, WG_STAGES, WG_STAGE_BYTES>, WG_STAGES * WG_STAGE_BYTES)) return rc;
-    g_launches += 2;
-    if (dcomps_bf16)
-        head_bwd_data_kernel<true><<<grid_d, NTB, BwdSmem::total, stream>>>(dout, feat, ldf, Wb, W1, W2, W3, n_dev, n_max,
-                                                                           fea_progress, dcomps, static_cast<unsigned char*>(stage));
-    else
-        head_bwd_data_kernel<false><<<grid_d, NTB, BwdSmem::total, stream>>>(dout, feat, ldf, Wb, W1, W2, W3, n_dev, n_max,
-                                                                            fea_progress, dcomps, static_cast<unsigned char*>(stage));
-    head_bwd_wgrad_kernel<0, 4, WG_STAGES, WG_STAGE_BYTES><<<grid_w, TM, WG_STAGES * WG_STAGE_BYTES, stream>>>(
-        static_cast<const unsigned char*>(stage), n_dev, n_max, gWb, gW1, gb1, gW2, gb2, gW3, gb3);
+    unsigned char* st = static_cast<unsigned char*>(stage);
+#define JT_HBD(DC, WS)                                                                                              \
+    {                                                                                                               \
+        if (int rc = set_smem(head_bwd_data_kernel<DC, WS>, BwdSmem::total)) return rc;                             \
+        head_bwd_data_kernel<DC, WS><<<grid_d, NTB, BwdSmem::total, stream>>>(dout, feat, ldf, Wb, W1, W2, W3, n_dev, \
+                                                                            n_max, fea_progress, dcomps, st);       \
+    }
+    if (dcomps_bf16) { if (wg) JT_HBD(true, true) else JT_HBD(true, false) }
+    else { if (wg) JT_HBD(false, true) else JT_HBD(false, false) }
+#undef JT_HBD
+    g_launches += 1;
+    if (wg) {
+        if (int rc = set_smem(head_bwd_wgrad_kernel<0, 4, WG_STAGES, WG_STAGE_BYTES>, WG_STAGES * WG_STAGE_BYTES)) return rc;
+        g_launches += 1;
+        head_bwd_wgrad_kernel<0, 4, WG_STAGES, WG_STAGE_BYTES><<<grid_w, TM, WG_STAGES * WG_STAGE_BYTES, stream>>>(
+            st, n_dev, n_max, gWb, gW1, gb1, gW2, gb2, gW3, gb3);
+    }
     JT_RETURN_LAUNCH();
 }
 
 extern "C" int jt_sh_bwd_tc(const float* dout, const float* featdir, int ldf, const float* Wb, const int* n_dev,
                             int n_max, void* dcomps, int dcomps_bf16, void* stage, float* gWb, cudaStream_t stream) {
-    JT_CHECK_ARG(dout && featdir && Wb && dcomps && stage && gWb && ldf >= 32 && ldf % 4 == 0);
+    // gWb = NULL (frozen basis_mat): no weight gradient, and `stage` may be NULL (a forward without staging)
+    JT_CHECK_ARG(dout && featdir && Wb && dcomps && (stage || !gWb) && ldf >= 32 && ldf % 4 == 0);
     JT_CHECK_ARG(dcomps_bf16 == 1);                     // dcomps rows are bf16 [A][144] (what jt_vm_scatter_rays reads)
     JT_CHECK_ARG((reinterpret_cast<uintptr_t>(stage) & 127) == 0 && (reinterpret_cast<uintptr_t>(dcomps) & 15) == 0);
     if (n_max <= 0) return JT_OK;
     long long tiles = ((long long)n_max + TM - 1) / TM;
     int grid_d = (int)(tiles < 2 * kNumSMs ? tiles : 2 * kNumSMs);
     int grid_w = (int)(tiles < kNumSMs ? tiles : kNumSMs);
-    if (int rc = set_smem(sh_bwd_data_kernel, ShBwdSmem::total)) return rc;
-    if (int rc = set_smem(head_bwd_wgrad_kernel<3, 1, WG_SH_STAGES, WG_SH_STAGE_BYTES>, WG_SH_STAGES * WG_SH_STAGE_BYTES)) return rc;
-    g_launches += 2;
     unsigned char* st = static_cast<unsigned char*>(stage);
-    sh_bwd_data_kernel<<<grid_d, NTB, ShBwdSmem::total, stream>>>(dout, featdir, ldf, Wb, n_dev, n_max,
-                                                                 static_cast<unsigned short*>(dcomps), st);
+    unsigned short* dc = static_cast<unsigned short*>(dcomps);
+    g_launches += 1;
+    if (!gWb) {
+        if (int rc = set_smem(sh_bwd_data_kernel<false>, ShBwdSmem::total)) return rc;
+        sh_bwd_data_kernel<false><<<grid_d, NTB, ShBwdSmem::total, stream>>>(dout, featdir, ldf, Wb, n_dev, n_max, dc, nullptr);
+        JT_RETURN_LAUNCH();
+    }
+    if (int rc = set_smem(sh_bwd_data_kernel<true>, ShBwdSmem::total)) return rc;
+    if (int rc = set_smem(head_bwd_wgrad_kernel<3, 1, WG_SH_STAGES, WG_SH_STAGE_BYTES>, WG_SH_STAGES * WG_SH_STAGE_BYTES)) return rc;
+    g_launches += 1;
+    sh_bwd_data_kernel<true><<<grid_d, NTB, ShBwdSmem::total, stream>>>(dout, featdir, ldf, Wb, n_dev, n_max, dc, st);
     head_bwd_wgrad_kernel<3, 1, WG_SH_STAGES, WG_SH_STAGE_BYTES><<<grid_w, TM, WG_SH_STAGES * WG_SH_STAGE_BYTES, stream>>>(
         st, n_dev, n_max, gWb, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
     JT_RETURN_LAUNCH();

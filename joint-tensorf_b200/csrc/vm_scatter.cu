@@ -112,7 +112,10 @@ struct StepPos {          // tap position of one sample on one plane/line pair
 
 // B16: the factor taps are bf16 (8-byte quads: half the staging traffic), everything else is unchanged -- the
 // gradients and the arithmetic stay fp32.
-template <bool APP, int NQ, int I, bool GB16, bool B16, int THR = SC_THREADS>
+// FG = false: coordinate-only walk for a frozen field (test-time pose optimisation). The corner / line gradient
+// accumulators, the cell bookkeeping of their flushes and every RED into the factor gradients are compiled out; the
+// tap staging, the look-ahead and the per-ray sums (all the pose gradient needs) are the same code as with FG.
+template <bool APP, int NQ, int I, bool GB16, bool B16, bool FG, int THR = SC_THREADS>
 __device__ __forceinline__ void walk_plane(const ScatterArgs& A, const int e0, const int e1, const int q, const int qs,
                                            int& ray, int& ray_end, RaySums& rs,
                                            typename std::conditional<B16, uint2, float4>::type* __restrict__ sm) {
@@ -124,8 +127,8 @@ __device__ __forceinline__ void walk_plane(const ScatterArgs& A, const int e0, c
     if (q >= C) return;
     const ElemT* __restrict__ P = reinterpret_cast<const ElemT*>(F.plane[I]) + q;
     const ElemT* __restrict__ Ln = reinterpret_cast<const ElemT*>(F.line[I]) + q;
-    float* __restrict__ GP = A.G.plane[I] + q;
-    float* __restrict__ GL = A.G.line[I] + q;
+    float* __restrict__ GP = FG ? A.G.plane[I] + q : nullptr;
+    float* __restrict__ GL = FG ? A.G.line[I] + q : nullptr;
     const float sclx = 0.5f * (float)(W - 1), scly = 0.5f * (float)(H - 1), scll = 0.5f * (float)(L - 1);
     // this lane's staging slots (float4 index = slot * SC_THREADS): plane buffer b, tap c, quad k -> (b*4 + c)*NQ + k;
     // line buffer b, tap c, quad k -> 8 NQ + (b*2 + c)*NQ + k
@@ -278,7 +281,7 @@ __device__ __forceinline__ void walk_plane(const ScatterArgs& A, const int e0, c
         const float mx0 = (x0 >= 0 && x0 < W) ? 1.f : 0.f, mx1 = (x0 + 1 >= 0 && x0 + 1 < W) ? 1.f : 0.f;
         const float my0 = (y0 >= 0 && y0 < H) ? 1.f : 0.f, my1 = (y0 + 1 >= 0 && y0 + 1 < H) ? 1.f : 0.f;
         const float ml0 = (l0 >= 0 && l0 < L) ? 1.f : 0.f, ml1 = (l0 + 1 >= 0 && l0 + 1 < L) ? 1.f : 0.f;
-        if (x0 != cx || y0 != cy) {                          // plane cell changed: flush the 4 corners
+        if (FG && (x0 != cx || y0 != cy)) {                  // plane cell changed: flush the 4 corners
             if (cx != INT_MIN) {
 #pragma unroll
                 for (int k = 0; k < NQ; ++k) {
@@ -290,7 +293,7 @@ __device__ __forceinline__ void walk_plane(const ScatterArgs& A, const int e0, c
             for (int k = 0; k < NQ; ++k) { g00[k] = f4z(); g10[k] = f4z(); g01[k] = f4z(); g11[k] = f4z(); }
             cx = x0; cy = y0; s00 = o00; s10 = o10; s01 = o01; s11 = o11;
         }
-        if (l0 != cl) {                                      // line cell changed
+        if (FG && l0 != cl) {                                // line cell changed
             if (cl != INT_MIN) {
 #pragma unroll
                 for (int k = 0; k < NQ; ++k) { red_add_v4(GL + sl0 + k * qs, gl0[k]); red_add_v4(GL + sl1 + k * qs, gl1[k]); }
@@ -315,8 +318,10 @@ __device__ __forceinline__ void walk_plane(const ScatterArgs& A, const int e0, c
             const float4 g4 = gin_value(gc, k);
             const float4 gl = f4_mul2(g4, lv);       // dL/dP (interpolated plane value)
             const float4 gp = f4_mul2(g4, pv);       // dL/dL (interpolated line value)
-            f4_fma(g00[k], gl, w00); f4_fma(g10[k], gl, w10); f4_fma(g01[k], gl, w01); f4_fma(g11[k], gl, w11);
-            f4_fma(gl0[k], gp, wl0p); f4_fma(gl1[k], gp, wl1p);
+            if constexpr (FG) {
+                f4_fma(g00[k], gl, w00); f4_fma(g10[k], gl, w10); f4_fma(g01[k], gl, w01); f4_fma(g11[k], gl, w11);
+                f4_fma(gl0[k], gp, wl0p); f4_fma(gl1[k], gp, wl1p);
+            }
             f2_dot_acc(dA2, gl, a); f2_dot_acc(dB2, gl, b); f2_dot_acc(dC2, gl, c); f2_dot_acc(dD2, gl, d);
             f2_dot_acc(dLa2, gp, la); f2_dot_acc(dLb2, gp, lb4);
         }
@@ -332,21 +337,21 @@ __device__ __forceinline__ void walk_plane(const ScatterArgs& A, const int e0, c
         rs.o[al] += dul; rs.d[al] = fmaf(dul, t, rs.d[al]);
     }
     cp_async_wait0();
-    if (cx != INT_MIN) {
+    if (FG && cx != INT_MIN) {
 #pragma unroll
         for (int k = 0; k < NQ; ++k) {
             red_add_v4(GP + s00 + k * qs, g00[k]); red_add_v4(GP + s10 + k * qs, g10[k]);
             red_add_v4(GP + s01 + k * qs, g01[k]); red_add_v4(GP + s11 + k * qs, g11[k]);
         }
     }
-    if (cl != INT_MIN) {
+    if (FG && cl != INT_MIN) {
 #pragma unroll
         for (int k = 0; k < NQ; ++k) { red_add_v4(GL + sl0 + k * qs, gl0[k]); red_add_v4(GL + sl1 + k * qs, gl1[k]); }
     }
     flush_ray();
 }
 
-template <bool APP, int NQ, int MINB, bool GB16, int LWC, bool B16>
+template <bool APP, int NQ, int MINB, bool GB16, int LWC, bool B16, bool FG>
 __global__ void __launch_bounds__(SC_THREADS, MINB) vm_scatter_walk_kernel(const ScatterArgs A, int LW_rt, int walkers_per_cta) {
     extern __shared__ __align__(16) unsigned char sc_smem[];   // 12 NQ slots x SC_THREADS quads (16 B fp32 / 8 B bf16)
     using SlotT = typename std::conditional<B16, uint2, float4>::type;
@@ -376,9 +381,9 @@ __global__ void __launch_bounds__(SC_THREADS, MINB) vm_scatter_walk_kernel(const
         RaySums rs;
 #pragma unroll
         for (int a = 0; a < 3; ++a) rs.o[a] = rs.d[a] = 0.f;
-        if (A.plane_mask & 1) walk_plane<APP, NQ, 0, GB16, B16>(A, e0, e1, q, qs, ray, ray_end, rs, sm);
-        if (A.plane_mask & 2) walk_plane<APP, NQ, 1, GB16, B16>(A, e0, e1, q, qs, ray, ray_end, rs, sm);
-        if (A.plane_mask & 4) walk_plane<APP, NQ, 2, GB16, B16>(A, e0, e1, q, qs, ray, ray_end, rs, sm);
+        if (A.plane_mask & 1) walk_plane<APP, NQ, 0, GB16, B16, FG>(A, e0, e1, q, qs, ray, ray_end, rs, sm);
+        if (A.plane_mask & 2) walk_plane<APP, NQ, 1, GB16, B16, FG>(A, e0, e1, q, qs, ray, ray_end, rs, sm);
+        if (A.plane_mask & 4) walk_plane<APP, NQ, 2, GB16, B16, FG>(A, e0, e1, q, qs, ray, ray_end, rs, sm);
     }
 }
 
@@ -390,16 +395,17 @@ extern "C" int jt_vm_scatter_rays(int app, const void* const* h_factors, void* c
                                   const int* h_dims, const float* samp, const int* slot, const int* sidx,
                                   const int* n_dev, int n_max, const void* gin, int gin_bf16, int n_samples, const float* h_inv,
                                   float* d_o, float* d_d, int max_ctas, int plane_mask, cudaStream_t stream) {
-    JT_CHECK_ARG(h_factors && h_factor_grads && h_dims && samp && sidx && gin && h_inv && d_o && d_d && n_samples > 0);
+    JT_CHECK_ARG(h_factors && h_dims && samp && sidx && gin && h_inv && d_o && d_d && n_samples > 0);
     JT_CHECK_ARG(plane_mask > 0 && plane_mask <= 7);
     if (n_max <= 0) return JT_OK;
     ScatterArgs A;
     if (int rc = fill_factors(A.F, h_factors, h_dims)) return rc;
+    const bool fg = h_factor_grads != nullptr;              // NULL: coordinate-only walk (d_o / d_d alone)
     int cmax = 0;
     for (int i = 0; i < 3; ++i) {
-        A.G.plane[i] = static_cast<float*>(h_factor_grads[i]);
-        A.G.line[i] = static_cast<float*>(h_factor_grads[3 + i]);
-        JT_CHECK_ARG(A.G.plane[i] && A.G.line[i]);
+        A.G.plane[i] = fg ? static_cast<float*>(h_factor_grads[i]) : nullptr;
+        A.G.line[i] = fg ? static_cast<float*>(h_factor_grads[3 + i]) : nullptr;
+        JT_CHECK_ARG(!fg || (A.G.plane[i] && A.G.line[i]));
         cmax = A.F.C[i] > cmax ? A.F.C[i] : cmax;
         JT_CHECK_ARG((long long)A.F.H[i] * A.F.W[i] * A.F.C[i] < 2147483647LL);
     }
@@ -432,27 +438,36 @@ extern "C" int jt_vm_scatter_rays(int app, const void* const* h_factors, void* c
     const int threads = ((wpc * LW + 31) / 32) * 32;
     long long units = ((long long)n_max + A.seg - 1) / A.seg;
     long long want = (units + wpc - 1) / wpc;
-    const int resident = nq == 3 ? 2 : (nq == 2 || app) ? 3 : 4;   // CTAs per SM of the variant launched below (MINB)
+    // CTAs per SM of the variant launched below (its MINB). Without the gradient accumulators the coordinate-only
+    // variants fit more CTAs per SM; nq = 3 with fp32 taps is then bound by shared memory (3 x 72 KB).
+    const int resident = fg ? (nq == 3 ? 2 : (nq == 2 || app) ? 3 : 4) : (nq == 3 ? 3 : nq == 2 ? 4 : 5);
     long long cap = max_ctas > 0 ? (long long)max_ctas
                                  : (A.seg_target > 0 ? (long long)kNumSMs * resident : (long long)kNumSMs * 32);
     if (A.seg_target > 0) want = cap;                         // one resident wave; the kernel sizes the segments to fit
     int grid = (int)(want < cap ? (want < 1 ? 1 : want) : cap);
     g_launches += 1;
     const int smem = 12 * nq * SC_THREADS * (A.F.bf16 ? 8 : 16);
-#define JT_SCB(APPV, NQV, MB, GB, LWV, BV)                                                                          \
+#define JT_SCB(APPV, NQV, MB, GB, LWV, BV, FGV)                                                                     \
     {                                                                                                               \
         if (smem > 48 * 1024 &&                                                                                     \
-            cudaFuncSetAttribute(vm_scatter_walk_kernel<APPV, NQV, MB, GB, LWV, BV>,                                \
+            cudaFuncSetAttribute(vm_scatter_walk_kernel<APPV, NQV, MB, GB, LWV, BV, FGV>,                           \
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess)                 \
             return JT_ERR_LAUNCH;                                                                                   \
-        vm_scatter_walk_kernel<APPV, NQV, MB, GB, LWV, BV><<<grid, threads, smem, stream>>>(A, LW, wpc);            \
+        vm_scatter_walk_kernel<APPV, NQV, MB, GB, LWV, BV, FGV><<<grid, threads, smem, stream>>>(A, LW, wpc);       \
     }
-#define JT_SC(APPV, NQV, MB, GB, LWV) { if (A.F.bf16) JT_SCB(APPV, NQV, MB, GB, LWV, true) else JT_SCB(APPV, NQV, MB, GB, LWV, false) }
+#define JT_SC(APPV, NQV, MB, GB, LWV) { if (A.F.bf16) JT_SCB(APPV, NQV, MB, GB, LWV, true, true) else JT_SCB(APPV, NQV, MB, GB, LWV, false, true) }
+#define JT_SCC(APPV, NQV, MB, GB, LWV) { if (A.F.bf16) JT_SCB(APPV, NQV, MB, GB, LWV, true, false) else JT_SCB(APPV, NQV, MB, GB, LWV, false, false) }
     // (64-thread CTAs with a 200-register cap -- five CTAs per SM instead of two -- spill and lose: 1.55 vs 1.22 ms;
     // a minimum-blocks bound of 3 (168 registers) likewise: 2.28 ms.)
-    if (app && gin_bf16) { if (nq == 3) JT_SC(true, 3, 2, true, 4) else if (nq == 2) JT_SC(true, 2, 3, true, 4) else JT_SC(true, 1, 3, true, 0) }
+    if (!fg) {      // coordinate-only: MINB as `resident` above (no spills at these bounds, -Xptxas -v)
+        if (app && gin_bf16) { if (nq == 3) JT_SCC(true, 3, 3, true, 4) else if (nq == 2) JT_SCC(true, 2, 4, true, 4) else JT_SCC(true, 1, 5, true, 0) }
+        else if (app) { if (nq == 3) JT_SCC(true, 3, 3, false, 4) else if (nq == 2) JT_SCC(true, 2, 4, false, 4) else JT_SCC(true, 1, 5, false, 0) }
+        else { if (nq == 3) JT_SCC(false, 3, 3, false, 4) else if (nq == 2) JT_SCC(false, 2, 4, false, 4) else JT_SCC(false, 1, 5, false, 0) }
+    }
+    else if (app && gin_bf16) { if (nq == 3) JT_SC(true, 3, 2, true, 4) else if (nq == 2) JT_SC(true, 2, 3, true, 4) else JT_SC(true, 1, 3, true, 0) }
     else if (app) { if (nq == 3) JT_SC(true, 3, 2, false, 4) else if (nq == 2) JT_SC(true, 2, 3, false, 4) else JT_SC(true, 1, 3, false, 0) }
     else { if (nq == 3) JT_SC(false, 3, 2, false, 4) else if (nq == 2) JT_SC(false, 2, 3, false, 4) else JT_SC(false, 1, 4, false, 0) }
+#undef JT_SCC
 #undef JT_SC
 #undef JT_SCB
     JT_RETURN_LAUNCH();

@@ -290,7 +290,9 @@ __device__ __forceinline__ uint32_t chunk_pos_mask(const uint4 q) {     // 8 bf1
 }
 
 // dout [A][4] = dL/d(pre-sigmoid) (jt_render_bwd folds the sigmoid derivative in) -> dcomps [A][60] fp32 for the VM
-// scatter; stages D2, D1, DF, DO next to the forward's tiles for the weight-gradient kernel.
+// scatter; stages D2, D1, DF, DO next to the forward's tiles for the weight-gradient kernel (WST = false: a frozen
+// head and basis_mat, nothing is staged and dcomps is the same bit for bit).
+template <bool WST>
 __global__ void __launch_bounds__(NT) wv_head_bwd_data_kernel(const float* __restrict__ dout, const float* __restrict__ featdir,
                                                               const float* __restrict__ Wb, const float* __restrict__ W1,
                                                               const float* __restrict__ W2, const float* __restrict__ W3,
@@ -335,7 +337,7 @@ __global__ void __launch_bounds__(NT) wv_head_bwd_data_kernel(const float* __res
         // ---- S0: dh2 = (dout W3[:, 12:]) . [h2 > 0] -> D2 ; dout -> DO
         {
             const float v0[8] = {go[0], go[1], go[2], 0.f, 0.f, 0.f, 0.f, 0.f};
-            store_chunk(DO, nullptr, TM, 0, r, v0);
+            if (WST) store_chunk(DO, nullptr, TM, 0, r, v0);
 #pragma unroll
             for (int c = 0; c < HW / 8; ++c) {
                 const uint4 q = __ldg(reinterpret_cast<const uint4*>(st + OFF_WA3 + (size_t)c * TM * 16 + r * 16));
@@ -356,9 +358,11 @@ __global__ void __launch_bounds__(NT) wv_head_bwd_data_kernel(const float* __res
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem + T_DH1, D2, nullptr, w2t, nullptr, HW, HW, HW);
             mma_commit(&bar);
-            bulk_s2g(st + OFF_WD2, D2, SZ_WD2);
-            bulk_s2g(st + OFF_WDO, DO, SZ_WDO);
-            bulk_commit();
+            if (WST) {
+                bulk_s2g(st + OFF_WD2, D2, SZ_WD2);
+                bulk_s2g(st + OFF_WDO, DO, SZ_WDO);
+                bulk_commit();
+            }
         }
         mbar_wait(&bar, phase); phase ^= 1;
         tc_fence_after();
@@ -383,8 +387,10 @@ __global__ void __launch_bounds__(NT) wv_head_bwd_data_kernel(const float* __res
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem + T_DIN, D1, nullptr, w1t, nullptr, HW, K1W, K1W);
             mma_commit(&bar);
-            bulk_s2g(st + OFF_WD1, D1, SZ_WD1);
-            bulk_commit();
+            if (WST) {
+                bulk_s2g(st + OFF_WD1, D1, SZ_WD1);
+                bulk_commit();
+            }
         }
         mbar_wait(&bar, phase); phase ^= 1;
         tc_fence_after();
@@ -433,8 +439,10 @@ __global__ void __launch_bounds__(NT) wv_head_bwd_data_kernel(const float* __res
             tc_fence_after();
             issue_gemm_kmajor<1>(tmem + T_DC, DF, nullptr, wbt, nullptr, NBW, KB, KB);
             mma_commit(&bar);
-            bulk_s2g(st + OFF_WDF, DF, SZ_WDF);
-            bulk_commit();
+            if (WST) {
+                bulk_s2g(st + OFF_WDF, DF, SZ_WDF);
+                bulk_commit();
+            }
         }
         mbar_wait(&bar, phase); phase ^= 1;
         tc_fence_after();
@@ -452,11 +460,11 @@ __global__ void __launch_bounds__(NT) wv_head_bwd_data_kernel(const float* __res
                 }
             }
         }
-        if (tid == 0) bulk_wait_read0();       // D2 / D1 / DF / DO have left shared memory
+        if (WST && tid == 0) bulk_wait_read0();       // D2 / D1 / DF / DO have left shared memory
         tc_fence_before();
         __syncthreads();
     }
-    if (tid == 0) bulk_wait0();
+    if (WST && tid == 0) bulk_wait0();
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem, 256);
@@ -623,7 +631,8 @@ extern "C" int jt_wv_head_bwd_tc(const float* dout, const float* featdir, const 
                                  float* gWb, float* gW1, float* gb1, float* gW2, float* gb2, float* gW3, float* gb3,
                                  cudaStream_t stream) {
     JT_CHECK_ARG(dout && featdir && Wb && W1 && W2 && W3 && dcomps && stage);
-    JT_CHECK_ARG(gWb && gW1 && gb1 && gW2 && gb2 && gW3 && gb3);
+    const int n_wg = !!gWb + !!gW1 + !!gb1 + !!gW2 + !!gb2 + !!gW3 + !!gb3;
+    JT_CHECK_ARG(n_wg == 0 || n_wg == 7);                // all weight gradients, or none (frozen head + basis_mat)
     JT_CHECK_ARG((reinterpret_cast<uintptr_t>(stage) & 127) == 0 && (reinterpret_cast<uintptr_t>(dcomps) & 15) == 0);
     if (n_max <= 0) return JT_OK;
     long long tiles = ((long long)n_max + TM - 1) / TM;
@@ -632,12 +641,19 @@ extern "C" int jt_wv_head_bwd_tc(const float* dout, const float* featdir, const 
     // each CTA of the data kernel owns 256 of the SM's 512 TMEM columns: ask for enough shared memory that no third
     // CTA becomes resident and waits inside tcgen05.alloc
     const int smem_d = BwdSmemW::total > 100 * 1024 ? BwdSmemW::total : 100 * 1024;
-    if (int rc = set_smem(wv_head_bwd_data_kernel, smem_d)) return rc;
-    if (int rc = set_smem(wv_head_bwd_wgrad_kernel, WGW_STAGES * WGW_STAGE_BYTES)) return rc;
-    g_launches += 2;
     unsigned char* st = static_cast<unsigned char*>(stage);
-    wv_head_bwd_data_kernel<<<grid_d, NT, smem_d, stream>>>(dout, featdir, Wb, W1, W2, W3, n_dev, n_max, fea_progress,
-                                                                    dcomps, st);
+    g_launches += 1;
+    if (n_wg == 0) {
+        if (int rc = set_smem(wv_head_bwd_data_kernel<false>, smem_d)) return rc;
+        wv_head_bwd_data_kernel<false><<<grid_d, NT, smem_d, stream>>>(dout, featdir, Wb, W1, W2, W3, n_dev, n_max,
+                                                                       fea_progress, dcomps, st);
+        JT_RETURN_LAUNCH();
+    }
+    if (int rc = set_smem(wv_head_bwd_data_kernel<true>, smem_d)) return rc;
+    if (int rc = set_smem(wv_head_bwd_wgrad_kernel, WGW_STAGES * WGW_STAGE_BYTES)) return rc;
+    g_launches += 1;
+    wv_head_bwd_data_kernel<true><<<grid_d, NT, smem_d, stream>>>(dout, featdir, Wb, W1, W2, W3, n_dev, n_max, fea_progress,
+                                                                  dcomps, st);
     wv_head_bwd_wgrad_kernel<<<grid_w, TM, WGW_STAGES * WGW_STAGE_BYTES, stream>>>(st, n_dev, n_max, gWb, gW1, gb1, gW2, gb2, gW3, gb3);
     JT_RETURN_LAUNCH();
 }

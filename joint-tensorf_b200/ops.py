@@ -196,8 +196,8 @@ def vm_gather_bwd(app, fs, gp, gl, samp, slot, n_dev, n_max, gin, dsamp, accumul
 def vm_scatter_rays(app, fs, gp, gl, samp, slot, sidx, n_dev, n_max, gin, n_samples, h_inv, d_o, d_d, max_ctas=0,
                     plane_mask=7):
     """Run-merged factor-gradient scatter + per-ray pose-path gradients (vm_scatter.cu). plane_mask: which of the
-    three plane / line pairs this launch walks (7 = all)."""
-    gptrs = ptrs([g.data_ptr() for g in gp] + [g.data_ptr() for g in gl])
+    three plane / line pairs this launch walks (7 = all). gp = gl = None: coordinate-only walk (d_o / d_d alone)."""
+    gptrs = None if gp is None else ptrs([g.data_ptr() for g in gp] + [g.data_ptr() for g in gl])
     with TIMER.span("vm_app_bwd" if app else "vm_density_bwd"):
         check(_lib.lib().jt_vm_scatter_rays(int(app), fs.ptrs, gptrs, fs.dims, _p(samp), _p(slot), _p(sidx),
                                             _p(n_dev), int(n_max), _p(gin), int(gin.dtype == torch.bfloat16),
@@ -280,7 +280,7 @@ def app_basis_sh_fwd_tc(split, fs, samp, aidx, sidx, rays_d, n_samples, normaliz
 
 
 def sh_bwd_tc(dout, featdir, wb, n_dev, n_max, dcomps, stage, g_basis):
-    """g_basis [27][144] zero-initialised by the caller (accumulated)."""
+    """g_basis [27][144] zero-initialised by the caller (accumulated), or None (frozen basis_mat; stage may be None)."""
     with TIMER.span("sh_bwd_tc"):
         check(_lib.lib().jt_sh_bwd_tc(_p(dout), _p(featdir), int(featdir.shape[1]), _p(wb), _p(n_dev), int(n_max),
                                       _p(dcomps), int(dcomps.dtype == torch.bfloat16), _p(stage), _p(g_basis),
@@ -295,8 +295,9 @@ def head_mlp_fwd_tc(split, featdir, w1, b1, w2, b2, w3, b3, n_dev, n_max, fprog,
 
 
 def head_bwd_tc(dout, feat, wb, w1, w2, w3, n_dev, n_max, fprog, dcomps, stage, grads):
-    """grads = (gWb, gW1, gb1, gW2, gb2, gW3, gb3), zero-initialised by the caller.
+    """grads = (gWb, gW1, gb1, gW2, gb2, gW3, gb3), zero-initialised by the caller, or None (no weight gradients).
     feat: [A][ldf] rows whose first 27 floats are the basis projection (ldf = 28 or 32)."""
+    grads = grads if grads is not None else (None,) * 7
     with TIMER.span("head_bwd_tc"):
         check(_lib.lib().jt_head_bwd_tc(_p(dout), _p(feat), int(feat.shape[1]), _p(wb), _p(w1), _p(w2), _p(w3), _p(n_dev), int(n_max),
                                         float(fprog), _p(dcomps), int(dcomps.dtype == torch.bfloat16), _p(stage),
@@ -321,7 +322,9 @@ def wv_head_fwd_tc(comps, aidx, sidx, rays_d, n_samples, normalize_dir, wb, w1, 
 
 
 def wv_head_bwd_tc(dout, featdir, wb, w1, w2, w3, n_dev, n_max, fprog, dcomps, stage, grads):
-    """grads = (gWb, gW1, gb1, gW2, gb2, gW3, gb3), zero-initialised by the caller; dcomps [A][60] fp32."""
+    """grads = (gWb, gW1, gb1, gW2, gb2, gW3, gb3), zero-initialised by the caller, or None (no weight gradients);
+    dcomps [A][60] fp32."""
+    grads = grads if grads is not None else (None,) * 7
     with TIMER.span("wv_head_bwd_tc"):
         check(_lib.lib().jt_wv_head_bwd_tc(_p(dout), _p(featdir), _p(wb), _p(w1), _p(w2), _p(w3), _p(n_dev), int(n_max),
                                            float(fprog), _p(dcomps), _p(stage), *[_p(g) for g in grads], _stream()),
@@ -387,7 +390,10 @@ class BlurGroup(torch.autograd.Function):
             full.append((hq, wq, c, axes, ts))
         ys = blur_multi(xs, full, tapsets, 0)
         ctx.meta = (full, tapsets, [tuple(xp.shape) for xp in xs])
-        return tuple(y.view(1, m[0], m[1], m[2]).permute(0, 3, 1, 2) for y, m in zip(ys, full))
+        outs = tuple(y.view(1, m[0], m[1], m[2]).permute(0, 3, 1, 2) for y, m in zip(ys, full))
+        # a blurred copy of a frozen factor is frozen too, so that the render op sees which factors need a gradient
+        ctx.mark_non_differentiable(*[y for i, y in enumerate(outs) if not ctx.needs_input_grad[2 + i]])
+        return outs
 
     @staticmethod
     def backward(ctx, *gys):

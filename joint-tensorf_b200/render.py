@@ -14,6 +14,10 @@ index, SURVEY.md section 2b):
             (pose-path gradients accumulate inside the scatters; with a gradient synchroniser attached the
             appearance part of the flat gradient bucket is all-reduced while the density scatter runs)
 
+The backward computes only the gradients autograd asks for (ctx.needs_input_grad). With a frozen scene (test-time
+pose optimisation: freeze_scene()) it runs the head backward without weight gradients and both scatters
+coordinate-only, and allocates no factor-gradient bucket.
+
 Sample counts (V valid samples, A appearance samples) stay on the device; the
 kernels read them from `ray_off[N]` / `app_off[N]` and run persistent grids.
 """
@@ -125,36 +129,47 @@ class _Head:
         return rgb
 
     @staticmethod
-    def backward(cfg, ws, dout, feat, ldf, aidx, sidx, rays_d, a_count, cap, params, dev):
-        """dout [cap,4] -> dfeat [cap, ldf]; returns (dfeat, param grads list)."""
+    def backward(cfg, ws, dout, feat, ldf, aidx, sidx, rays_d, a_count, cap, params, dev, wgrad=True):
+        """dout [cap,4] -> dfeat [cap, ldf]; returns (dfeat, param grads list). wgrad=False (frozen head): the weight
+        gradient GEMMs are skipped and the list is empty."""
         F, H = cfg.app_dim, cfg.hidden
         dfeat = torch.empty((cap, ldf), device=dev)
         if cfg.shading == "SH":
             ops.sh_shade(1, feat, ldf, aidx, sidx, rays_d, cfg.n_samples, cfg.ndc, a_count, cap, None, dout, dfeat, ldf)
             return dfeat, []
         w1, b1, w2, b2, w3, b3 = params
-        gw1, gb1, gw2, gb2, gw3, gb3 = [torch.zeros_like(t) for t in params]
+        gw1, gb1, gw2, gb2, gw3, gb3 = [torch.zeros_like(t) for t in params] if wgrad else [None] * 6
         x, ldi, in_dim, h1 = ws["x"], ws["ldi"], ws["in_dim"], ws["h1"]
         dh2 = torch.empty((cap, H), device=dev)
         dh1 = torch.empty((cap, H), device=dev)
         if cfg.shading == "MLP_Fea":
             h2 = ws["h2"]
-            ops.gemm_tn(dout, 4, h2, H, a_count, cap, 3, H, gw3, H, gb3, name="mlp_l3_bwd_w")
+            if wgrad:
+                ops.gemm_tn(dout, 4, h2, H, a_count, cap, 3, H, gw3, H, gb3, name="mlp_l3_bwd_w")
             ops.gemm_nt(dout, 4, w3, H, 1, None, dh2, H, h2, H, a_count, cap, H, 3, 0, name="mlp_l3_bwd_x")
         else:
             mid, ldm, nv = ws["mid"], ws["ldm"], ws["nv"]
-            ops.gemm_tn(dout, 4, mid, ldm, a_count, cap, 3, ldm, gw3, ldm, gb3, name="mlp_l3_bwd_w")
+            if wgrad:
+                ops.gemm_tn(dout, 4, mid, ldm, a_count, cap, 3, ldm, gw3, ldm, gb3, name="mlp_l3_bwd_w")
             ops.gemm_nt(dout, 4, w3, ldm, 1, None, dh2, H, mid, ldm, a_count, cap, H, 3, 0, name="mlp_l3_bwd_x",
                         w_off=nv, mask_off=nv)
-        ops.gemm_tn(dh2, H, h1, H, a_count, cap, H, H, gw2, H, gb2, name="mlp_l2_bwd_w")
+        if wgrad:
+            ops.gemm_tn(dh2, H, h1, H, a_count, cap, H, H, gw2, H, gb2, name="mlp_l2_bwd_w")
         ops.gemm_nt(dh2, H, w2, H, 1, None, dh1, H, h1, H, a_count, cap, H, H, 0, name="mlp_l2_bwd_x")
-        ops.gemm_tn(dh1, H, x, ldi, a_count, cap, H, in_dim, gw1, in_dim, gb1, name="mlp_l1_bwd_w")
+        if wgrad:
+            ops.gemm_tn(dh1, H, x, ldi, a_count, cap, H, in_dim, gw1, in_dim, gb1, name="mlp_l1_bwd_w")
         # the encoded input is dead after dW1: reuse its buffer for its own gradient
         ops.gemm_nt(dh1, H, w1, in_dim, 1, None, x, ldi, None, 0, a_count, cap, in_dim, H, 0, name="mlp_l1_bwd_x")
         mode = 0 if cfg.shading == "MLP_Fea" else 1
         ops.pe_encode(1, F, cfg.fea_pe, cfg.view_pe, mode, cfg.fea_prog, cfg.view_prog, cfg.n_samples, cfg.ndc,
                       feat, ldf, None, None, None, a_count, cap, dfeat, ldf, None, 0, x, ldi)
-        return dfeat, [gw1, gb1, gw2, gb2, gw3, gb3]
+        return dfeat, ([gw1, gb1, gw2, gb2, gw3, gb3] if wgrad else [])
+
+
+def _full_backward(cfg):
+    """An active gradient synchroniser (data parallel, outside `sync.paused()`) runs the full backward on every rank."""
+    sync = getattr(cfg, "grad_sync", None)
+    return sync is not None and sync._active()
 
 
 class VMRender(torch.autograd.Function):
@@ -245,7 +260,10 @@ class VMRender(torch.autograd.Function):
             tc_supported(cfg, afs, raise_if_not=True)
             rgb = torch.empty((cap, 4), device=dev)
             feat = torch.empty((cap, 32), device=dev)             # feat 0..26 | 0 | view dir 28..30 | 0
-            ws["stage"] = ops.head_tc_stage(cap, dev) if train else None
+            # SH: the staged component tile only feeds the basis_mat weight gradient (MLP_Fea: the data backward
+            # reads the staged relu tiles as well)
+            sh_stage = ctx.needs_input_grad[16] or _full_backward(cfg)
+            ws["stage"] = ops.head_tc_stage(cap, dev) if train and (cfg.shading != "SH" or sh_stage) else None
             if cfg.shading == "SH":
                 ops.app_basis_sh_fwd_tc(cfg.tc_fwd_split, afs, comp.samp, aidx, comp.sidx, rays_d, S, cfg.ndc,
                                         basis_w, a_count, cap, feat, rgb, ws["stage"])
@@ -323,61 +341,88 @@ class VMRender(torch.autograd.Function):
                                           weight=b["weight"].clone(), trans=b["trans"].clone(), rgb=b["rgb"].clone(),
                                           sigfeat=b["sigfeat"].clone(), a_count=b["a_count"].clone())
 
+        # Only the gradients autograd asks for. Input order: cfg, rays_o, rays_d, aux, 6 density factors, 6 appearance
+        # factors, basis_mat, head parameters. With an active gradient synchroniser every rank runs the full backward,
+        # so that all ranks issue the same collectives whatever their parameters' requires_grad.
+        sync = cfg.grad_sync if _full_backward(cfg) else None      # None: world size 1, or inside `sync.paused()`
+        ng = ctx.needs_input_grad
+        if sync is not None:
+            need_rays = need_dens = need_app = need_basis = need_head = True
+        else:
+            need_rays, need_dens, need_app = ng[1] or ng[2], any(ng[4:10]), any(ng[10:16])
+            need_basis, need_head = ng[16], any(ng[17:])
+        need_wgrad = need_basis or need_head
+
         # One flat zero-filled bucket for every gradient this node produces (one memset; also the unit the
-        # data-parallel all-reduce works on): [app planes, app lines | density planes, density lines | basis, head].
-        # The appearance part comes first and is complete first, so a gradient synchroniser
-        # (parallel.OverlappedGradSync) can reduce it across ranks while the density scatter still runs.
-        sync = getattr(cfg, "grad_sync", None)
-        if sync is not None and not sync._active():       # world size 1, or inside `with sync.paused():`
-            sync = None
-        shapes = [p.shape for p in afs.planes] + [l.shape for l in afs.lines] + \
-                 [p.shape for p in dfs.planes] + [l.shape for l in dfs.lines] + \
-                 [b["basis_w"].shape] + [t.shape for t in b["head"]]
+        # data-parallel all-reduce works on): [app planes, app lines | density planes, density lines | basis, head],
+        # each group present only when it is needed. The appearance part comes first and is complete first, so a
+        # gradient synchroniser (parallel.OverlappedGradSync) can reduce it across ranks while the density scatter
+        # still runs.
+        shapes = ([p.shape for p in afs.planes] + [l.shape for l in afs.lines] if need_app else []) + \
+                 ([p.shape for p in dfs.planes] + [l.shape for l in dfs.lines] if need_dens else []) + \
+                 ([b["basis_w"].shape] if need_basis else []) + ([t.shape for t in b["head"]] if need_head else [])
         sizes = [int(torch.Size(s).numel()) for s in shapes]
         flat = torch.zeros((sum(sizes),), device=dev)
         views, o = [], 0
         for s, n in zip(shapes, sizes):
             views.append(flat[o:o + n].view(s))
             o += n
-        gap, gal, gdp, gdl = views[0:3], views[3:6], views[6:9], views[9:12]
-        g_basis, head_grads = views[12], views[13:]
-        n_app = sum(sizes[0:6])
+        it = iter(views)
+        gap, gal = ([next(it) for _ in range(3)], [next(it) for _ in range(3)]) if need_app else (None, None)
+        gdp, gdl = ([next(it) for _ in range(3)], [next(it) for _ in range(3)]) if need_dens else (None, None)
+        g_basis = next(it) if need_basis else None
+        head_grads = [next(it) for _ in b["head"]] if need_head else None
+        n_app = sum(sizes[0:6]) if need_app else 0
 
         d_o = torch.empty((N, 3), device=dev)
         d_d = torch.empty((N, 3), device=dev)
         with TIMER.span("ray_init"):
             check(lib.jt_ray_init(_p(b["rays_d"]), _p(dnorm), N, _p(d_o), _p(d_d), _stream()), "jt_ray_init")
 
-        # tensor-core head: dcomps crosses HBM as bf16 (its GEMM operands are bf16 already)
-        wv_tc = cfg.head == "tc" and cfg.shading == "MLP_Fea_WeakView"
-        dcomps = torch.empty((cap, afs.ctot), device=dev,
-                             dtype=torch.bfloat16 if (cfg.head == "tc" and not wv_tc) else torch.float32)
-        if wv_tc:
-            w1, b1, w2, b2, w3, b3 = b["head"]
-            ops.wv_head_bwd_tc(dout, b["feat"], b["basis_w"], w1, w2, w3, b["a_count"], cap, cfg.fea_prog, dcomps,
-                               ws["stage"], (g_basis, *head_grads))
-        elif cfg.head == "tc" and cfg.shading == "SH":
-            ops.sh_bwd_tc(dout, b["feat"], b["basis_w"], b["a_count"], cap, dcomps, ws["stage"], g_basis)
-        elif cfg.head == "tc":
-            w1, b1, w2, b2, w3, b3 = b["head"]
-            ops.head_bwd_tc(dout, b["feat"], b["basis_w"], w1, w2, w3, b["a_count"], cap, cfg.fea_prog, dcomps,
-                            ws["stage"], (g_basis, *head_grads))
-        else:
-            dfeat, hg = _Head.backward(cfg, ws, dout, b["feat"], ldf, b["aidx"], comp.sidx, b["rays_d"],
-                                       b["a_count"], cap, b["head"], dev)
-            if cfg.shading != "SH":
-                ws["consumed"] = True
-            for dst, src in zip(head_grads, hg):
-                dst.copy_(src)
-            ops.gemm_tn(dfeat, ldf, b["comps"], afs.ctot, b["a_count"], cap, F, afs.ctot, g_basis, afs.ctot, None,
-                        name="basis_bwd_w")
-            ops.gemm_nt(dfeat, ldf, b["basis_w"], afs.ctot, 1, None, dcomps, afs.ctot, None, 0, b["a_count"], cap,
-                        afs.ctot, F, 0, name="basis_bwd_x")
+        # the head backward and dcomps feed the appearance scatter (factor or ray gradients) and the weight gradients
+        dcomps = None
+        if need_app or need_rays or need_wgrad:
+            # the tensor-core heads produce all weight gradients or none: a frozen one gets scratch that is dropped
+            wgrads = None
+            if need_wgrad:
+                wgrads = (g_basis if need_basis else torch.zeros_like(b["basis_w"]),
+                          *(head_grads if need_head else [torch.zeros_like(t) for t in b["head"]]))
+            # tensor-core head: dcomps crosses HBM as bf16 (its GEMM operands are bf16 already)
+            wv_tc = cfg.head == "tc" and cfg.shading == "MLP_Fea_WeakView"
+            dcomps = torch.empty((cap, afs.ctot), device=dev,
+                                 dtype=torch.bfloat16 if (cfg.head == "tc" and not wv_tc) else torch.float32)
+            if wv_tc:
+                w1, b1, w2, b2, w3, b3 = b["head"]
+                ops.wv_head_bwd_tc(dout, b["feat"], b["basis_w"], w1, w2, w3, b["a_count"], cap, cfg.fea_prog, dcomps,
+                                   ws["stage"], wgrads)
+            elif cfg.head == "tc" and cfg.shading == "SH":
+                # no staged component tile when basis_mat was frozen in the forward: no weight gradient either
+                sh_gb = g_basis if (need_basis and ws["stage"] is not None) else None
+                ops.sh_bwd_tc(dout, b["feat"], b["basis_w"], b["a_count"], cap, dcomps, ws["stage"], sh_gb)
+            elif cfg.head == "tc":
+                w1, b1, w2, b2, w3, b3 = b["head"]
+                ops.head_bwd_tc(dout, b["feat"], b["basis_w"], w1, w2, w3, b["a_count"], cap, cfg.fea_prog, dcomps,
+                                ws["stage"], wgrads)
+            else:
+                dfeat, hg = _Head.backward(cfg, ws, dout, b["feat"], ldf, b["aidx"], comp.sidx, b["rays_d"],
+                                           b["a_count"], cap, b["head"], dev, wgrad=need_head)
+                if cfg.shading != "SH":
+                    ws["consumed"] = True
+                for dst, src in zip(head_grads or [], hg):
+                    dst.copy_(src)
+                if need_basis:
+                    ops.gemm_tn(dfeat, ldf, b["comps"], afs.ctot, b["a_count"], cap, F, afs.ctot, g_basis, afs.ctot,
+                                None, name="basis_bwd_w")
+                ops.gemm_nt(dfeat, ldf, b["basis_w"], afs.ctot, 1, None, dcomps, afs.ctot, None, 0, b["a_count"], cap,
+                            afs.ctot, F, 0, name="basis_bwd_x")
+        # a frozen factor group is walked coordinate-only (no factor gradients) when the rays need a gradient
         if sync is None:
-            ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
-                                cfg.n_samples, cfg.h_inv, d_o, d_d)
-            ops.vm_scatter_rays(0, dfs, gdp, gdl, comp.samp, None, comp.sidx, comp.count, cap_v, dsig, cfg.n_samples,
-                                cfg.h_inv, d_o, d_d)
+            if need_app or need_rays:
+                ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
+                                    cfg.n_samples, cfg.h_inv, d_o, d_d)
+            if need_dens or need_rays:
+                ops.vm_scatter_rays(0, dfs, gdp, gdl, comp.samp, None, comp.sidx, comp.count, cap_v, dsig,
+                                    cfg.n_samples, cfg.h_inv, d_o, d_d)
         elif getattr(sync, "per_plane", False):
             # variant (OverlappedGradSync(per_plane=True)): the appearance planes are walked one launch per plane and
             # each plane's gradients are all-reduced while the next launches run -- [plane 0] [plane 1] [plane 2 + the
@@ -429,10 +474,11 @@ class VMRender(torch.autograd.Function):
             # them to p.grad, clone them, feed the adjoint blur) sees the cross-rank sums
             sync.on_rest(flat[n_app:])
 
-        gdpn, gdln = FactorSet.grads_as_nchw(gdp, gdl)
-        gapn, galn = FactorSet.grads_as_nchw(gap, gal)
+        gdpn, gdln = FactorSet.grads_as_nchw(gdp, gdl) if need_dens else ([None] * 3, [None] * 3)
+        gapn, galn = FactorSet.grads_as_nchw(gap, gal) if need_app else ([None] * 3, [None] * 3)
         VMRender.last_grad_bucket = flat
-        return (None, d_o, d_d, None, *gdpn, *gdln, *gapn, *galn, g_basis, *head_grads)
+        return (None, d_o if need_rays else None, d_d if need_rays else None, None, *gdpn, *gdln, *gapn, *galn, g_basis,
+                *(head_grads if need_head else [None] * ctx.n_head))
 
 
 VMRender.last_grad_bucket = None
