@@ -64,6 +64,61 @@ __global__ void __launch_bounds__(256, 4) vm_fwd_kernel(Factors F, const float4*
     }
 }
 
+// Density feature of a field whose three planes all have 16 channels (every shipped config). vm_fwd_kernel<false>
+// spends most of its issue slots on per-sample setup -- record load, 3 x 3 tap positions, weights, offsets -- that
+// each of the 4 lanes of a sample repeats for one quad of channels. Here 2 lanes share a sample and lane h owns
+// quads 2h and 2h + 1 (channels 8h .. 8h + 7), so a warp covers 16 samples for about the same setup work, and the
+// offsets are 32-bit (the host checks H W C < 2^31). The sum keeps vm_fwd_kernel's order -- per quad k,
+// a_k = ((0 + dot_0k) + dot_1k) + dot_2k over the planes, then (a_0 + a_1) + (a_2 + a_3) -- so the result is
+// bit-identical to it.
+template <bool B16>
+__device__ __forceinline__ void dens16_plane(const Factors& F, const int i, const float u[3], const int q,
+                                             float& a0, float& a1) {
+    const Tap tx = make_tap(u[mat0(i)], F.W[i]), ty = make_tap(u[mat1(i)], F.H[i]), tl = make_tap(u[vecm(i)], F.L[i]);
+    const unsigned W = (unsigned)F.W[i];
+    const unsigned r0 = (unsigned)ty.i0 * W, r1 = (unsigned)ty.i1 * W;
+    const unsigned o00 = (r0 + tx.i0) * 16u + q, o10 = (r0 + tx.i1) * 16u + q;
+    const unsigned o01 = (r1 + tx.i0) * 16u + q, o11 = (r1 + tx.i1) * 16u + q;
+    const unsigned ol0 = (unsigned)tl.i0 * 16u + q, ol1 = (unsigned)tl.i1 * 16u + q;
+    const float w00 = tx.w0 * ty.w0, w10 = tx.w1 * ty.w0, w01 = tx.w0 * ty.w1, w11 = tx.w1 * ty.w1;
+    const float* P = F.plane[i];
+    const float* Ln = F.line[i];
+    float4 a[2], b[2], c[2], d[2], la[2], lb[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+        a[k] = ld_tap4<B16>(P, o00 + 4 * k); b[k] = ld_tap4<B16>(P, o10 + 4 * k);
+        c[k] = ld_tap4<B16>(P, o01 + 4 * k); d[k] = ld_tap4<B16>(P, o11 + 4 * k);
+        la[k] = ld_tap4<B16>(Ln, ol0 + 4 * k); lb[k] = ld_tap4<B16>(Ln, ol1 + 4 * k);
+    }
+    a0 += f4_dot(f4_bilin(a[0], w00, b[0], w10, c[0], w01, d[0], w11), f4_lerp2(la[0], tl.w0, lb[0], tl.w1));
+    a1 += f4_dot(f4_bilin(a[1], w00, b[1], w10, c[1], w01, d[1], w11), f4_lerp2(la[1], tl.w0, lb[1], tl.w1));
+}
+
+template <bool B16>
+__global__ void __launch_bounds__(256, 4) vm_density16_fwd_kernel(Factors F, const float4* __restrict__ samp,
+                                                                const int* __restrict__ slot, const int* __restrict__ n_dev,
+                                                                int n_fixed, float* __restrict__ out) {
+    const int n = n_dev ? *n_dev : n_fixed;
+    const int lane = threadIdx.x & 31, h = lane & 1, grp = lane >> 1;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int nwarps = (gridDim.x * blockDim.x) >> 5;
+    for (int base = warp * 16; base < n; base += nwarps * 16) {
+        const int e = base + grp;
+        const bool act = e < n;
+        float a0 = 0.f, a1 = 0.f;                        // quads 2h, 2h + 1
+        if (act) {
+            const int j = slot ? slot[e] : e;
+            const float4 u4 = samp[j];
+            const float u[3] = {u4.x, u4.y, u4.z};
+#pragma unroll
+            for (int i = 0; i < 3; ++i) dens16_plane<B16>(F, i, u, h * 8, a0, a1);
+        }
+        float acc = a0 + a1;
+        acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+        if (act && h == 0) out[e] = acc;
+    }
+}
+
 // Backward of the above. gin: density -> dL/dsigma_feature [n]; app -> dL/dcomponents [n][ctot].
 // dsamp[j] (float4, xyz used) receives dL/du in normalised coordinates; `accumulate`
 // selects store (density pass, runs first) or add (appearance pass; each sample
@@ -162,11 +217,17 @@ extern "C" int jt_vm_gather_fwd(int app, const void* const* h_factors, const int
     if (n_max <= 0) return JT_OK;
     Factors F;
     if (int rc = fill_factors(F, h_factors, h_dims)) return rc;
-    int grid = grid_for(n_max);
+    bool dens16 = !app;                            // density, 16 channels per plane: vm_density16_fwd_kernel
+    for (int i = 0; i < 3; ++i)
+        dens16 = dens16 && F.C[i] == 16 && (long long)F.H[i] * F.W[i] * 16 < 2147483647LL && F.L[i] < (1 << 26);
+    // the same CTA passes over the sample list: 16 samples per warp instead of 8
+    int grid = dens16 ? grid_for((n_max + 1) / 2) : grid_for(n_max);
     g_launches += 1;
     const float4* sp = reinterpret_cast<const float4*>(samp);
     if (app && F.bf16) vm_fwd_kernel<true, true><<<grid, 256, 0, stream>>>(F, sp, slot, n_dev, n_max, out);
     else if (app) vm_fwd_kernel<true, false><<<grid, 256, 0, stream>>>(F, sp, slot, n_dev, n_max, out);
+    else if (dens16 && F.bf16) vm_density16_fwd_kernel<true><<<grid, 256, 0, stream>>>(F, sp, slot, n_dev, n_max, out);
+    else if (dens16) vm_density16_fwd_kernel<false><<<grid, 256, 0, stream>>>(F, sp, slot, n_dev, n_max, out);
     else if (F.bf16) vm_fwd_kernel<false, true><<<grid, 256, 0, stream>>>(F, sp, slot, n_dev, n_max, out);
     else vm_fwd_kernel<false, false><<<grid, 256, 0, stream>>>(F, sp, slot, n_dev, n_max, out);
     JT_RETURN_LAUNCH();

@@ -82,6 +82,14 @@ struct ScatterArgs {
 // (plane index is a compile-time constant of walk_plane). Walkers are laid out over the
 // CTA's threads contiguously and use no warp-level collectives.
 //
+// Walking the three 16-channel density planes in ONE pass instead (per step: one record / sidx / gin load and one
+// ray-change test; per plane only the cell state, 4 lanes x 1 quad per plane, 36 staging slots per lane) is slower:
+// it needs 247 registers without spills (MINB 2; at MINB 3 it spills 420 B), so 8 warps per SM instead of 16, and
+// the three planes' cell state costs more moves than the shared loads save (static loop body 1418 SASS instructions
+// vs 3 x 486). Measured on one B200 at 1000 W (profiles/r03_density_onepass_ab.jsonl): density scatter
+// 0.405 -> 0.563 ms on cfg2_sh, 0.555 -> 0.731 ms on cfg4; coordinate-only (134 registers, MINB 3) no faster either.
+// The 2 lanes x 2 quads layout doubles the per-lane accumulators and cannot fit at all.
+//
 // Tap staging: the kernel is latency-bound, not RED-bound, once the REDs are merged, and the
 // accumulators leave no registers to keep loads in flight. So each lane owns a private,
 // double-buffered shared-memory slot set for the taps of its quads: when the look-ahead
