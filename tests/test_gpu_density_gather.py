@@ -9,43 +9,10 @@ import torch
 
 import joint_tensorf_b200 as jt
 from joint_tensorf_b200 import ops
+from vm_reference import density_feature
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-MAT = ((0, 1), (0, 2), (1, 2))
-VEC = (2, 1, 0)
-
-
-def _axis(g, n):
-    """fp32 tap setup of make_tap (jt_common.cuh): clamped indices and weights (0 for out-of-range taps)"""
-    scale = torch.tensor(0.5 * (n - 1), dtype=torch.float32, device=g.device)
-    x = (g + 1.0) * scale
-    xf = torch.floor(x)
-    f = x - xf
-    i0 = torch.clamp(xf, -2.0, float(n)).to(torch.int64)
-    i1 = i0 + 1
-    m0 = ((i0 >= 0) & (i0 < n)).float()
-    m1 = ((i1 >= 0) & (i1 < n)).float()
-    return i0.clamp(0, n - 1), i1.clamp(0, n - 1), (1.0 - f) * m0, f * m1
-
-
-def _reference(fs, u):
-    """float64 sum_i sum_c P_ic(u) L_ic(u) and sum_i sum_c |P_ic(u) L_ic(u)| with fp32 tap weights"""
-    val = torch.zeros(u.shape[0], dtype=torch.float64, device=DEV)
-    mag = torch.zeros_like(val)
-    for i in range(3):
-        P, L = fs.planes[i].double(), fs.lines[i].double()          # [H,W,C], [L,C]
-        H, W, _ = fs.planes[i].shape
-        x0, x1, wx0, wx1 = _axis(u[:, MAT[i][0]], W)
-        y0, y1, wy0, wy1 = _axis(u[:, MAT[i][1]], H)
-        l0, l1, wl0, wl1 = _axis(u[:, VEC[i]], L.shape[0])
-        w = [(wx0 * wy0), (wx1 * wy0), (wx0 * wy1), (wx1 * wy1)]    # fp32 products, as the kernel forms them
-        pv = (P[y0, x0] * w[0].double()[:, None] + P[y0, x1] * w[1].double()[:, None] +
-              P[y1, x0] * w[2].double()[:, None] + P[y1, x1] * w[3].double()[:, None])
-        lv = L[l0] * wl0.double()[:, None] + L[l1] * wl1.double()[:, None]
-        val += (pv * lv).sum(1)
-        mag += (pv * lv).abs().sum(1)
-    return val, mag
 
 
 def _batch(wl):
@@ -87,7 +54,7 @@ def test_density_feature_matches_float64_evaluation(wl, bf16_factors):
         ref_fs = ops.FactorSet([s.float().permute(2, 0, 1)[None] for s in fs.store[:3]],
                                [s.float().t()[None, :, :, None] for s in fs.store[3:]])
     u = comp.samp[:n, :3]
-    val, mag = _reference(ref_fs, u)
+    val, mag = density_feature(ref_fs.planes, ref_fs.lines, u)
     got = out[:n].double()
     assert torch.isfinite(got).all()
     rel = float(((got - val).abs() / mag.clamp_min(1e-30)).max())
