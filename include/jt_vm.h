@@ -324,6 +324,27 @@ int jt_alpha_mask_build(const float* alpha, int W, int H, int D, float thres, fl
  * channel-last layout: in [H][W][C] -> out [H2][W2][C]; a line factor is W = W2 = 1. */
 int jt_resize_bilinear_cl(const float* in, int H, int W, int C, float* out, int H2, int W2, cudaStream_t stream);
 
+/* ---- mesh export: marching cubes over the dense alpha grid ----------------- */
+/* The step TensoRF-family exporters take after getDenseAlpha (tensorBase.py:618-633): marching cubes on a dense fp32
+ * volume vol [gz][gy][gx] (jt_field_alpha's dense layout) at `level`; a lattice point is inside when value > level.
+ * gx, gy, gz >= 2 and gx*gy*gz < 2^31. Two calls, with one host read of the totals in between to size the outputs:
+ *   jt_mc_count  classifies every cell and writes totals[2] (device long long) = {V, F};
+ *   jt_mc_emit   writes verts [V][3] fp32 and faces [F][3] int32 from the scratch jt_mc_count left for the same vol,
+ *                grid and level; it writes nothing when V or F exceeds INT32_MAX.
+ * Vertices: one per lattice edge whose ends straddle the level, ordered by the linear index (z*gy + y)*gx + x of the
+ * edge's lower end, then by axis x < y < z; position p_a + t (p_b - p_a), t = (level - a)/(b - a), in fp32, where
+ * lattice point (i, j, k) is aabb0*(1-s) + aabb1*s with s from lin_x[i], lin_y[j], lin_z[k] (torch.linspace(0, 1, g),
+ * as jt_field_alpha), h_aabb = {aabb0[3], aabb1[3]} (host). Faces: ordered by the linear index of the cell's corner 0,
+ * then by the case table (csrc/mc_tables.cuh); normals point toward decreasing value.
+ * scratch: jt_mc_scratch_bytes(gx, gy, gz) = ceil(gx*gy*gz / 2048) * 1304 bytes (0.64 bytes per lattice point),
+ * 16-byte aligned; returns -1 for a grid outside the limits above. */
+long long jt_mc_scratch_bytes(int gx, int gy, int gz);
+int jt_mc_count(const float* vol, int gx, int gy, int gz, float level, void* scratch, long long* totals,
+                cudaStream_t stream);
+int jt_mc_emit(const float* vol, int gx, int gy, int gz, float level, const float* lin_x, const float* lin_y,
+               const float* lin_z, const float* h_aabb, const void* scratch, const long long* totals, float* verts,
+               int* faces, cudaStream_t stream);
+
 /* ---- 2-D supervision pre-processing and the render loss (next row, SURVEY.md section 8f-4) -- */
 /* Model.process_GT_images (model/nerf.py:57-113): separable blur of n_img single-channel images [n_img][H][W]
  * (the reference reshapes [B,3,H,W] to [B*3,H,W]): replicate pad + cross-correlation with h_taps (HOST, ntaps odd,

@@ -44,6 +44,8 @@ SIGNATURES = {
     "jt_field_alpha": [_P, _P, _P, _P, ctypes.c_longlong, _P, _P, _P, _P, _P, _P, _P, _F, _I, _F, _P, _P],
     "jt_alpha_mask_build": [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P],
     "jt_resize_bilinear_cl": [_P, _I, _I, _I, _P, _I, _I, _P],
+    "jt_mc_count": [_P, _I, _I, _I, _F, _P, _P, _P],
+    "jt_mc_emit": [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P, _P, _P, _P],
     "jt_image_blur": [_P, _P, _P, _I, _I, _I, _P, _I, _P],
     "jt_edge_mask": [_P, _I, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P],
     "jt_render_loss_fwd": [_P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _F, _F, _P, _P, _P],
@@ -84,6 +86,8 @@ def lib():
         cdll.jt_wv_stage_bytes.restype = ctypes.c_longlong
         cdll.jt_edge_mask_ws_floats.argtypes = [_I, _I, _I]
         cdll.jt_edge_mask_ws_floats.restype = ctypes.c_longlong
+        cdll.jt_mc_scratch_bytes.argtypes = [_I, _I, _I]
+        cdll.jt_mc_scratch_bytes.restype = ctypes.c_longlong
         cdll.jt_launch_count.argtypes = []
         cdll.jt_launch_count.restype = ctypes.c_longlong
         _lib = cdll

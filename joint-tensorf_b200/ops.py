@@ -6,6 +6,8 @@ csrc/*.cu. Nothing in this file computes on the CPU or falls back to ATen
 operators for the hot path.
 """
 import contextlib
+import ctypes
+import math
 
 import torch
 
@@ -558,6 +560,54 @@ def alpha_mask_build(alpha_zyx, thres):
         check(_lib.lib().jt_alpha_mask_build(_p(alpha_zyx), w, h, d, float(thres), _p(tmp), _p(vol), _p(bits),
                                              _p(stats), _stream()), "jt_alpha_mask_build")
     return vol, bits, stats
+
+
+def marching_cubes(vol_zyx, level, lin, aabb):
+    """Marching cubes on a dense volume: vol_zyx [gz,gy,gx] fp32 (contiguous, CUDA), inside where value > level.
+    lin = the three device tables [x, y, z] with s = torch.linspace(0, 1, g); aabb [2,3] (host values). Lattice
+    point (i, j, k) is aabb[0]*(1-s) + aabb[1]*s, the dense_xyz of getDenseAlpha.
+    Returns (verts [V,3] fp32, faces [F,3] int32) on the volume's device; [0,3] tensors when nothing crosses.
+    One vertex per lattice edge whose ends straddle the level, interpolated linearly along the edge, so the
+    vertices are those of any marching cubes; the triangulation inside a cell comes from the project's generated
+    case table (csrc/gen_mc_tables.py) and may differ from PyMCubes or skimage. The mesh is closed where the
+    surface does not reach the volume's border, and normals point toward decreasing value. Order: vertices by the
+    linear index of the edge's lower end, then axis x < y < z; faces by cell, then table order. One 16-byte host
+    read of the counts sizes the outputs."""
+    if not isinstance(vol_zyx, torch.Tensor):
+        raise _lib.JtError("marching_cubes: the volume must be a tensor")
+    _need_cuda(vol_zyx, "volume")
+    if vol_zyx.dtype != torch.float32 or vol_zyx.dim() != 3 or not vol_zyx.is_contiguous():
+        raise _lib.JtError(f"marching_cubes: the volume must be a contiguous fp32 [gz,gy,gx] tensor, got "
+                           f"{vol_zyx.dtype} {tuple(vol_zyx.shape)}")
+    gz, gy, gx = vol_zyx.shape
+    if min(gx, gy, gz) < 2:
+        raise _lib.JtError(f"marching_cubes: every dimension must be >= 2, got {tuple(vol_zyx.shape)}")
+    lv = ctypes.c_float(float(level)).value
+    if not math.isfinite(lv):
+        raise _lib.JtError(f"marching_cubes: level {level!r} is not a finite fp32 value")
+    for t, g, name in zip(lin, (gx, gy, gz), "xyz"):
+        if t.device != vol_zyx.device or t.dtype != torch.float32 or t.shape != (g,) or not t.is_contiguous():
+            raise _lib.JtError(f"marching_cubes: lin_{name} must be a contiguous fp32 [{g}] tensor on the volume's device")
+    h_aabb = torch.as_tensor(aabb, dtype=torch.float32).reshape(6).tolist()
+    nbytes = int(_lib.lib().jt_mc_scratch_bytes(gx, gy, gz))
+    if nbytes < 0:
+        raise _lib.JtError(f"marching_cubes: grid {gx}x{gy}x{gz} has 2^31 or more points")
+    dev = vol_zyx.device
+    scratch = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+    totals = torch.empty((2,), dtype=torch.int64, device=dev)
+    with TIMER.span("mc_count"):
+        check(_lib.lib().jt_mc_count(_p(vol_zyx), gx, gy, gz, lv, _p(scratch), _p(totals), _stream()), "jt_mc_count")
+    nv, nf = totals.tolist()
+    if max(nv, nf) > 2 ** 31 - 1:
+        raise _lib.JtError(f"marching_cubes: {nv} vertices / {nf} triangles do not fit int32 indices")
+    verts = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+    faces = torch.empty((nf, 3), dtype=torch.int32, device=dev)
+    if nv > 0 or nf > 0:
+        with TIMER.span("mc_emit"):
+            check(_lib.lib().jt_mc_emit(_p(vol_zyx), gx, gy, gz, lv, _p(lin[0]), _p(lin[1]), _p(lin[2]),
+                                        floats(h_aabb), _p(scratch), _p(totals), _p(verts), _p(faces), _stream()),
+                  "jt_mc_emit")
+    return verts, faces
 
 
 def resize_bilinear_cl(x, h2, w2):

@@ -687,6 +687,32 @@ class B200_VMSplit(torch.nn.Module):
         return self._dense_alpha_zyx(gridSize).permute(2, 1, 0), dense_xyz
 
     @torch.no_grad()
+    def extract_mesh(self, level=0.005, gridSize=None):
+        """The field's geometry as a triangle mesh: marching cubes (ops.marching_cubes) on the dense alpha grid of
+        getDenseAlpha(gridSize) at alpha `level` (0.005 is TensoRF's exporter level). Honours the alpha mask and a
+        cached density blur exactly as getDenseAlpha does. Returns (verts [V,3] fp32 world coordinates, faces [F,3]
+        int32) on the module's device; normals point out of the high-alpha region."""
+        gridSize = self._grid if gridSize is None else [int(v) for v in gridSize]
+        return ops.marching_cubes(self._dense_alpha_zyx(gridSize), level, self._dense_tables(gridSize), self._h_aabb)
+
+    def export_mesh(self, path, level=0.005, gridSize=None):
+        """extract_mesh written to `path` as a binary little-endian PLY (float x, y, z per vertex; `list uchar int
+        vertex_indices` per face). Returns (V, F)."""
+        verts, faces = self.extract_mesh(level, gridSize)
+        v = verts.cpu().numpy().astype("<f4")
+        f = np.empty((faces.shape[0],), dtype=[("n", "u1"), ("i", "<i4", (3,))])
+        f["n"] = 3
+        f["i"] = faces.cpu().numpy()
+        header = ("ply\nformat binary_little_endian 1.0\n"
+                  f"element vertex {v.shape[0]}\nproperty float x\nproperty float y\nproperty float z\n"
+                  f"element face {f.shape[0]}\nproperty list uchar int vertex_indices\nend_header\n")
+        with open(path, "wb") as fh:
+            fh.write(header.encode("ascii"))
+            fh.write(v.tobytes())
+            fh.write(f.tobytes())
+        return v.shape[0], f.shape[0]
+
+    @torch.no_grad()
     def updateAlphaMask(self, gridSize=(200, 200, 200)):
         """tensorBase.py:635-661: dense alpha -> clamp -> max_pool3d(5) -> threshold -> mask + new aabb, four
         launches and one 28-byte read-back (the reference synchronises here too: boolean indexing, prints)."""
