@@ -90,11 +90,11 @@ class OverlappedGradSync:
         self.works = []
         self.bytes = 0
         self.enabled = True
-        # planes 0+1 | plane 2 | density with a collective after each launch (render.py). "auto": when it pays --
+        # planes 0+1 | plane 2 | density with a collective after each launch (scatter_schedule). "auto": when it pays --
         # 4 or more ranks and an appearance part that dominates the bucket (measured: N=8 cfg2_sh 3.21 -> 3.12 ms,
         # N=2 3.04 -> 3.04, N=2 cfg4 2.15 -> 2.29)
         self.split21 = split21
-        self.per_plane = per_plane        # one scatter launch + all-reduce per appearance plane (render.py)
+        self.per_plane = per_plane        # one scatter launch + all-reduce per appearance plane (scatter_schedule)
         self.reserve_sms = reserve_sms    # SMs the density scatter leaves to the collective running next to it
 
     def use_split21(self, n_app, n_total):
@@ -169,6 +169,38 @@ class OverlappedGradSync:
                         g = p.grad
                     self._reduce(g)
         self.wait()
+
+
+def scatter_schedule(sync, need_app, need_dens, need_rays, sizes, n_app, dens_resident):
+    """The render op's factor-gradient scatter launches, in order: (app, max_ctas, plane_mask, cut) each -- app 1 walks
+    the appearance factors, 0 the density factors; max_ctas and plane_mask are jt_vm_scatter_rays's launch form; after
+    the launch the flat gradient bucket is complete up to offset `cut`, handed to `sync.on_app_grads` (None: no cut).
+    sizes: numel of the bucket's tensors, appearance first; n_app: the appearance part; dens_resident: density-scatter
+    CTAs per SM. Without a synchroniser a frozen factor group is walked coordinate-only if the rays need a gradient."""
+    if sync is None:
+        return [(app, 0, 7, None) for app, need in ((1, need_app), (0, need_dens)) if need or need_rays]
+    if sync.per_plane:
+        # variant (OverlappedGradSync(per_plane=True)): the appearance planes are walked one launch per plane and
+        # each plane's gradients are all-reduced while the next launches run -- [plane 0] [plane 1] [plane 2 + the
+        # three lines] [density + basis_mat + head]. Measured at N = 2 (profiles/r02e): the exposed wait halves
+        # (0.21 -> 0.12 ms) but the non-persistent per-plane launches cost 0.11 ms more than they save.
+        return [(1, -80, 1, sizes[0]), (1, -80, 2, sizes[0] + sizes[1]), (1, -80, 4, n_app), (0, -80, 7, None)]
+    if sync.use_split21(n_app, sum(sizes)):
+        # data parallel, 4+ ranks with an appearance-dominated bucket: [appearance planes 0+1: one persistent
+        # launch] -> all-reduce of their 2/4 of the bucket starts -> [appearance plane 2] -> all-reduce of plane 2
+        # + the three lines -> [density scatter] -> all-reduce of the rest. The collectives get a 0.7 ms window
+        # (plane 2 + density) instead of the 0.4 ms of the density scatter alone, which at N = 8 is shorter than
+        # the 69 MB all-reduce itself; the two launches that run next to a collective use fixed 80-sample segments
+        # on a non-persistent grid, because NCCL's CTAs can only get onto an SM when scatter CTAs retire (a
+        # persistent wave holds every SM until its kernel ends). Measured (profiles/r02l_*, r02n8c_*): N = 8:
+        # exposed wait 0.36 -> 0.16 ms, the two scatters that share the SMs with a collective lose 0.10 ms, step
+        # 3.21 -> 3.12 ms; N = 2: 3.04 vs 3.04 ms; cfg4 at N = 2 gets slower (2.15 -> 2.29: its bucket is half
+        # density) -- hence use_split21.
+        return [(1, 0, 3, sizes[0] + sizes[1]), (1, -80, 4, n_app), (0, -80, 7, None)]
+    # 2 ranks / density-heavy buckets: the appearance part of the bucket is all-reduced while the density scatter
+    # runs (non-persistent grid, or a persistent wave on the 148 SMs but sync.reserve_sms left to the collective)
+    reserve = int(sync.reserve_sms)
+    return [(1, 0, 7, n_app), (0, (148 - reserve) * dens_resident if reserve > 0 else -80, 7, None)]
 
 
 def seed_all_ranks(seed):

@@ -23,8 +23,8 @@ kernels read them from `ray_off[N]` / `app_off[N]` and run persistent grids.
 """
 import torch
 
-from . import _lib, ops
-from ._lib import check, floats
+from . import _lib, ops, parallel
+from ._lib import check
 from .ops import FactorSet, TIMER, _p, _stream
 
 
@@ -67,103 +67,197 @@ class RenderCfg:
         self.__dict__.update(kw)
 
 
-def tc_supported(cfg, afs=None, raise_if_not=False, comps=None):
-    """The tensor-core heads are specialised for the shipped configurations: Blender = 3 x 48 appearance
-    components, app_dim 27, MLP_Fea (hidden 64, fea_pe = view_pe = 2) or SH shading."""
-    comps = list(afs.C) if afs is not None else (list(comps) if comps is not None else None)
-    c48 = comps is None or all(int(c) == 48 for c in comps)
-    ok = (cfg.shading == "MLP_Fea" and cfg.app_dim == 27 and cfg.hidden == 64 and cfg.fea_pe == 2 and
-          cfg.view_pe == 2 and c48)
-    ok = ok or (cfg.shading == "SH" and cfg.app_dim == 27 and c48)
-    # LLFF = 3 x 20 components, app_dim 20, MLP_Fea_WeakView (hidden 32, fea_pe = view_pe = 2): csrc/weakview_tc.cu
-    c20 = comps is None or all(int(c) == 20 for c in comps)
-    ok = ok or (cfg.shading == "MLP_Fea_WeakView" and cfg.app_dim == 20 and cfg.hidden == 32 and cfg.fea_pe == 2 and
-                cfg.view_pe == 2 and c20)
-    if not ok and raise_if_not:
-        raise _lib.JtError("head='tc' needs 3 x 48 appearance components, app_dim 27 and MLP_Fea (hidden 64, pe 2) or "
-                           "SH shading, or 3 x 20 components, app_dim 20 and MLP_Fea_WeakView (hidden 32, pe 2); "
-                           "use head='fp32'")
-    return ok
+class _HeadImpl:
+    """One implementation of the shading head on the compacted appearance samples. `forward` returns rgb [cap,4] and
+    keeps, as attributes, what its `backward` needs; `backward` writes dcomps [cap, sum C_app] (dtype `dcomps_dtype`)
+    for the appearance scatter and the basis_mat / head weight gradients into `g_basis` / `head_grads` (None: not
+    wanted)."""
+    dcomps_dtype = torch.float32
+
+    def __init__(self, cfg, afs, comp, aidx, rays_d, basis_w, params, a_count, cap):
+        self.cfg, self.afs, self.comp, self.aidx, self.rays_d = cfg, afs, comp, aidx, rays_d
+        self.basis_w, self.params, self.a_count, self.cap = basis_w, params, a_count, cap
+        self.dev = rays_d.device
+        self.shade_act = 2 if cfg.shading == "SH" else 1      # output activation jt_render_bwd differentiates
+
+    @classmethod
+    def supports(cls, shading, app_dim, hidden, fea_pe, view_pe, comps):
+        """The tensor-core heads are specialised for the shipped configurations (class attributes)."""
+        return (shading == cls.shading and app_dim == cls.app_dim and all(int(c) == cls.comps for c in comps) and
+                (cls.mlp is None or (hidden, fea_pe, view_pe) == cls.mlp))
+
+    def _wgrads(self, g_basis, head_grads):
+        """The tensor-core MLP heads write all seven weight gradients or none: a frozen group gets dropped scratch."""
+        if g_basis is None and head_grads is None:
+            return None
+        return (g_basis if g_basis is not None else torch.zeros_like(self.basis_w),
+                *(head_grads if head_grads is not None else [torch.zeros_like(t) for t in self.params]))
 
 
-class _Head:
-    """Forward/backward of the shading head on compacted appearance samples."""
+class _Fp32Head(_HeadImpl):
+    """Strict fp32 SIMT chain, any head: appearance gather -> basis_mat GEMM -> SH shading or PE + MLP GEMMs."""
+    consumed = False
 
-    @staticmethod
-    def forward(cfg, ws, feat, ldf, aidx, sidx, rays_d, a_count, cap, params, dev):
-        F, H = cfg.app_dim, cfg.hidden
+    def forward(self, train, basis_grad):
+        cfg, afs, comp, aidx, a_count, cap = self.cfg, self.afs, self.comp, self.aidx, self.a_count, self.cap
+        F, H, ldf, dev = cfg.app_dim, cfg.hidden, _r4(cfg.app_dim), self.dev
+        self.comps = torch.empty((cap, afs.ctot), device=dev)
+        ops.vm_gather_fwd(1, afs, comp.samp, aidx, a_count, cap, self.comps)
+        self.feat = feat = torch.empty((cap, ldf), device=dev)
+        ops.gemm_nt(self.comps, afs.ctot, self.basis_w, afs.ctot, 0, None, feat, ldf, None, 0, a_count, cap, F,
+                    afs.ctot, 0, name="basis_fwd")
         rgb = torch.empty((cap, 4), device=dev)
         if cfg.shading == "SH":
-            ops.sh_shade(0, feat, ldf, aidx, sidx, rays_d, cfg.n_samples, cfg.ndc, a_count, cap, rgb, None, None, 0)
+            ops.sh_shade(0, feat, ldf, aidx, comp.sidx, self.rays_d, cfg.n_samples, cfg.ndc, a_count, cap, rgb, None,
+                         None, 0)
             return rgb
-        w1, b1, w2, b2, w3, b3 = params
+        w1, b1, w2, b2, w3, b3 = self.params
         if cfg.shading == "MLP_Fea":
-            in_dim = F + 3 + 2 * cfg.fea_pe * F + 6 * cfg.view_pe
-            ldi = _r4(in_dim)
-            x = torch.empty((cap, ldi), device=dev)
+            self.in_dim = in_dim = F + 3 + 2 * cfg.fea_pe * F + 6 * cfg.view_pe
+            self.ldi = ldi = _r4(in_dim)
+            self.x = x = torch.empty((cap, ldi), device=dev)
             ops.pe_encode(0, F, cfg.fea_pe, cfg.view_pe, 0, cfg.fea_prog, cfg.view_prog, cfg.n_samples, cfg.ndc,
-                          feat, ldf, aidx, sidx, rays_d, a_count, cap, x, ldi)
-            h1 = torch.empty((cap, H), device=dev)
+                          feat, ldf, aidx, comp.sidx, self.rays_d, a_count, cap, x, ldi)
+            self.h1 = h1 = torch.empty((cap, H), device=dev)
             ops.gemm_nt(x, ldi, w1, in_dim, 0, b1, h1, H, None, 0, a_count, cap, H, in_dim, 1, name="mlp_l1_fwd")
-            h2 = torch.empty((cap, H), device=dev)
+            self.h2 = h2 = torch.empty((cap, H), device=dev)
             ops.gemm_nt(h1, H, w2, H, 0, b2, h2, H, None, 0, a_count, cap, H, H, 1, name="mlp_l2_fwd")
             ops.gemm_nt(h2, H, w3, H, 0, b3, rgb, 4, None, 0, a_count, cap, 3, H, 2, name="mlp_l3_fwd")
-            ws.update(x=x, ldi=ldi, in_dim=in_dim, h1=h1, h2=h2)
         elif cfg.shading == "MLP_Fea_WeakView":
-            in_dim = F + 2 * cfg.fea_pe * F
-            ldi = _r4(in_dim)
-            nv = 6 * cfg.view_pe
+            self.in_dim = in_dim = F + 2 * cfg.fea_pe * F
+            self.ldi = ldi = _r4(in_dim)
+            self.nv = nv = 6 * cfg.view_pe
             assert nv % 4 == 0, "view_pe must be even for the WeakView layout"
-            ldm = nv + H
-            x = torch.empty((cap, ldi), device=dev)
-            mid = torch.empty((cap, ldm), device=dev)
+            self.ldm = ldm = nv + H
+            self.x = x = torch.empty((cap, ldi), device=dev)
+            self.mid = mid = torch.empty((cap, ldm), device=dev)
             ops.pe_encode(0, F, cfg.fea_pe, cfg.view_pe, 1, cfg.fea_prog, cfg.view_prog, cfg.n_samples, cfg.ndc,
-                          feat, ldf, aidx, sidx, rays_d, a_count, cap, x, ldi, mid, ldm)
-            h1 = torch.empty((cap, H), device=dev)
+                          feat, ldf, aidx, comp.sidx, self.rays_d, a_count, cap, x, ldi, mid, ldm)
+            self.h1 = h1 = torch.empty((cap, H), device=dev)
             ops.gemm_nt(x, ldi, w1, in_dim, 0, b1, h1, H, None, 0, a_count, cap, H, in_dim, 1, name="mlp_l1_fwd")
             ops.gemm_nt(h1, H, w2, H, 0, b2, mid, ldm, None, 0, a_count, cap, H, H, 1, name="mlp_l2_fwd", y_off=nv)
             ops.gemm_nt(mid, ldm, w3, ldm, 0, b3, rgb, 4, None, 0, a_count, cap, 3, ldm, 2, name="mlp_l3_fwd")
-            ws.update(x=x, ldi=ldi, in_dim=in_dim, h1=h1, mid=mid, ldm=ldm, nv=nv)
         else:
             raise _lib.JtError(f"shading model {cfg.shading!r} is not implemented by the B200 path")
         return rgb
 
-    @staticmethod
-    def backward(cfg, ws, dout, feat, ldf, aidx, sidx, rays_d, a_count, cap, params, dev, wgrad=True):
-        """dout [cap,4] -> dfeat [cap, ldf]; returns (dfeat, param grads list). wgrad=False (frozen head): the weight
-        gradient GEMMs are skipped and the list is empty."""
-        F, H = cfg.app_dim, cfg.hidden
+    def backward(self, dout, dcomps, g_basis, head_grads):
+        if self.consumed:
+            raise _lib.JtError("second backward through the same render call: the strict-fp32 MLP head reuses its "
+                               "encoded-input buffer for the input gradient (2.6 GB at 4096 x 1000 samples); call "
+                               "forward again, or use head_precision='tc' / SH shading, whose backward is re-entrant")
+        cfg, afs, feat, a_count, cap, dev = self.cfg, self.afs, self.feat, self.a_count, self.cap, self.dev
+        F, H, ldf = cfg.app_dim, cfg.hidden, _r4(cfg.app_dim)
         dfeat = torch.empty((cap, ldf), device=dev)
         if cfg.shading == "SH":
-            ops.sh_shade(1, feat, ldf, aidx, sidx, rays_d, cfg.n_samples, cfg.ndc, a_count, cap, None, dout, dfeat, ldf)
-            return dfeat, []
-        w1, b1, w2, b2, w3, b3 = params
-        gw1, gb1, gw2, gb2, gw3, gb3 = [torch.zeros_like(t) for t in params] if wgrad else [None] * 6
-        x, ldi, in_dim, h1 = ws["x"], ws["ldi"], ws["in_dim"], ws["h1"]
-        dh2 = torch.empty((cap, H), device=dev)
-        dh1 = torch.empty((cap, H), device=dev)
-        if cfg.shading == "MLP_Fea":
-            h2 = ws["h2"]
-            if wgrad:
-                ops.gemm_tn(dout, 4, h2, H, a_count, cap, 3, H, gw3, H, gb3, name="mlp_l3_bwd_w")
-            ops.gemm_nt(dout, 4, w3, H, 1, None, dh2, H, h2, H, a_count, cap, H, 3, 0, name="mlp_l3_bwd_x")
+            ops.sh_shade(1, feat, ldf, self.aidx, self.comp.sidx, self.rays_d, cfg.n_samples, cfg.ndc, a_count, cap,
+                         None, dout, dfeat, ldf)
         else:
-            mid, ldm, nv = ws["mid"], ws["ldm"], ws["nv"]
-            if wgrad:
-                ops.gemm_tn(dout, 4, mid, ldm, a_count, cap, 3, ldm, gw3, ldm, gb3, name="mlp_l3_bwd_w")
-            ops.gemm_nt(dout, 4, w3, ldm, 1, None, dh2, H, mid, ldm, a_count, cap, H, 3, 0, name="mlp_l3_bwd_x",
-                        w_off=nv, mask_off=nv)
-        if wgrad:
-            ops.gemm_tn(dh2, H, h1, H, a_count, cap, H, H, gw2, H, gb2, name="mlp_l2_bwd_w")
-        ops.gemm_nt(dh2, H, w2, H, 1, None, dh1, H, h1, H, a_count, cap, H, H, 0, name="mlp_l2_bwd_x")
-        if wgrad:
-            ops.gemm_tn(dh1, H, x, ldi, a_count, cap, H, in_dim, gw1, in_dim, gb1, name="mlp_l1_bwd_w")
-        # the encoded input is dead after dW1: reuse its buffer for its own gradient
-        ops.gemm_nt(dh1, H, w1, in_dim, 1, None, x, ldi, None, 0, a_count, cap, in_dim, H, 0, name="mlp_l1_bwd_x")
-        mode = 0 if cfg.shading == "MLP_Fea" else 1
-        ops.pe_encode(1, F, cfg.fea_pe, cfg.view_pe, mode, cfg.fea_prog, cfg.view_prog, cfg.n_samples, cfg.ndc,
-                      feat, ldf, None, None, None, a_count, cap, dfeat, ldf, None, 0, x, ldi)
-        return dfeat, ([gw1, gb1, gw2, gb2, gw3, gb3] if wgrad else [])
+            self.consumed = True
+            w1, b1, w2, b2, w3, b3 = self.params
+            # the bucket views are zero-filled: the weight-gradient GEMMs write into them directly
+            gw1, gb1, gw2, gb2, gw3, gb3 = head_grads if head_grads is not None else [None] * 6
+            x, ldi, in_dim, h1 = self.x, self.ldi, self.in_dim, self.h1
+            dh2 = torch.empty((cap, H), device=dev)
+            dh1 = torch.empty((cap, H), device=dev)
+            # layer 3 reads h2 (MLP_Fea) or [view PE | h2] (WeakView, whose dh2 skips the view columns)
+            l3, ld3, off = (self.h2, H, 0) if cfg.shading == "MLP_Fea" else (self.mid, self.ldm, self.nv)
+            if gw3 is not None:
+                ops.gemm_tn(dout, 4, l3, ld3, a_count, cap, 3, ld3, gw3, ld3, gb3, name="mlp_l3_bwd_w")
+            ops.gemm_nt(dout, 4, w3, ld3, 1, None, dh2, H, l3, ld3, a_count, cap, H, 3, 0, name="mlp_l3_bwd_x",
+                        w_off=off, mask_off=off)
+            if gw2 is not None:
+                ops.gemm_tn(dh2, H, h1, H, a_count, cap, H, H, gw2, H, gb2, name="mlp_l2_bwd_w")
+            ops.gemm_nt(dh2, H, w2, H, 1, None, dh1, H, h1, H, a_count, cap, H, H, 0, name="mlp_l2_bwd_x")
+            if gw1 is not None:
+                ops.gemm_tn(dh1, H, x, ldi, a_count, cap, H, in_dim, gw1, in_dim, gb1, name="mlp_l1_bwd_w")
+            # the encoded input is dead after dW1: reuse its buffer for its own gradient
+            ops.gemm_nt(dh1, H, w1, in_dim, 1, None, x, ldi, None, 0, a_count, cap, in_dim, H, 0, name="mlp_l1_bwd_x")
+            ops.pe_encode(1, F, cfg.fea_pe, cfg.view_pe, int(cfg.shading != "MLP_Fea"), cfg.fea_prog, cfg.view_prog,
+                          cfg.n_samples, cfg.ndc, feat, ldf, None, None, None, a_count, cap, dfeat, ldf, None, 0, x, ldi)
+        if g_basis is not None:
+            ops.gemm_tn(dfeat, ldf, self.comps, afs.ctot, a_count, cap, F, afs.ctot, g_basis, afs.ctot, None,
+                        name="basis_bwd_w")
+        ops.gemm_nt(dfeat, ldf, self.basis_w, afs.ctot, 1, None, dcomps, afs.ctot, None, 0, a_count, cap, afs.ctot, F,
+                    0, name="basis_bwd_x")
+
+
+class _ShTcHead(_HeadImpl):
+    """tcgen05 SH head: appearance gather + basis_mat + SHRender in one kernel; bf16 dcomps (bf16 GEMM operands)."""
+    shading, app_dim, comps, mlp = "SH", 27, 48, None           # Blender: 3 x 48 components, app_dim 27
+    dcomps_dtype = torch.bfloat16
+
+    def forward(self, train, basis_grad):
+        cfg, cap = self.cfg, self.cap
+        rgb = torch.empty((cap, 4), device=self.dev)
+        self.feat = torch.empty((cap, 32), device=self.dev)       # feat 0..26 | 0 | view dir 28..30 | 0
+        # the staged component tile only feeds the basis_mat weight gradient
+        self.stage = ops.head_tc_stage(cap, self.dev) if train and basis_grad else None
+        ops.app_basis_sh_fwd_tc(cfg.tc_fwd_split, self.afs, self.comp.samp, self.aidx, self.comp.sidx, self.rays_d,
+                                cfg.n_samples, cfg.ndc, self.basis_w, self.a_count, cap, self.feat, rgb, self.stage)
+        return rgb
+
+    def backward(self, dout, dcomps, g_basis, head_grads):
+        # no staged component tile when basis_mat was frozen in the forward: no weight gradient either
+        ops.sh_bwd_tc(dout, self.feat, self.basis_w, self.a_count, self.cap, dcomps, self.stage,
+                      g_basis if self.stage is not None else None)
+
+
+class _MlpTcHead(_HeadImpl):
+    """tcgen05 MLP_Fea head: appearance gather + basis_mat, then the MLP; bf16 dcomps."""
+    shading, app_dim, comps, mlp = "MLP_Fea", 27, 48, (64, 2, 2)    # mlp: (hidden, fea_pe, view_pe)
+    dcomps_dtype = torch.bfloat16
+
+    def forward(self, train, basis_grad):
+        cfg, cap = self.cfg, self.cap
+        rgb = torch.empty((cap, 4), device=self.dev)
+        self.feat = torch.empty((cap, 32), device=self.dev)       # feat 0..26 | 0 | view dir 28..30 | 0
+        # the data backward reads the staged relu tiles as well as the component tile
+        self.stage = ops.head_tc_stage(cap, self.dev) if train else None
+        ops.app_basis_fwd_tc(cfg.tc_fwd_split, self.afs, self.comp.samp, self.aidx, self.comp.sidx, self.rays_d,
+                             cfg.n_samples, cfg.ndc, self.basis_w, self.a_count, cap, self.feat, self.stage)
+        # inference: fp16 operand tiles (one MMA per product, half the shared memory, two CTAs per SM); the
+        # training forward keeps the hi+lo bf16 split because its staged tiles feed the bf16 backward GEMMs
+        split = 3 if (not train and cfg.tc_infer_fp16 and cfg.tc_fwd_split == 2) else cfg.tc_fwd_split
+        ops.head_mlp_fwd_tc(split, self.feat, *self.params, self.a_count, cap, cfg.fea_prog, cfg.view_prog, rgb,
+                            self.stage)
+        return rgb
+
+    def backward(self, dout, dcomps, g_basis, head_grads):
+        w1, b1, w2, b2, w3, b3 = self.params
+        ops.head_bwd_tc(dout, self.feat, self.basis_w, w1, w2, w3, self.a_count, self.cap, self.cfg.fea_prog, dcomps,
+                        self.stage, self._wgrads(g_basis, head_grads))
+
+
+class _WeakViewTcHead(_HeadImpl):
+    """tcgen05 MLP_Fea_WeakView head (csrc/weakview_tc.cu): fp32 appearance gather, then basis_mat + PE + MLP."""
+    shading, app_dim, comps, mlp = "MLP_Fea_WeakView", 20, 20, (32, 2, 2)    # LLFF: 3 x 20 components
+
+    def forward(self, train, basis_grad):
+        cfg, cap = self.cfg, self.cap
+        comps = torch.empty((cap, self.afs.ctot), device=self.dev)   # the staged bf16 tile replaces it in the backward
+        ops.vm_gather_fwd(1, self.afs, self.comp.samp, self.aidx, self.a_count, cap, comps)
+        self.feat = torch.empty((cap, 32), device=self.dev)       # feat 0..19 | 0 | view dir 28..30 | 0
+        rgb = torch.empty((cap, 4), device=self.dev)
+        self.stage = ops.wv_stage(cap, self.dev) if train else None
+        ops.wv_head_fwd_tc(comps, self.aidx, self.comp.sidx, self.rays_d, cfg.n_samples, cfg.ndc, self.basis_w,
+                           *self.params, self.a_count, cap, cfg.fea_prog, cfg.view_prog, self.feat, rgb, self.stage)
+        return rgb
+
+    def backward(self, dout, dcomps, g_basis, head_grads):
+        w1, b1, w2, b2, w3, b3 = self.params
+        ops.wv_head_bwd_tc(dout, self.feat, self.basis_w, w1, w2, w3, self.a_count, self.cap, self.cfg.fea_prog,
+                           dcomps, self.stage, self._wgrads(g_basis, head_grads))
+
+
+def tc_head(shading, app_dim, hidden, fea_pe, view_pe, comps):
+    """The tensor-core head implementation covering this configuration, or None."""
+    return next((h for h in (_ShTcHead, _MlpTcHead, _WeakViewTcHead)
+                 if h.supports(shading, app_dim, hidden, fea_pe, view_pe, comps)), None)
+
+
+# VMRender.apply's inputs as ctx.needs_input_grad indexes them: cfg, rays_o, rays_d, aux, then these groups
+_RAYS, _DENS, _APP, _BASIS, _HEAD = slice(1, 3), slice(4, 10), slice(10, 16), slice(16, 17), slice(17, None)
 
 
 def _full_backward(cfg):
@@ -188,7 +282,8 @@ class VMRender(torch.autograd.Function):
         dev = rays_o.device
         rays_o = rays_o.detach().contiguous().float()
         rays_d = rays_d.detach().contiguous().float()
-        dens, app, basis_w, head = tensors[0:6], tensors[6:12], tensors[12], tensors[13:]
+        inputs = (cfg, rays_o, rays_d, aux) + tensors
+        dens, app, basis_w, head = inputs[_DENS], inputs[_APP], inputs[_BASIS][0], inputs[_HEAD]
         head = [t.detach().contiguous() for t in head]
         basis_w = basis_w.detach().contiguous()
         dfs = FactorSet([t.detach() for t in dens[:3]], [t.detach() for t in dens[3:]])
@@ -205,9 +300,15 @@ class VMRender(torch.autograd.Function):
                 dfs32, afs32 = dfs, afs
         N, S = rays_o.shape[0], cfg.n_samples
         F = cfg.app_dim
-        ldf = _r4(F)
         if basis_w.shape != (F, afs.ctot):
             raise _lib.JtError(f"basis_mat weight {tuple(basis_w.shape)} != ({F}, {afs.ctot})")
+        Head = _Fp32Head
+        if cfg.head == "tc":
+            Head = tc_head(cfg.shading, F, cfg.hidden, cfg.fea_pe, cfg.view_pe, afs.C)
+            if Head is None:
+                raise _lib.JtError("head='tc' needs 3 x 48 appearance components, app_dim 27 and MLP_Fea (hidden 64, "
+                                   "pe 2) or SH shading, or 3 x 20 components, app_dim 20 and MLP_Fea_WeakView (hidden "
+                                   "32, pe 2); use head='fp32'")
 
         comp = ops.march_compact(rays_o, rays_d, aux, cfg.ndc, S, cfg.h_geom, cfg.mask)
         cap = comp.cap
@@ -244,44 +345,8 @@ class VMRender(torch.autograd.Function):
             acap = max(int(a_count.item()), 1)
         cap_v, cap = cap, acap                    # from here on `cap` sizes the APPEARANCE stage; cap_v = N*S
 
-        ws = {}
-        comps = None
-        if cfg.head == "tc" and cfg.shading == "MLP_Fea_WeakView":
-            tc_supported(cfg, afs, raise_if_not=True)
-            comps = torch.empty((cap, afs.ctot), device=dev)
-            ops.vm_gather_fwd(1, afs, comp.samp, aidx, a_count, cap, comps)
-            feat = torch.empty((cap, 32), device=dev)             # feat 0..19 | 0 | view dir 28..30 | 0
-            rgb = torch.empty((cap, 4), device=dev)
-            ws["stage"] = ops.wv_stage(cap, dev) if train else None
-            ops.wv_head_fwd_tc(comps, aidx, comp.sidx, rays_d, S, cfg.ndc, basis_w, *head, a_count, cap, cfg.fea_prog,
-                               cfg.view_prog, feat, rgb, ws["stage"])
-            comps = None                                          # the staged bf16 tile replaces it in the backward
-        elif cfg.head == "tc":
-            tc_supported(cfg, afs, raise_if_not=True)
-            rgb = torch.empty((cap, 4), device=dev)
-            feat = torch.empty((cap, 32), device=dev)             # feat 0..26 | 0 | view dir 28..30 | 0
-            # SH: the staged component tile only feeds the basis_mat weight gradient (MLP_Fea: the data backward
-            # reads the staged relu tiles as well)
-            sh_stage = ctx.needs_input_grad[16] or _full_backward(cfg)
-            ws["stage"] = ops.head_tc_stage(cap, dev) if train and (cfg.shading != "SH" or sh_stage) else None
-            if cfg.shading == "SH":
-                ops.app_basis_sh_fwd_tc(cfg.tc_fwd_split, afs, comp.samp, aidx, comp.sidx, rays_d, S, cfg.ndc,
-                                        basis_w, a_count, cap, feat, rgb, ws["stage"])
-            else:
-                ops.app_basis_fwd_tc(cfg.tc_fwd_split, afs, comp.samp, aidx, comp.sidx, rays_d, S, cfg.ndc, basis_w,
-                                     a_count, cap, feat, ws["stage"])
-                # inference: fp16 operand tiles (one MMA per product, half the shared memory, two CTAs per SM); the
-                # training forward keeps the hi+lo bf16 split because its staged tiles feed the bf16 backward GEMMs
-                mlp_split = 3 if (not train and cfg.tc_infer_fp16 and cfg.tc_fwd_split == 2) else cfg.tc_fwd_split
-                ops.head_mlp_fwd_tc(mlp_split, feat, *head, a_count, cap, cfg.fea_prog, cfg.view_prog, rgb,
-                                    ws["stage"])
-        else:
-            comps = torch.empty((cap, afs.ctot), device=dev)
-            ops.vm_gather_fwd(1, afs, comp.samp, aidx, a_count, cap, comps)
-            feat = torch.empty((cap, ldf), device=dev)
-            ops.gemm_nt(comps, afs.ctot, basis_w, afs.ctot, 0, None, feat, ldf, None, 0, a_count, cap, F, afs.ctot, 0,
-                        name="basis_fwd")
-            rgb = _Head.forward(cfg, ws, feat, ldf, aidx, comp.sidx, rays_d, a_count, cap, head, dev)
+        h = Head(cfg, afs, comp, aidx, rays_d, basis_w, head, a_count, cap)
+        rgb = h.forward(train, any(ctx.needs_input_grad[_BASIS]) or _full_backward(cfg))
 
         rgb_pre = torch.empty((N, 3), device=dev)
         rgb_map = torch.empty((N, 3), device=dev)
@@ -292,12 +357,8 @@ class VMRender(torch.autograd.Function):
                                        int(cfg.white_bg), float(cfg.depth_bias), _p(rgb_pre), _p(rgb_map),
                                        _p(depth), _p(opacity), int(cap), _stream()), "jt_composite_fwd")
 
-        ctx.cfg, ctx.comp, ctx.dfs, ctx.afs, ctx.ws = cfg, comp, dfs32, afs32, ws
-        ctx.bufs = dict(rays_d=rays_d, sigfeat=sigfeat, weight=weight, trans=trans, app_off=app_off, aidx=aidx,
-                        app_of=app_of, comps=comps, feat=feat, rgb=rgb, rgb_pre=rgb_pre, basis_w=basis_w, head=head,
-                        a_count=a_count)
-        ctx.n_head = len(head)
-        ctx.acap = cap
+        ctx.cfg, ctx.comp, ctx.dfs, ctx.afs, ctx.head = cfg, comp, dfs32, afs32, h
+        ctx.bufs = dict(sigfeat=sigfeat, weight=weight, trans=trans, app_of=app_of, rgb=rgb, rgb_pre=rgb_pre)
         # version check only: the kernels read the parameters' storage directly, so an in-place update between
         # forward and backward (an optimizer step, load_state_dict) must raise as it does for the reference's ATen
         # nodes instead of silently differentiating the new values
@@ -312,19 +373,12 @@ class VMRender(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_rgb, g_depth, g_acc):
         lib = _lib.lib()
-        cfg, comp, dfs, afs, ws, b = ctx.cfg, ctx.comp, ctx.dfs, ctx.afs, ctx.ws, ctx.bufs
+        cfg, comp, dfs, afs, h, b = ctx.cfg, ctx.comp, ctx.dfs, ctx.afs, ctx.head, ctx.bufs
         _ = ctx.saved_tensors                                 # raises if a parameter was modified in place since forward
-        if ws.get("consumed"):
-            raise _lib.JtError("second backward through the same render call: the strict-fp32 MLP head reuses its "
-                               "encoded-input buffer for the input gradient (2.6 GB at 4096 x 1000 samples); call "
-                               "forward again, or use head_precision='tc' / SH shading, whose backward is re-entrant")
         dev = g_rgb.device
-        N, cap_v, cap = comp.n_rays, comp.cap, ctx.acap       # cap: appearance-stage capacity, cap_v = N*S
-        F = cfg.app_dim
-        ldf = _r4(F)
+        N, cap_v, cap = comp.n_rays, comp.cap, h.cap          # cap: appearance-stage capacity, cap_v = N*S
         g_rgb = g_rgb.contiguous().float()
         g_acc = g_acc.contiguous().float() if g_acc is not None else None
-        shade_act = 2 if cfg.shading == "SH" else 1
 
         dout = torch.empty((cap, 4), device=dev)
         dsig = torch.empty((cap_v,), device=dev)
@@ -333,25 +387,19 @@ class VMRender(torch.autograd.Function):
             check(lib.jt_render_bwd(_p(comp.ray_off), N, _p(b["sigfeat"]), _p(comp.dist), _p(b["weight"]),
                                     _p(b["trans"]), _p(b["app_of"]), _p(b["rgb"]), _p(b["rgb_pre"]), _p(g_rgb),
                                     _p(g_acc), float(cfg.density_shift), cfg.act, float(cfg.distance_scale),
-                                    int(cfg.white_bg), shade_act, _p(dout), _p(dsig), _p(dnorm), _stream()),
+                                    int(cfg.white_bg), h.shade_act, _p(dout), _p(dsig), _p(dnorm), _stream()),
                   "jt_render_bwd")
 
         if VMRender.debug_capture is not None:            # diagnostics (scripts/debug_cfg4_grad.py): per-sample gradients
             VMRender.debug_capture.update(dsig=dsig.clone(), dout=dout.clone(), count=comp.count.clone(),
                                           weight=b["weight"].clone(), trans=b["trans"].clone(), rgb=b["rgb"].clone(),
-                                          sigfeat=b["sigfeat"].clone(), a_count=b["a_count"].clone())
+                                          sigfeat=b["sigfeat"].clone(), a_count=h.a_count.clone())
 
-        # Only the gradients autograd asks for. Input order: cfg, rays_o, rays_d, aux, 6 density factors, 6 appearance
-        # factors, basis_mat, head parameters. With an active gradient synchroniser every rank runs the full backward,
+        # Only the gradients autograd asks for. With an active gradient synchroniser every rank runs the full backward,
         # so that all ranks issue the same collectives whatever their parameters' requires_grad.
         sync = cfg.grad_sync if _full_backward(cfg) else None      # None: world size 1, or inside `sync.paused()`
-        ng = ctx.needs_input_grad
-        if sync is not None:
-            need_rays = need_dens = need_app = need_basis = need_head = True
-        else:
-            need_rays, need_dens, need_app = ng[1] or ng[2], any(ng[4:10]), any(ng[10:16])
-            need_basis, need_head = ng[16], any(ng[17:])
-        need_wgrad = need_basis or need_head
+        need = [sync is not None or any(ctx.needs_input_grad[s]) for s in (_RAYS, _DENS, _APP, _BASIS, _HEAD)]
+        need_rays, need_dens, need_app, need_basis, need_head = need
 
         # One flat zero-filled bucket for every gradient this node produces (one memset; also the unit the
         # data-parallel all-reduce works on): [app planes, app lines | density planes, density lines | basis, head],
@@ -360,117 +408,38 @@ class VMRender(torch.autograd.Function):
         # still runs.
         shapes = ([p.shape for p in afs.planes] + [l.shape for l in afs.lines] if need_app else []) + \
                  ([p.shape for p in dfs.planes] + [l.shape for l in dfs.lines] if need_dens else []) + \
-                 ([b["basis_w"].shape] if need_basis else []) + ([t.shape for t in b["head"]] if need_head else [])
+                 ([h.basis_w.shape] if need_basis else []) + ([t.shape for t in h.params] if need_head else [])
         sizes = [int(torch.Size(s).numel()) for s in shapes]
         flat = torch.zeros((sum(sizes),), device=dev)
-        views, o = [], 0
-        for s, n in zip(shapes, sizes):
-            views.append(flat[o:o + n].view(s))
-            o += n
-        it = iter(views)
+        it = iter([v.view(s) for v, s in zip(flat.split(sizes), shapes)])
         gap, gal = ([next(it) for _ in range(3)], [next(it) for _ in range(3)]) if need_app else (None, None)
         gdp, gdl = ([next(it) for _ in range(3)], [next(it) for _ in range(3)]) if need_dens else (None, None)
         g_basis = next(it) if need_basis else None
-        head_grads = [next(it) for _ in b["head"]] if need_head else None
+        head_grads = [next(it) for _ in h.params] if need_head else None
         n_app = sum(sizes[0:6]) if need_app else 0
 
         d_o = torch.empty((N, 3), device=dev)
         d_d = torch.empty((N, 3), device=dev)
         with TIMER.span("ray_init"):
-            check(lib.jt_ray_init(_p(b["rays_d"]), _p(dnorm), N, _p(d_o), _p(d_d), _stream()), "jt_ray_init")
+            check(lib.jt_ray_init(_p(h.rays_d), _p(dnorm), N, _p(d_o), _p(d_d), _stream()), "jt_ray_init")
 
         # the head backward and dcomps feed the appearance scatter (factor or ray gradients) and the weight gradients
         dcomps = None
-        if need_app or need_rays or need_wgrad:
-            # the tensor-core heads produce all weight gradients or none: a frozen one gets scratch that is dropped
-            wgrads = None
-            if need_wgrad:
-                wgrads = (g_basis if need_basis else torch.zeros_like(b["basis_w"]),
-                          *(head_grads if need_head else [torch.zeros_like(t) for t in b["head"]]))
-            # tensor-core head: dcomps crosses HBM as bf16 (its GEMM operands are bf16 already)
-            wv_tc = cfg.head == "tc" and cfg.shading == "MLP_Fea_WeakView"
-            dcomps = torch.empty((cap, afs.ctot), device=dev,
-                                 dtype=torch.bfloat16 if (cfg.head == "tc" and not wv_tc) else torch.float32)
-            if wv_tc:
-                w1, b1, w2, b2, w3, b3 = b["head"]
-                ops.wv_head_bwd_tc(dout, b["feat"], b["basis_w"], w1, w2, w3, b["a_count"], cap, cfg.fea_prog, dcomps,
-                                   ws["stage"], wgrads)
-            elif cfg.head == "tc" and cfg.shading == "SH":
-                # no staged component tile when basis_mat was frozen in the forward: no weight gradient either
-                sh_gb = g_basis if (need_basis and ws["stage"] is not None) else None
-                ops.sh_bwd_tc(dout, b["feat"], b["basis_w"], b["a_count"], cap, dcomps, ws["stage"], sh_gb)
-            elif cfg.head == "tc":
-                w1, b1, w2, b2, w3, b3 = b["head"]
-                ops.head_bwd_tc(dout, b["feat"], b["basis_w"], w1, w2, w3, b["a_count"], cap, cfg.fea_prog, dcomps,
-                                ws["stage"], wgrads)
-            else:
-                dfeat, hg = _Head.backward(cfg, ws, dout, b["feat"], ldf, b["aidx"], comp.sidx, b["rays_d"],
-                                           b["a_count"], cap, b["head"], dev, wgrad=need_head)
-                if cfg.shading != "SH":
-                    ws["consumed"] = True
-                for dst, src in zip(head_grads or [], hg):
-                    dst.copy_(src)
-                if need_basis:
-                    ops.gemm_tn(dfeat, ldf, b["comps"], afs.ctot, b["a_count"], cap, F, afs.ctot, g_basis, afs.ctot,
-                                None, name="basis_bwd_w")
-                ops.gemm_nt(dfeat, ldf, b["basis_w"], afs.ctot, 1, None, dcomps, afs.ctot, None, 0, b["a_count"], cap,
-                            afs.ctot, F, 0, name="basis_bwd_x")
-        # a frozen factor group is walked coordinate-only (no factor gradients) when the rays need a gradient
-        if sync is None:
-            if need_app or need_rays:
-                ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
-                                    cfg.n_samples, cfg.h_inv, d_o, d_d)
-            if need_dens or need_rays:
-                ops.vm_scatter_rays(0, dfs, gdp, gdl, comp.samp, None, comp.sidx, comp.count, cap_v, dsig,
-                                    cfg.n_samples, cfg.h_inv, d_o, d_d)
-        elif getattr(sync, "per_plane", False):
-            # variant (OverlappedGradSync(per_plane=True)): the appearance planes are walked one launch per plane and
-            # each plane's gradients are all-reduced while the next launches run -- [plane 0] [plane 1] [plane 2 + the
-            # three lines] [density + basis_mat + head]. Measured at N = 2 (profiles/r02e): the exposed wait halves
-            # (0.21 -> 0.12 ms) but the non-persistent per-plane launches cost 0.11 ms more than they save.
-            o = 0
-            for i in range(3):
-                ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
-                                    cfg.n_samples, cfg.h_inv, d_o, d_d, max_ctas=-80, plane_mask=1 << i)
-                end = o + sizes[i] if i < 2 else n_app
-                sync.on_app_grads(flat[o:end])
-                o = end
-            ops.vm_scatter_rays(0, dfs, gdp, gdl, comp.samp, None, comp.sidx, comp.count, cap_v, dsig, cfg.n_samples,
-                                cfg.h_inv, d_o, d_d, max_ctas=-80)
-            sync.on_rest(flat[n_app:])
-        elif sync.use_split21(n_app, flat.numel()):
-            # data parallel, 4+ ranks with an appearance-dominated bucket: [appearance planes 0+1: one persistent launch] -> all-reduce of their 2/4 of the
-            # bucket starts -> [appearance plane 2] -> all-reduce of plane 2 + the three lines -> [density scatter] ->
-            # all-reduce of the rest. The collectives get a 0.7 ms window (plane 2 + density) instead of the 0.4 ms of the
-            # density scatter alone, which at N = 8 is shorter than the 69 MB all-reduce itself; the two launches that run
-            # next to a collective use fixed 80-sample segments on a non-persistent grid, because NCCL's CTAs can only
-            # get onto an SM when scatter CTAs retire (a persistent wave holds every SM until its kernel ends).
-            # Measured (profiles/r02l_*, r02n8c_*): N = 8: exposed wait 0.36 -> 0.16 ms, the two scatters that share the
-            # SMs with a collective lose 0.10 ms, step 3.21 -> 3.12 ms; N = 2: 3.04 vs 3.04 ms; cfg4 at N = 2 gets slower
-            # (2.15 -> 2.29: its bucket is half density) -- hence OverlappedGradSync.use_split21.
-            ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
-                                cfg.n_samples, cfg.h_inv, d_o, d_d, plane_mask=3)
-            n01 = sizes[0] + sizes[1]
-            sync.on_app_grads(flat[:n01])
-            ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
-                                cfg.n_samples, cfg.h_inv, d_o, d_d, max_ctas=-80, plane_mask=4)
-            sync.on_app_grads(flat[n01:n_app])
-            ops.vm_scatter_rays(0, dfs, gdp, gdl, comp.samp, None, comp.sidx, comp.count, cap_v, dsig, cfg.n_samples,
-                                cfg.h_inv, d_o, d_d, max_ctas=-80)
+        if need_app or need_rays or need_basis or need_head:
+            dcomps = torch.empty((cap, afs.ctot), device=dev, dtype=h.dcomps_dtype)
+            h.backward(dout, dcomps, g_basis, head_grads)
+        o = 0
+        for app, max_ctas, plane_mask, cut in parallel.scatter_schedule(sync, need_app, need_dens, need_rays, sizes,
+                                                                        n_app, 4 if dfs.C[0] == 16 else 3):
+            fs, gp, gl, slot, n_dev, n_max, gin = ((afs, gap, gal, h.aidx, h.a_count, cap, dcomps) if app else
+                                                   (dfs, gdp, gdl, None, comp.count, cap_v, dsig))
+            ops.vm_scatter_rays(app, fs, gp, gl, comp.samp, slot, comp.sidx, n_dev, n_max, gin, cfg.n_samples,
+                                cfg.h_inv, d_o, d_d, max_ctas=max_ctas, plane_mask=plane_mask)
+            if cut is not None:
+                sync.on_app_grads(flat[o:cut])
+                o = cut
+        if sync is not None:
             # the current stream waits here for all reductions: whatever autograd does with the views next (hand
-            # them to p.grad, clone them, feed the adjoint blur) sees the cross-rank sums
-            sync.on_rest(flat[n_app:])
-        else:
-            # 2 ranks / density-heavy buckets: the appearance part of the bucket is all-reduced while the density
-            # scatter runs (non-persistent grid, or a persistent wave that leaves sync.reserve_sms SMs to the collective)
-            ops.vm_scatter_rays(1, afs, gap, gal, comp.samp, b["aidx"], comp.sidx, b["a_count"], cap, dcomps,
-                                cfg.n_samples, cfg.h_inv, d_o, d_d)
-            sync.on_app_grads(flat[:n_app])
-            reserve = int(getattr(sync, "reserve_sms", 0))
-            resident = 4 if dfs.C[0] == 16 else 3
-            ops.vm_scatter_rays(0, dfs, gdp, gdl, comp.samp, None, comp.sidx, comp.count, cap_v, dsig, cfg.n_samples,
-                                cfg.h_inv, d_o, d_d, max_ctas=((148 - reserve) * resident if reserve > 0 else -80))
-            # the current stream waits here for both reductions: whatever autograd does with the views next (hand
             # them to p.grad, clone them, feed the adjoint blur) sees the cross-rank sums
             sync.on_rest(flat[n_app:])
 
@@ -478,7 +447,7 @@ class VMRender(torch.autograd.Function):
         gapn, galn = FactorSet.grads_as_nchw(gap, gal) if need_app else ([None] * 3, [None] * 3)
         VMRender.last_grad_bucket = flat
         return (None, d_o if need_rays else None, d_d if need_rays else None, None, *gdpn, *gdln, *gapn, *galn, g_basis,
-                *(head_grads if need_head else [None] * ctx.n_head))
+                *(head_grads if need_head else [None] * len(h.params)))
 
 
 VMRender.last_grad_bucket = None

@@ -17,7 +17,7 @@ import torch.nn.functional as F
 from . import _lib, ops
 from ._lib import floats, ints
 from .ops import MAT_MODE, VEC_MODE
-from .render import RenderCfg, VMRender
+from .render import RenderCfg, VMRender, tc_head
 
 CL = torch.channels_last
 
@@ -629,10 +629,8 @@ class B200_VMSplit(torch.nn.Module):
         """True when the tcgen05 shading-head kernels cover this configuration (what head_precision="auto" picks):
         3 x 48 appearance components with app_dim 27 and MLP_Fea (hidden 64, pe 2) or SH shading (Blender configs), or
         3 x 20 components with app_dim 20 and MLP_Fea_WeakView (hidden 32, pe 2) (the LLFF config)."""
-        from .render import tc_supported
-        cfg = RenderCfg(shading=self.shadingMode, app_dim=int(self.app_dim), fea_pe=int(self.fea_pe),
-                        view_pe=int(self.view_pe), hidden=int(self.featureC))
-        return tc_supported(cfg, comps=self.app_n_comp)
+        return tc_head(self.shadingMode, int(self.app_dim), int(self.featureC), int(self.fea_pe), int(self.view_pe),
+                       self.app_n_comp) is not None
 
     def _check_opt(self, opt):
         arch = opt.arch
