@@ -344,6 +344,16 @@ int jt_mc_count(const float* vol, int gx, int gy, int gz, float level, void* scr
 int jt_mc_emit(const float* vol, int gx, int gy, int gz, float level, const float* lin_x, const float* lin_y,
                const float* lin_z, const float* h_aabb, const void* scratch, const long long* totals, float* verts,
                int* faces, cudaStream_t stream);
+/* Vertex normals of that mesh: normals [V][3] fp32 in jt_mc_emit's vertex order, from the scratch jt_mc_count left
+ * for the same vol, grid and level (arguments as jt_mc_emit; it writes nothing when V or F exceeds INT32_MAX).
+ * With c_a(i) the lattice coordinate above, the gradient at lattice point i along axis a is
+ * (v[i+1] - v[i-1]) / (c_a(i+1) - c_a(i-1)), one-sided at the border ((v[1] - v[0]) / (c(1) - c(0)) and the same at
+ * the top end). The normal of the vertex on edge p0 -> p1 is -normalize((1-t) g(p0) + t g(p1)) with jt_mc_emit's
+ * fp32 t, (0,0,0) when that vector is zero: it points toward decreasing value, as the face winding does. One warp
+ * per 32-point chunk with crossings, no atomics: the output is deterministic. */
+int jt_mc_normals(const float* vol, int gx, int gy, int gz, float level, const float* lin_x, const float* lin_y,
+                  const float* lin_z, const float* h_aabb, const void* scratch, const long long* totals,
+                  float* normals, cudaStream_t stream);
 
 /* ---- 2-D supervision pre-processing and the render loss (next row, SURVEY.md section 8f-4) -- */
 /* Model.process_GT_images (model/nerf.py:57-113): separable blur of n_img single-channel images [n_img][H][W]

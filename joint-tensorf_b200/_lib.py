@@ -46,6 +46,7 @@ SIGNATURES = {
     "jt_resize_bilinear_cl": [_P, _I, _I, _I, _P, _I, _I, _P],
     "jt_mc_count": [_P, _I, _I, _I, _F, _P, _P, _P],
     "jt_mc_emit": [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P, _P, _P, _P],
+    "jt_mc_normals": [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P, _P, _P],
     "jt_image_blur": [_P, _P, _P, _I, _I, _I, _P, _I, _P],
     "jt_edge_mask": [_P, _I, _I, _I, _I, _F, _P, _P, _P, _P, _P, _P],
     "jt_render_loss_fwd": [_P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _F, _F, _P, _P, _P],

@@ -10,6 +10,8 @@
 //   emit      one warp per chunk, chunks without crossings skipped: vertex id = tile base + chunk offset + popc of
 //             the chunk's bits below the lane; triangles of the non-empty cells look up the ids of edges owned by
 //             neighbouring points the same way.
+//   normals   (optional, after classify + scan) the same walk over chunks with crossings: per vertex the volume
+//             gradient at both ends of its edge (central differences), blended with emit's t, negated, normalised.
 // Scratch: 20 bytes per chunk of 32 points + 24 bytes per tile (jt_mc_scratch_bytes).
 #include <climits>
 
@@ -240,6 +242,76 @@ __global__ void __launch_bounds__(kMcThreads) mc_emit_kernel(const float* __rest
     }
 }
 
+// Volume gradient at lattice point p = (x, y, z) in world units: central difference (v[i+1] - v[i-1]) /
+// (c(i+1) - c(i-1)) per axis, one-sided at the grid's border. fp32, no contraction: the same value wherever it is
+// evaluated.
+__device__ __forceinline__ void mc_grad(const float* __restrict__ vol, const McEmitArgs& A, int p, const int idx[3],
+                                        const int stride[3], float g[3]) {
+    const int dims[3] = {A.gx, A.gy, A.gz};
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const int lo = idx[a] > 0 ? idx[a] - 1 : idx[a], hi = idx[a] + 1 < dims[a] ? idx[a] + 1 : idx[a];
+        const float dv = __fsub_rn(__ldg(vol + p + (hi - idx[a]) * stride[a]), __ldg(vol + p + (lo - idx[a]) * stride[a]));
+        g[a] = __fdiv_rn(dv, __fsub_rn(mc_coord(A, a, hi), mc_coord(A, a, lo)));
+    }
+}
+
+// One warp per chunk with crossing edges, vertex ids as in mc_emit_kernel. Normal = -normalize((1-t) g(p0) + t g(p1))
+// with emit's fp32 t; (0,0,0) when that vector is zero. Scaled by its largest component before the length, so small
+// gradients neither underflow nor lose precision.
+__global__ void __launch_bounds__(kMcThreads) mc_normals_kernel(const float* __restrict__ vol, McEmitArgs A, McScratch S,
+                                                                const long long* __restrict__ totals,
+                                                                float* __restrict__ normals) {
+    if (totals[0] > INT_MAX || totals[1] > INT_MAX) return;      // the caller cannot have allocated the output
+    const int lane = threadIdx.x & 31;
+    const int sy = A.gx, sz = A.gx * A.gy, n = sz * A.gz;
+    const int nchunks = (n + 31) >> 5;
+    const unsigned below = (1u << lane) - 1u;
+    for (int chunk = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; chunk < nchunks;
+         chunk += (gridDim.x * blockDim.x) >> 5) {
+        const uint4 b = S.bits[chunk];
+        if ((b.x | b.y | b.z) == 0) continue;
+        const int own = ((b.x >> lane) & 1) | (((b.y >> lane) & 1) << 1) | (((b.z >> lane) & 1) << 2);
+        if (!own) continue;
+        const int p = chunk * 32 + lane;
+        const int x = p % A.gx, r = p / A.gx, y = r % A.gy, z = r / A.gy;
+        int id = (int)S.tile_base[chunk / kMcTileChunks].x + (int)(S.loc[chunk] & 0xFFFFu) + __popc(b.x & below) +
+                 __popc(b.y & below) + __popc(b.z & below);
+        const float v0 = __ldg(vol + p);
+        const int idx[3] = {x, y, z}, stride[3] = {1, sy, sz};
+        float g0[3];
+        mc_grad(vol, A, p, idx, stride, g0);
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            if (!((own >> a) & 1)) continue;
+            const float v1 = __ldg(vol + p + stride[a]);
+            const float t = __fdiv_rn(__fsub_rn(A.level, v0), __fsub_rn(v1, v0));
+            int idx1[3] = {x, y, z};
+            ++idx1[a];
+            float g1[3];
+            mc_grad(vol, A, p + stride[a], idx1, stride, g1);
+            const float s = __fsub_rn(1.0f, t);
+            float q[3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) q[c] = __fadd_rn(__fmul_rn(s, g0[c]), __fmul_rn(t, g1[c]));
+            const float m = fmaxf(fabsf(q[0]), fmaxf(fabsf(q[1]), fabsf(q[2])));
+            float nrm[3] = {0.0f, 0.0f, 0.0f};
+            if (m > 0.0f) {
+#pragma unroll
+                for (int c = 0; c < 3; ++c) q[c] = __fdiv_rn(q[c], m);
+                const float len = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(q[0], q[0]), __fmul_rn(q[1], q[1])),
+                                                       __fmul_rn(q[2], q[2])));
+#pragma unroll
+                for (int c = 0; c < 3; ++c) nrm[c] = -__fdiv_rn(q[c], len);
+            }
+            normals[3LL * id] = nrm[0];
+            normals[3LL * id + 1] = nrm[1];
+            normals[3LL * id + 2] = nrm[2];
+            ++id;
+        }
+    }
+}
+
 }  // namespace jt
 
 using namespace jt;
@@ -266,6 +338,22 @@ extern "C" int jt_mc_count(const float* vol, int gx, int gy, int gz, float level
     JT_RETURN_LAUNCH();
 }
 
+// Launch set-up shared by the two per-vertex passes: lattice description and a persistent grid of warps over chunks.
+static McEmitArgs mc_args(int gx, int gy, int gz, float level, const float* lin_x, const float* lin_y,
+                          const float* lin_z, const float* h_aabb) {
+    McEmitArgs A;
+    A.lin[0] = lin_x; A.lin[1] = lin_y; A.lin[2] = lin_z;
+    for (int a = 0; a < 3; ++a) { A.a0[a] = h_aabb[a]; A.a1[a] = h_aabb[3 + a]; }
+    A.gx = gx; A.gy = gy; A.gz = gz; A.level = level;
+    return A;
+}
+
+static int mc_chunk_grid(long long n) {
+    const long long warps = (n + 31) / 32;
+    const long long want = (warps + 7) / 8;
+    return (int)(want < (long long)kNumSMs * 8 ? want : (long long)kNumSMs * 8);
+}
+
 extern "C" int jt_mc_emit(const float* vol, int gx, int gy, int gz, float level, const float* lin_x,
                           const float* lin_y, const float* lin_z, const float* h_aabb, const void* scratch,
                           const long long* totals, float* verts, int* faces, cudaStream_t stream) {
@@ -273,14 +361,21 @@ extern "C" int jt_mc_emit(const float* vol, int gx, int gy, int gz, float level,
     JT_CHECK_ARG(mc_grid_ok(gx, gy, gz) && (reinterpret_cast<uintptr_t>(scratch) & 15) == 0);
     const long long n = (long long)gx * gy * gz;
     McScratch S = mc_scratch(const_cast<void*>(scratch), mc_tiles(n));
-    McEmitArgs A;
-    A.lin[0] = lin_x; A.lin[1] = lin_y; A.lin[2] = lin_z;
-    for (int a = 0; a < 3; ++a) { A.a0[a] = h_aabb[a]; A.a1[a] = h_aabb[3 + a]; }
-    A.gx = gx; A.gy = gy; A.gz = gz; A.level = level;
-    const long long warps = (n + 31) / 32;
-    const long long want = (warps + 7) / 8;
-    const int grid = (int)(want < (long long)kNumSMs * 8 ? want : (long long)kNumSMs * 8);
-    mc_emit_kernel<<<grid, kMcThreads, 0, stream>>>(vol, A, S, totals, verts, faces);
+    mc_emit_kernel<<<mc_chunk_grid(n), kMcThreads, 0, stream>>>(
+        vol, mc_args(gx, gy, gz, level, lin_x, lin_y, lin_z, h_aabb), S, totals, verts, faces);
+    ++g_launches;
+    JT_RETURN_LAUNCH();
+}
+
+extern "C" int jt_mc_normals(const float* vol, int gx, int gy, int gz, float level, const float* lin_x,
+                             const float* lin_y, const float* lin_z, const float* h_aabb, const void* scratch,
+                             const long long* totals, float* normals, cudaStream_t stream) {
+    JT_CHECK_ARG(vol && lin_x && lin_y && lin_z && h_aabb && scratch && totals && normals);
+    JT_CHECK_ARG(mc_grid_ok(gx, gy, gz) && (reinterpret_cast<uintptr_t>(scratch) & 15) == 0);
+    const long long n = (long long)gx * gy * gz;
+    McScratch S = mc_scratch(const_cast<void*>(scratch), mc_tiles(n));
+    mc_normals_kernel<<<mc_chunk_grid(n), kMcThreads, 0, stream>>>(
+        vol, mc_args(gx, gy, gz, level, lin_x, lin_y, lin_z, h_aabb), S, totals, normals);
     ++g_launches;
     JT_RETURN_LAUNCH();
 }

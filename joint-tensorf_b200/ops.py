@@ -562,7 +562,7 @@ def alpha_mask_build(alpha_zyx, thres):
     return vol, bits, stats
 
 
-def marching_cubes(vol_zyx, level, lin, aabb):
+def marching_cubes(vol_zyx, level, lin, aabb, normals=False):
     """Marching cubes on a dense volume: vol_zyx [gz,gy,gx] fp32 (contiguous, CUDA), inside where value > level.
     lin = the three device tables [x, y, z] with s = torch.linspace(0, 1, g); aabb [2,3] (host values). Lattice
     point (i, j, k) is aabb[0]*(1-s) + aabb[1]*s, the dense_xyz of getDenseAlpha.
@@ -572,7 +572,11 @@ def marching_cubes(vol_zyx, level, lin, aabb):
     case table (csrc/gen_mc_tables.py) and may differ from PyMCubes or skimage. The mesh is closed where the
     surface does not reach the volume's border, and normals point toward decreasing value. Order: vertices by the
     linear index of the edge's lower end, then axis x < y < z; faces by cell, then table order. One 16-byte host
-    read of the counts sizes the outputs."""
+    read of the counts sizes the outputs.
+    normals=True also returns normals [V,3] fp32 (jt_mc_normals): per vertex -normalize((1-t) g(p0) + t g(p1)), g the
+    volume's central-difference gradient in world units at the two ends of the vertex's edge (one-sided at the
+    border), t the vertex's position on the edge; (0,0,0) where that vector is zero. They point toward decreasing
+    value, as the faces do."""
     if not isinstance(vol_zyx, torch.Tensor):
         raise _lib.JtError("marching_cubes: the volume must be a tensor")
     _need_cuda(vol_zyx, "volume")
@@ -607,7 +611,15 @@ def marching_cubes(vol_zyx, level, lin, aabb):
             check(_lib.lib().jt_mc_emit(_p(vol_zyx), gx, gy, gz, lv, _p(lin[0]), _p(lin[1]), _p(lin[2]),
                                         floats(h_aabb), _p(scratch), _p(totals), _p(verts), _p(faces), _stream()),
                   "jt_mc_emit")
-    return verts, faces
+    if not normals:
+        return verts, faces
+    nrm = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+    if nv > 0:
+        with TIMER.span("mc_normals"):
+            check(_lib.lib().jt_mc_normals(_p(vol_zyx), gx, gy, gz, lv, _p(lin[0]), _p(lin[1]), _p(lin[2]),
+                                           floats(h_aabb), _p(scratch), _p(totals), _p(nrm), _stream()),
+                  "jt_mc_normals")
+    return verts, faces, nrm
 
 
 def resize_bilinear_cl(x, h2, w2):

@@ -21,6 +21,8 @@ coordinate-only, and allocates no factor-gradient bucket.
 Sample counts (V valid samples, A appearance samples) stay on the device; the
 kernels read them from `ray_off[N]` / `app_off[N]` and run persistent grids.
 """
+import copy
+
 import torch
 
 from . import _lib, ops, parallel
@@ -256,6 +258,38 @@ def tc_head(shading, app_dim, hidden, fea_pe, view_pe, comps):
                  if h.supports(shading, app_dim, hidden, fea_pe, view_pe, comps)), None)
 
 
+def head_class(cfg, comps):
+    """The head implementation a call with `cfg` runs on appearance components `comps`: the tensor-core head under
+    cfg.head == "tc" (an error when none covers the configuration), else the strict fp32 chain."""
+    if cfg.head != "tc":
+        return _Fp32Head
+    Head = tc_head(cfg.shading, cfg.app_dim, cfg.hidden, cfg.fea_pe, cfg.view_pe, comps)
+    if Head is None:
+        raise _lib.JtError("head='tc' needs 3 x 48 appearance components, app_dim 27 and MLP_Fea (hidden 64, "
+                           "pe 2) or SH shading, or 3 x 20 components, app_dim 20 and MLP_Fea_WeakView (hidden "
+                           "32, pe 2); use head='fp32'")
+    return Head
+
+
+def shade_points(cfg, afs, xyz_norm, viewdirs, basis_w, params):
+    """Colour of the field at n points: rgb [n,3] of the head head_class(cfg, afs.C) runs, for normalised coordinates
+    xyz_norm [n,3] (zero components outside [-1,1], as grid_sample's zero padding) and view directions viewdirs [n,3]
+    taken as given (no normalisation). Each point is a one-sample ray whose sample is its own appearance sample, so
+    the head's no-grad forward shades it exactly as it shades a render sample; rows are independent of each other.
+    cfg supplies the head fields (shading, sizes, head, tc_fwd_split, tc_infer_fp16, PE progress)."""
+    n = xyz_norm.shape[0]
+    dev = xyz_norm.device
+    Head = head_class(cfg, afs.C)
+    cfg = copy.copy(cfg)
+    cfg.n_samples, cfg.ndc = 1, False
+    comp = ops.Compacted()
+    comp.samp = ops._samp_from_xyz(xyz_norm)
+    comp.sidx = torch.arange(max(n, 1), device=dev, dtype=torch.int32)
+    count = torch.full((1,), n, device=dev, dtype=torch.int32)
+    h = Head(cfg, afs, comp, comp.sidx, viewdirs.contiguous().float(), basis_w, params, count, max(n, 1))
+    return h.forward(train=False, basis_grad=False)[:n, :3]
+
+
 # VMRender.apply's inputs as ctx.needs_input_grad indexes them: cfg, rays_o, rays_d, aux, then these groups
 _RAYS, _DENS, _APP, _BASIS, _HEAD = slice(1, 3), slice(4, 10), slice(10, 16), slice(16, 17), slice(17, None)
 
@@ -302,13 +336,7 @@ class VMRender(torch.autograd.Function):
         F = cfg.app_dim
         if basis_w.shape != (F, afs.ctot):
             raise _lib.JtError(f"basis_mat weight {tuple(basis_w.shape)} != ({F}, {afs.ctot})")
-        Head = _Fp32Head
-        if cfg.head == "tc":
-            Head = tc_head(cfg.shading, F, cfg.hidden, cfg.fea_pe, cfg.view_pe, afs.C)
-            if Head is None:
-                raise _lib.JtError("head='tc' needs 3 x 48 appearance components, app_dim 27 and MLP_Fea (hidden 64, "
-                                   "pe 2) or SH shading, or 3 x 20 components, app_dim 20 and MLP_Fea_WeakView (hidden "
-                                   "32, pe 2); use head='fp32'")
+        Head = head_class(cfg, afs.C)
 
         comp = ops.march_compact(rays_o, rays_d, aux, cfg.ndc, S, cfg.h_geom, cfg.mask)
         cap = comp.cap

@@ -17,7 +17,7 @@ import torch.nn.functional as F
 from . import _lib, ops
 from ._lib import floats, ints
 from .ops import MAT_MODE, VEC_MODE
-from .render import RenderCfg, VMRender, tc_head
+from .render import RenderCfg, VMRender, shade_points, tc_head
 
 CL = torch.channels_last
 
@@ -537,6 +537,50 @@ class B200_VMSplit(torch.nn.Module):
                                       self.kernel_density if self.c2f_mode is not None else None)
         return ops.FactorSet([p.detach() for p in planes], [l.detach() for l in lines])
 
+    def _app_factorset(self):
+        """Appearance factors as the last forward saw them (blurred with the cached colour kernel, batBase.py:37)."""
+        planes, lines = self._blurred(self.app_plane, self.app_line,
+                                      self.kernel_color if self.c2f_mode is not None else None)
+        return ops.FactorSet([p.detach() for p in planes], [l.detach() for l in lines])
+
+    _RGB_CHUNK = 1 << 20      # points per head call: bounds the strict-fp32 head's ~2 KB per point of buffers
+
+    @torch.no_grad()
+    def compute_rgb(self, xyz_locs, viewdirs):
+        """Colour of the field at world points xyz_locs [..., 3] seen along viewdirs [..., 3] (or one [3] for all
+        points): rgb [..., 3], the reference's renderModule(pts, viewdirs, compute_appfeature(pts)) as a no-grad
+        forward computes it. The head is the one forward picks (head_precision, tc_fwd_split, tc_infer_fp16,
+        factor_storage); the appearance factors are blurred with the colour kernel the last forward cached, so
+        colour and compute_alpha's geometry come from the same field state; the PE progress is 1. viewdirs reach
+        the head as given (not normalised). Points outside the aabb shade zero appearance components, as
+        grid_sample's zero padding gives. Rows are independent: the result does not depend on how many points are
+        passed at once or in which order."""
+        shape = xyz_locs.shape[:-1]
+        ops._need_cuda(xyz_locs, "xyz_locs")
+        xyz = xyz_locs.reshape(-1, 3).float()
+        n = xyz.shape[0]
+        if viewdirs.dim() == 1:
+            dirs = viewdirs.reshape(1, 3).float().expand(n, 3)
+        else:
+            dirs = viewdirs.reshape(-1, 3).float()
+            if dirs.shape[0] != n:
+                raise _lib.JtError(f"compute_rgb: {dirs.shape[0]} view directions for {n} points")
+        ops._need_cuda(dirs, "viewdirs")
+        storage = self._checked_storage()
+        rgb = torch.empty((n, 3), device=xyz.device)
+        if n == 0:
+            return rgb.view(*shape, 3)
+        afs = self._app_factorset()
+        if storage == "bf16":          # the bf16 copy is cached, like forward's, only for the unblurred Parameters
+            afs = afs.with_bf16_store(self._store_cache[1] if self.c2f_mode is None else None)
+        cfg = RenderCfg(**self._head_fields())
+        basis_w = self.basis_mat.weight.detach().contiguous()
+        head = [t.detach().contiguous() for t in self.renderModule.head_params()] if self.renderModule is not None else []
+        for s in range(0, n, self._RGB_CHUNK):
+            e = min(n, s + self._RGB_CHUNK)
+            rgb[s:e] = shade_points(cfg, afs, self.normalize_coord(xyz[s:e]), dirs[s:e], basis_w, head)
+        return rgb.view(*shape, 3)
+
     @torch.no_grad()
     def compute_alpha(self, xyz_locs, length=1):
         """BatBase.compute_alpha (batBase.py:27-42) as one kernel: mask test, normalisation, density gather,
@@ -596,18 +640,12 @@ class B200_VMSplit(torch.nn.Module):
             mask=(self.alphaMask if (self.alphaMask is not None and not blur_active) else None),   # batBase.py:76
             density_shift=float(self.density_shift), act=(0 if self.fea2denseAct == "softplus" else 1),
             distance_scale=float(self.distance_scale), thres=float(self.rayMarch_weight_thres),
-            depth_bias=-float(self.near_far[0]) + 0.05, shading=self.shadingMode, app_dim=int(self.app_dim),
-            fea_pe=int(self.fea_pe), view_pe=int(self.view_pe), hidden=int(self.featureC),
-            fea_prog=float(fea_pe_progress), view_prog=float(view_pe_progress), tc_fwd_split=int(self.tc_fwd_split),
-            tc_infer_fp16=bool(self.tc_infer_fp16))
-        if self.head_precision == "tc" or (self.head_precision == "auto" and self.tc_available()):
-            cfg.head = "tc"
+            depth_bias=-float(self.near_far[0]) + 0.05, fea_prog=float(fea_pe_progress),
+            view_prog=float(view_pe_progress), **self._head_fields())
 
         cfg.grad_sync = self.grad_sync
         cfg.grad_enabled = torch.is_grad_enabled()
-        if self.factor_storage not in ("fp32", "bf16"):
-            raise _lib.JtError(f"factor_storage {self.factor_storage!r}: expected 'fp32' or 'bf16'")
-        cfg.storage = self.factor_storage
+        cfg.storage = self._checked_storage()
         if self.app_capacity == "auto" and cfg.grad_enabled:
             cfg.app_cap = self._app_tracker.capacity(center.reshape(-1, 3).shape[0], center.reshape(-1, 3).shape[0] * n_samples)
             cfg.app_monitor = self._app_tracker.submit
@@ -624,6 +662,18 @@ class B200_VMSplit(torch.nn.Module):
                               self.basis_mat.weight, *head)
 
     render = forward      # north_star calls the entry point `render`; the reference engine calls forward
+
+    def _head_fields(self):
+        """The RenderCfg fields that choose and size the shading head (forward and compute_rgb)."""
+        tc = self.head_precision == "tc" or (self.head_precision == "auto" and self.tc_available())
+        return dict(shading=self.shadingMode, app_dim=int(self.app_dim), fea_pe=int(self.fea_pe),
+                    view_pe=int(self.view_pe), hidden=int(self.featureC), tc_fwd_split=int(self.tc_fwd_split),
+                    tc_infer_fp16=bool(self.tc_infer_fp16), head="tc" if tc else "fp32")
+
+    def _checked_storage(self):
+        if self.factor_storage not in ("fp32", "bf16"):
+            raise _lib.JtError(f"factor_storage {self.factor_storage!r}: expected 'fp32' or 'bf16'")
+        return self.factor_storage
 
     def tc_available(self):
         """True when the tcgen05 shading-head kernels cover this configuration (what head_precision="auto" picks):
@@ -685,24 +735,47 @@ class B200_VMSplit(torch.nn.Module):
         return self._dense_alpha_zyx(gridSize).permute(2, 1, 0), dense_xyz
 
     @torch.no_grad()
-    def extract_mesh(self, level=0.005, gridSize=None):
+    def extract_mesh(self, level=0.005, gridSize=None, colors=False):
         """The field's geometry as a triangle mesh: marching cubes (ops.marching_cubes) on the dense alpha grid of
         getDenseAlpha(gridSize) at alpha `level` (0.005 is TensoRF's exporter level). Honours the alpha mask and a
         cached density blur exactly as getDenseAlpha does. Returns (verts [V,3] fp32 world coordinates, faces [F,3]
-        int32) on the module's device; normals point out of the high-alpha region."""
+        int32) on the module's device; normals point out of the high-alpha region.
+        colors=True returns (verts, faces, normals, rgb) with the same verts and faces: normals [V,3] are the unit
+        gradients of the alpha volume the surface was extracted from (ops.marching_cubes(normals=True)), pointing out
+        of the high-alpha region, and rgb [V,3] = compute_rgb(verts, -normals), the colour seen looking at the surface
+        head-on (a vertex with a zero normal is shaded with a zero view direction). For an NDC (LLFF) field the
+        vertices, normals and view directions are all in the field's NDC coordinates."""
         gridSize = self._grid if gridSize is None else [int(v) for v in gridSize]
-        return ops.marching_cubes(self._dense_alpha_zyx(gridSize), level, self._dense_tables(gridSize), self._h_aabb)
+        mesh = ops.marching_cubes(self._dense_alpha_zyx(gridSize), level, self._dense_tables(gridSize), self._h_aabb,
+                                  normals=colors)
+        if not colors:
+            return mesh
+        verts, faces, normals = mesh
+        return verts, faces, normals, self.compute_rgb(verts, -normals)
 
-    def export_mesh(self, path, level=0.005, gridSize=None):
+    def export_mesh(self, path, level=0.005, gridSize=None, colors=False):
         """extract_mesh written to `path` as a binary little-endian PLY (float x, y, z per vertex; `list uchar int
-        vertex_indices` per face). Returns (V, F)."""
-        verts, faces = self.extract_mesh(level, gridSize)
+        vertex_indices` per face). colors=True adds `float nx, ny, nz` and `uchar red, green, blue` per vertex (the
+        names MeshLab, Blender and Open3D read), colours quantised as floor(clamp(rgb, 0, 1) * 255 + 0.5) in fp32.
+        Returns (V, F)."""
+        mesh = self.extract_mesh(level, gridSize, colors=colors)
+        verts, faces = mesh[0], mesh[1]
         v = verts.cpu().numpy().astype("<f4")
+        props = "property float x\nproperty float y\nproperty float z\n"
+        if colors:
+            rgb = np.clip(mesh[3].cpu().numpy(), np.float32(0), np.float32(1))
+            vt = np.empty((v.shape[0],), dtype=[("p", "<f4", (3,)), ("n", "<f4", (3,)), ("c", "u1", (3,))])
+            vt["p"] = v
+            vt["n"] = mesh[2].cpu().numpy()
+            vt["c"] = np.floor(rgb * np.float32(255) + np.float32(0.5))
+            props += ("property float nx\nproperty float ny\nproperty float nz\n"
+                      "property uchar red\nproperty uchar green\nproperty uchar blue\n")
+            v = vt
         f = np.empty((faces.shape[0],), dtype=[("n", "u1"), ("i", "<i4", (3,))])
         f["n"] = 3
         f["i"] = faces.cpu().numpy()
         header = ("ply\nformat binary_little_endian 1.0\n"
-                  f"element vertex {v.shape[0]}\nproperty float x\nproperty float y\nproperty float z\n"
+                  f"element vertex {v.shape[0]}\n{props}"
                   f"element face {f.shape[0]}\nproperty list uchar int vertex_indices\nend_header\n")
         with open(path, "wb") as fh:
             fh.write(header.encode("ascii"))
