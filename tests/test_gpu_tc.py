@@ -80,100 +80,3 @@ def test_head_fwd_tc_matches_fp32(split, tol, a_count):
                     d["renderModule.mlp.4.bias"], cnt, a_count + 500, 0.8, 0.6, rgb, feat)
     assert (feat[:, :27].cpu() - feat_ref).abs().max() <= tol * max(1.0, float(feat_ref.abs().max()))
     assert (rgb[:, :3].cpu() - ref).abs().max() <= tol
-
-
-@pytest.mark.parametrize("dc_dtype", [torch.float32, torch.bfloat16])
-@pytest.mark.parametrize("a_count", [1, 128, 1000, 40000])
-def test_head_bwd_tc_matches_fp32_autograd(a_count, dc_dtype):
-    p, comps, rays_d, sidx, aidx, S = _head_inputs(a_count, seed=3)
-    g = torch.Generator().manual_seed(7)
-    dout = torch.randn(a_count, 3, generator=g) * 0.1
-    names = ["basis_mat.weight", "renderModule.mlp.0.weight", "renderModule.mlp.0.bias", "renderModule.mlp.2.weight",
-             "renderModule.mlp.2.bias", "renderModule.mlp.4.weight", "renderModule.mlp.4.bias"]
-    # fp32 autograd reference of the same op (pre-sigmoid output, so dout is its upstream gradient)
-    pr = {k: v.clone().requires_grad_(True) for k, v in p.items()}
-    cr = comps.clone().requires_grad_(True)
-    feat = cr @ pr["basis_mat.weight"].T
-    dirs = rays_d[(sidx[aidx.long()] // S).long()]
-    x = torch.cat([feat, dirs, vo.positional_encoding(feat, 2, 0.8), vo.positional_encoding(dirs, 2, 0.6)], -1)
-    h = torch.relu(x @ pr[names[1]].T + pr[names[2]])
-    h = torch.relu(h @ pr[names[3]].T + pr[names[4]])
-    out = h @ pr[names[5]].T + pr[names[6]]
-    (out * dout).sum().backward()
-    d = {k: v.to(DEV).contiguous() for k, v in p.items()}
-    dout4 = torch.zeros((a_count, 4), device=DEV)
-    dout4[:, :3] = dout.to(DEV)
-    dcomps = torch.zeros((a_count, 144), device=DEV, dtype=dc_dtype)
-    grads = [torch.zeros_like(d[k]) for k in names]
-    cnt = torch.tensor([a_count], device=DEV, dtype=torch.int32)
-    rgb = torch.zeros((a_count, 4), device=DEV)
-    feat_d = torch.zeros((a_count, 28), device=DEV)
-    stage = ops.head_tc_stage(a_count + 300, DEV)
-    ops.head_fwd_tc(2, comps.to(DEV), aidx.to(DEV), sidx.to(DEV), rays_d.to(DEV), S, False, *[d[k] for k in names],
-                    cnt, a_count + 300, 0.8, 0.6, rgb, feat_d, stage)
-    ops.head_bwd_tc(dout4, feat_d, d[names[0]], d[names[1]], d[names[3]], d[names[5]], cnt, a_count + 300, 0.8,
-                    dcomps, stage, grads)
-    torch.cuda.synchronize()
-    def rel(a, b):
-        return float((a.cpu().double() - b.double()).abs().max() / b.double().abs().max().clamp_min(1e-30))
-    # per-sample rows: a relu unit whose fp32 pre-activation is within rounding of 0 may take the other
-    # branch (a tie, ~1e-6 of all units) -- allow <= 0.02 % such rows, bound everything else by 2e-2
-    dcomps = dcomps.float()
-    err_rows = (dcomps.cpu().double() - cr.grad.double()).abs().amax(1) / cr.grad.double().abs().max()
-    assert float((err_rows > 2e-2).double().mean()) <= 2e-4, float((err_rows > 2e-2).double().mean())
-    assert float(torch.linalg.norm(dcomps.cpu().double() - cr.grad.double()) / torch.linalg.norm(cr.grad.double())) <= 2e-2
-    for k, gk in zip(names, grads):
-        assert rel(gk, pr[k].grad) <= 2e-2, (k, rel(gk, pr[k].grad))
-
-
-@pytest.mark.parametrize("split,tol", [(2, 3e-5), (1, 2e-2), (3, 1e-4)])
-@pytest.mark.parametrize("a_count", [1, 129, 5000])
-def test_app_basis_and_mlp_kernels_match_fp32(split, tol, a_count):
-    """jt_app_basis_fwd_tc (gather + basis_mat on tensor cores) against the SIMT gather + fp32 matmul,
-    then jt_head_mlp_fwd_tc on its rows against the oracle's MLP_Fea."""
-    from joint_tensorf_b200.ops import FactorSet
-    g = torch.Generator().manual_seed(5)
-    grid = [13, 11, 17]
-    p = vo.init_params(grid, [16] * 3, [48] * 3, 27, "MLP_Fea", 64, 2, 2, 0.3, 0.1, seed=5)
-    d = {k: v.to(DEV) for k, v in p.items()}
-    planes = [d[f"app_plane.{i}"].permute(0, 2, 3, 1).contiguous().permute(0, 3, 1, 2) for i in range(3)]
-    lines = [d[f"app_line.{i}"].permute(0, 2, 3, 1).contiguous().permute(0, 3, 1, 2) for i in range(3)]
-    fs = FactorSet(planes, lines)
-    n_rays, S, V = 37, 64, a_count + 77
-    samp = torch.zeros(V, 4)
-    samp[:, :3] = torch.rand(V, 3, generator=g) * 2.2 - 1.1          # some taps fall outside the grid
-    rays_d = torch.randn(n_rays, 3, generator=g)
-    sidx = (torch.randint(0, n_rays, (V,), generator=g) * S + torch.randint(0, S, (V,), generator=g)).int()
-    aidx = torch.randperm(V, generator=g)[:a_count].int()
-    samp_d, aidx_d, sidx_d, rays_dd = samp.to(DEV), aidx.to(DEV), sidx.to(DEV), rays_d.to(DEV)
-    cnt = torch.tensor([a_count], device=DEV, dtype=torch.int32)
-    cap = a_count + 300
-    # reference: SIMT gather -> fp32 matmul
-    comps = torch.zeros((cap, 144), device=DEV)
-    ops.vm_gather_fwd(1, fs, samp_d, aidx_d, cnt, cap, comps)
-    feat_ref = comps[:a_count] @ d["basis_mat.weight"].T
-    featdir = torch.full((cap, 32), 7.0, device=DEV)
-    stage = ops.head_tc_stage(cap, DEV)
-    # split 3 (fp16 operand tiles) exists for the inference call of the MLP kernel only
-    ops.app_basis_fwd_tc(min(split, 2), fs, samp_d, aidx_d, sidx_d, rays_dd, S, False,
-                         d["basis_mat.weight"].contiguous(), cnt, cap, featdir, stage)
-    tol_b = 3e-5 if split == 3 else tol
-    scale = max(1.0, float(feat_ref.abs().max()))
-    assert (featdir[:a_count, :27] - feat_ref).abs().max() <= tol_b * scale
-    dirs = rays_d[(sidx[aidx.long()] // S).long()]
-    assert torch.equal(featdir[:a_count, 28:31].cpu(), dirs)
-    assert float(featdir[a_count:].sub(7.0).abs().max()) == 0.0, "rows past the count must not be written"
-    # the saved bf16 component tile (first 128 rows) equals bf16(comps)
-    tile = stage[: 128 * 144 * 2].view(torch.bfloat16).view(18, 128, 8).permute(1, 0, 2).reshape(128, 144).float()
-    m = min(a_count, 128)
-    assert (tile[:m] - comps[:m].to(torch.bfloat16).float()).abs().max() <= 1e-2 * max(1e-3, float(comps.abs().max()))
-    # MLP kernel on the rows
-    rgb = torch.zeros((cap, 4), device=DEV)
-    names = ["renderModule.mlp.0.weight", "renderModule.mlp.0.bias", "renderModule.mlp.2.weight",
-             "renderModule.mlp.2.bias", "renderModule.mlp.4.weight", "renderModule.mlp.4.bias"]
-    ops.head_mlp_fwd_tc(split, featdir, *[d[k].contiguous() for k in names], cnt, cap, 0.8, 0.6, rgb,
-                        None if split == 3 else stage)
-    field = vo.Field(aabb=torch.zeros(2, 3), grid=grid, params=p)
-    ref = vo.shade_mlp_fea(field, dirs, featdir[:a_count, :27].cpu(), 0.6, 0.8)
-    assert (rgb[:a_count, :3].cpu() - ref).abs().max() <= tol
-    assert float(rgb[a_count:].abs().max()) == 0.0
