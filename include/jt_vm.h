@@ -46,7 +46,8 @@ typedef struct CUstream_st* cudaStream_t;
 
 /* ---- library ----------------------------------------------------------- */
 const char* jt_strerror(int code);
-int jt_version(void);            /* ABI version, bumped on any signature or argument-semantics change (3: NULL gradients) */
+int jt_version(void);            /* ABI version, bumped on any signature or argument-semantics change
+                                  * (3: NULL gradients; 4: jt_head_fwd_tc removed) */
 /* number of kernel launches issued through this library since load (for bench.py) */
 long long jt_launch_count(void);
 
@@ -152,23 +153,16 @@ int jt_sh_shade(int bwd, const float* feat, int ldf, const int* aidx, const int*
  * mode 2 = mode 0 with both operands stored as fp16. */
 int jt_tc_selftest(int mode, const float* A, int lda, const float* B, int ldb, float* D, int K, int N, int Ma,
                    cudaStream_t stream);
-/* basis_mat (tensoRF.py:270) + positional_encoding (tensorBase.py:43-55) + MLPRender_Fea
- * (tensorBase.py:116-126) fused per tile of 128 appearance samples, app_dim 27 / hidden 64 /
- * fea_pe = view_pe = 2: comps [A][144] -> rgb [A][4]. split = 1: bf16 operands; split = 2:
- * every operand as hi+lo bf16 terms, 3 MMAs per product (fp32-class accuracy). feat_out
- * (optional) [A][28] receives the basis projection. stage (optional, training): scratch of
- * jt_head_tc_stage_bytes(n_max) bytes, 128-byte aligned, that receives the bf16 operand tiles
- * (components, encoded input, relu(h1), relu(h2)) jt_head_bwd_tc needs. */
+/* Staging area of the training forward of the tensor-core head: jt_head_tc_stage_bytes(n_max) bytes, 128-byte
+ * aligned, one block per tile of 128 appearance samples. The two forward kernels below write the bf16 operand tiles
+ * jt_head_bwd_tc reads (exact relu masks and the operands of the weight-gradient GEMMs): jt_app_basis_fwd_tc the
+ * component tile, jt_head_mlp_fwd_tc the encoded-input, relu(h1) and relu(h2) tiles. The backward keeps its own
+ * gradient tiles in the rest of each block. The SH pair (jt_app_basis_sh_fwd_tc, jt_sh_bwd_tc) uses the same area. */
 long long jt_head_tc_stage_bytes(int n_max);
-/* (unit-test harness: the monolithic first version of the tensor-core head, components read from HBM; the
- * product path is jt_app_basis_fwd_tc + jt_head_mlp_fwd_tc. Kept because tests/test_gpu_tc.py stages the backward's
- * operand tiles from arbitrary component rows with it.) */
-int jt_head_fwd_tc(int split, const float* comps, const int* aidx, const int* sidx, const float* rays_d,
-                   int n_samples, int normalize_dir, const float* Wb, const float* W1, const float* b1,
-                   const float* W2, const float* b2, const float* W3, const float* b3, const int* n_dev, int n_max,
-                   float fea_progress, float view_progress, float* rgb, float* feat_out, void* stage,
-                   cudaStream_t stream);
-/* The same head as two kernels, the form the fused render op uses:
+/* basis_mat (tensoRF.py:270) + positional_encoding (tensorBase.py:43-55) + MLPRender_Fea (tensorBase.py:116-126)
+ * for app_dim 27 / hidden 64 / fea_pe = view_pe = 2 as two kernels, the form the fused render op uses.
+ * split = 1: bf16 operands; split = 2: every operand as hi+lo bf16 terms, 3 MMAs per product (fp32-class accuracy);
+ * split = 3 (jt_head_mlp_fwd_tc only, inference: stage NULL): fp16 operands.
  * jt_app_basis_fwd_tc = appearance gather (bateRF.py:97-128) + basis_mat (tensoRF.py:270) per tile
  * of 128 samples: the plane x line products go straight into the bf16 shared-memory operand tile
  * (never to HBM in fp32), one tcgen05 GEMM projects them; out featdir [A][32] = feat 0..26 | 0 |
@@ -185,7 +179,7 @@ int jt_head_mlp_fwd_tc(int split, const float* featdir, const float* W1, const f
                        float fea_progress, float view_progress, float* rgb, void* stage, cudaStream_t stream);
 /* Backward of the tensor-core head (bf16 tensor-core GEMMs, fp32 accumulation in TMEM): from dout
  * [A][4] (gradient at the head's pre-activation, from jt_render_bwd), feat [A][ldf] and the
- * tiles the forward left in `stage`, computes dcomps [A][144] (for jt_vm_gather_bwd) and ADDS
+ * tiles the forward left in `stage`, computes dcomps [A][144] (for jt_vm_scatter_rays) and ADDS
  * the weight gradients into gWb [27][144], gW1 [64][150], gb1, gW2 [64][64], gb2, gW3 [3][64],
  * gb3. relu masks are the forward's own; nothing is recomputed.
  * All seven weight-gradient pointers NULL (since version 3; frozen head and basis_mat): dcomps alone, bit-identical

@@ -26,7 +26,6 @@ SIGNATURES = {
     "jt_pe_encode": [_I, _I, _I, _I, _I, _F, _F, _I, _I, _P, _I, _P, _P, _P, _P, _I, _P, _I, _P, _I, _P, _I, _P],
     "jt_sh_shade": [_I, _P, _I, _P, _P, _P, _I, _I, _P, _I, _P, _P, _P, _I, _P],
     "jt_tc_selftest": [_I, _P, _I, _P, _I, _P, _I, _I, _I, _P],
-    "jt_head_fwd_tc": [_I, _P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _I, _F, _F, _P, _P, _P, _P],
     "jt_app_basis_fwd_tc": [_I, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P, _I, _P, _P, _P],
     "jt_head_mlp_fwd_tc": [_I, _P, _P, _P, _P, _P, _P, _P, _P, _I, _F, _F, _P, _P, _P],
     "jt_head_bwd_tc": [_P, _P, _I, _P, _P, _P, _P, _P, _I, _F, _P, _I, _P, _P, _P, _P, _P, _P, _P, _P, _P],

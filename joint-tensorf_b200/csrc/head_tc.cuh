@@ -1,6 +1,6 @@
-// Shared pieces of the tensor-core shading-head kernels (forward: shade_tc.cu, backward:
-// shade_tc_bwd.cu): dimensions of the MLP_Fea head, the tensor-core column order of
-// layer 1, operand staging and GEMM issue helpers.
+// Shared pieces of the tensor-core shading-head kernels (forward: app_basis_tc.cu +
+// head_mlp_tc.cu, backward: shade_tc_bwd.cu): dimensions of the MLP_Fea head, the
+// tensor-core column order of layer 1, operand staging and GEMM issue helpers.
 #pragma once
 #include "jt_common.cuh"
 #include "tc_common.cuh"

@@ -13,5 +13,5 @@ extern "C" const char* jt_strerror(int code) {
         default: return "unknown error";
     }
 }
-extern "C" int jt_version(void) { return 3; }
+extern "C" int jt_version(void) { return 4; }
 extern "C" long long jt_launch_count(void) { return jt::g_launches; }

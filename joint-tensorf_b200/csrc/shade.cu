@@ -5,8 +5,8 @@
 // positional_encoding (tensorBase.py:43-55), MLPRender_Fea.forward
 // (tensorBase.py:116-126), MLPRender_Fea_WeakView.forward (tensorBase.py:198-214),
 // SHRender (tensorBase.py:68-72) + eval_sh_bases deg 2 (sh.py:88-113) and their
-// autograd. This is the bit-faithful fp32 mode (<= 1e-4 parity class); the
-// tensor-core (tcgen05) fused head lives in shade_tc.cu.
+// autograd. This is the bit-faithful fp32 mode (<= 1e-4 parity class); the tensor-core
+// (tcgen05) heads live in app_basis_tc.cu, head_mlp_tc.cu, shade_tc_bwd.cu, weakview_tc.cu.
 #include "jt_common.cuh"
 #include "../../include/jt_vm.h"
 

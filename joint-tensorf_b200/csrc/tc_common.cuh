@@ -27,9 +27,6 @@ __device__ __forceinline__ void mbar_fence_init() { asm volatile("fence.mbarrier
 __device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     asm volatile(
         "{\n"
@@ -144,9 +141,6 @@ __device__ __forceinline__ uint32_t pack_f16(float a, float b) {
     __half2 h = __floats2half2_rn(a, b);
     return *reinterpret_cast<uint32_t*>(&h);
 }
-// residual of the bf16 rounding (second term of the 2-term split a = hi + lo)
-__device__ __forceinline__ float bf16_resid(float a) { return a - __bfloat162float(__float2bfloat16_rn(a)); }
-
 // hi/lo split of a float pair with packed conversions only: hi = bf16x2(a, b) (one F2FP), the
 // exact fp32 value of each half is a shift / mask of the packed word, lo = bf16x2 of the residuals.
 __device__ __forceinline__ void split_pair(float a, float b, uint32_t& hi, uint32_t& lo) {

@@ -254,15 +254,6 @@ def head_tc_stage(n_max, device):
     return torch.empty((nbytes,), device=device, dtype=torch.uint8)
 
 
-def head_fwd_tc(split, comps, aidx, sidx, rays_d, n_samples, normalize_dir, wb, w1, b1, w2, b2, w3, b3, n_dev, n_max,
-                fprog, vprog, rgb, feat_out=None, stage=None):
-    with TIMER.span("head_fwd_tc"):
-        check(_lib.lib().jt_head_fwd_tc(split, _p(comps), _p(aidx), _p(sidx), _p(rays_d), n_samples,
-                                        int(normalize_dir), _p(wb), _p(w1), _p(b1), _p(w2), _p(b2), _p(w3), _p(b3),
-                                        _p(n_dev), int(n_max), float(fprog), float(vprog), _p(rgb), _p(feat_out),
-                                        _p(stage), _stream()), "jt_head_fwd_tc")
-
-
 def app_basis_fwd_tc(split, fs, samp, aidx, sidx, rays_d, n_samples, normalize_dir, wb, n_dev, n_max, featdir,
                      stage=None):
     """appearance gather + basis_mat on tensor cores -> featdir [A][32] (feat | dir)."""

@@ -8,6 +8,7 @@ import pytest
 import torch
 
 import joint_tensorf_b200 as jt
+import test_gpu_head_reference as head_ref
 from common import golden_names, load_golden, rel_err
 from gpu_common import default_opt, forward_kwargs, module_from_golden, record_err
 from joint_tensorf_b200 import ops
@@ -169,18 +170,16 @@ def test_sh_bwd_tc_without_weight_gradient_is_bit_identical():
 
 
 @pytest.mark.parametrize("dc_dtype", [torch.float32, torch.bfloat16])
-def test_head_bwd_tc_without_weight_gradients_is_bit_identical(dc_dtype):
-    A, S, n_rays = 20000, 64, 37
+def test_head_bwd_tc_without_weight_gradients_is_bit_identical_after_two_kernel_forward(dc_dtype):
+    A = 20000
     gen = torch.Generator().manual_seed(3)
-    comps = (torch.rand(A, 144, generator=gen) * 0.05).to(DEV)
-    rays_d = torch.randn(n_rays, 3, generator=gen).to(DEV)
-    sidx = (torch.randint(0, n_rays, (A,), generator=gen) * S + torch.randint(0, S, (A,), generator=gen)).int().to(DEV)
-    aidx = torch.randperm(A, generator=gen).int().to(DEV)
+    I = head_ref._Inputs("mlp", A, seed=3)       # random 3 x 48-component appearance field and A samples of it
     wb, w1, b1, w2, b2, w3, b3 = _weights([(27, 144), (64, 150), (64,), (64, 64), (64,), (3, 64), (3,)], 4)
-    cnt = torch.tensor([A], device=DEV, dtype=torch.int32)
-    rgb, feat = torch.zeros((A, 4), device=DEV), torch.zeros((A, 28), device=DEV)
+    cnt = I.count
+    rgb, feat = torch.zeros((A, 4), device=DEV), torch.zeros((A, 32), device=DEV)
     stage = ops.head_tc_stage(A, DEV)
-    ops.head_fwd_tc(2, comps, aidx, sidx, rays_d, S, False, wb, w1, b1, w2, b2, w3, b3, cnt, A, 0.8, 0.6, rgb, feat, stage)
+    ops.app_basis_fwd_tc(2, I.afs, I.samp, I.aidx, I.sidx, I.rays_d, head_ref.S, False, wb, cnt, A, feat, stage)
+    ops.head_mlp_fwd_tc(2, feat, w1, b1, w2, b2, w3, b3, cnt, A, 0.8, 0.6, rgb, stage)
     dout = torch.zeros((A, 4), device=DEV)
     dout[:, :3] = (torch.randn(A, 3, generator=gen) * 0.1).to(DEV)
     dc_full, dc_frozen = torch.empty((A, 144), device=DEV, dtype=dc_dtype), torch.empty((A, 144), device=DEV, dtype=dc_dtype)
