@@ -234,6 +234,14 @@ int jt_render_bwd(const int* ray_off, int n_rays, const float* sigfeat, const fl
                   const float* trans, const int* app_of, const float* rgb, const float* rgb_pre,
                   const float* g_rgb, const float* g_acc, float density_shift, int act, float distance_scale,
                   int white_bg, int shade_act, float* dout, float* dsig, float* dnorm, cudaStream_t stream);
+/* Normal map of the rays jt_alpha_fwd composited: normal_map [N][3] = sum_j weight_j * normals_j over every valid
+ * sample j of ray r (ray_off as jt_march_compact writes it; the weights whose sum is the opacity), normals [V][3] the
+ * per-sample unit normals of jt_field_density_grad (normals = 1); not renormalised, so |normal_map[r]| <= acc[r].
+ * depth and opacity are written exactly as jt_composite_fwd writes them. One warp per ray in a fixed order: a ray's
+ * result does not depend on the other rays of the call. */
+int jt_normal_composite(const int* ray_off, int n_rays, const float* weight, const float* normals, const float* acc,
+                        const float* wz, const float* rays_d, float depth_bias, float* normal_map, float* depth,
+                        float* opacity, cudaStream_t stream);
 /* ---- K5: separable blur ------------------------------------------------ */
 /* BAT_VMSplit.convolute_plane / convolute_line (bateRF.py:8-39) on a channel-last
  * [H][W][C] array: replicate-padded cross-correlation with `h_taps` [ntaps] (HOST
@@ -308,6 +316,21 @@ int jt_field_alpha(const void* const* h_factors, const int* h_dims, const float*
                    long long n_points, const float* lin_x, const float* lin_y, const float* lin_z, const int* h_grid3,
                    const uint32_t* mask_bits, const int* h_mask_dims, const float* h_mask_geom, float density_shift,
                    int act, float length, float* alpha, cudaStream_t stream);
+/* Density and its spatial gradient at points, forward mode (no atomics, no gradient buffers; deterministic, and each
+ * point's result is independent of the others): sigma = feature2density(sigma_feature(p)) with jt_field_alpha's taps
+ * and summation order (so 1 - exp(-sigma * length) equals its alpha), and grad = d sigma / d p, the analytic derivative
+ * of the piecewise-multilinear field that grid_sample(bilinear, align_corners=True, zeros) evaluates (out-of-range
+ * taps count as 0; one-sided at cell boundaries as the tap rounding falls), times feature2density' and the per-axis
+ * invaabbSize of normalize_coord: the gradient is in the field's input coordinates (world, or NDC for an NDC field).
+ * Points: xyz != NULL: n_max explicit points [n][3] (slot and n_dev NULL), tested against the optional occupancy
+ * mask (rejected points give sigma 0, grad 0); samp != NULL: compacted float4 records (normalised coordinates, as
+ * jt_march_compact writes them), element e reads samp[slot ? slot[e] : e], count n_dev (device) or n_max; no mask.
+ * Exactly one of xyz / samp. normals = 1: grad receives the unit outward normal -grad / |grad| instead ((0,0,0) where
+ * grad is zero or not finite). sigma [n] may be NULL; grad [n][3]. Factors: fp32 (elem 0). */
+int jt_field_density_grad(const void* const* h_factors, const int* h_dims, const float* h_geom, const float* xyz,
+                          const float* samp, const int* slot, const int* n_dev, long long n_max,
+                          const uint32_t* mask_bits, const int* h_mask_dims, const float* h_mask_geom,
+                          float density_shift, int act, int normals, float* sigma, float* grad, cudaStream_t stream);
 /* The rest of updateAlphaMask (tensorBase.py:639-657): clamp(alpha, 0, 1) -> max_pool3d(kernel 5, pad 2, stride 1)
  * -> >= thres, on alpha [D][H][W]. Outputs: vol [D][H][W] floats {0,1} (AlphaGridMask.alpha_volume), bits = the same
  * bit-packed ((W*H*D+31)/32 words, layout of MaskGeom), stats7 = {min_x, max_x, min_y, max_y, min_z, max_z, count}

@@ -151,6 +151,12 @@ __global__ void __launch_bounds__(256) app_fill_kernel(const int* __restrict__ o
 }
 
 // ------------------------------------------------------------------ forward, pass C
+// batBase.py:160-162: depth = sum w*t + (1 - acc) * ray_dir_z - near + 0.05 (one expression for both compositing kernels,
+// so render_normals' depth is bit-identical to forward's)
+__device__ __forceinline__ float ray_depth(float wz, float acc, float dir_z, float depth_bias) {
+    return wz + (1.0f - acc) * dir_z + depth_bias;
+}
+
 // rgb_map = sum w*rgb (+ 1-acc if white) clamped; depth; opacity.
 __global__ void __launch_bounds__(256) composite_fwd_kernel(const int* __restrict__ aoff, int n_rays,
                                                             const int* __restrict__ aidx,
@@ -192,7 +198,38 @@ __global__ void __launch_bounds__(256) composite_fwd_kernel(const int* __restric
             rgb_map[3 * r + 0] = fminf(fmaxf(c0, 0.f), 1.f);
             rgb_map[3 * r + 1] = fminf(fmaxf(c1, 0.f), 1.f);
             rgb_map[3 * r + 2] = fminf(fmaxf(c2, 0.f), 1.f);
-            depth[r] = wz_in[r] + (1.0f - acc) * rays_d[3 * r + 2] + depth_bias;   // - near + 0.05
+            depth[r] = ray_depth(wz_in[r], acc, rays_d[3 * r + 2], depth_bias);
+            opacity[r] = acc;
+        }
+    }
+}
+
+// Normal map: normal[r] = sum_j w_j n_j over ALL valid samples of ray r (the weights whose sum is opacity), n [V][3] the
+// per-sample unit normals of jt_field_density_grad; depth and opacity as composite_fwd_kernel writes them. One warp
+// per ray, lane-strided sums then a fixed butterfly: the result does not depend on the batch the ray is rendered in.
+__global__ void __launch_bounds__(256) normal_composite_kernel(const int* __restrict__ off, int n_rays,
+                                                               const float* __restrict__ weight,
+                                                               const float* __restrict__ nrm,
+                                                               const float* __restrict__ acc_in,
+                                                               const float* __restrict__ wz_in,
+                                                               const float* __restrict__ rays_d, float depth_bias,
+                                                               float* __restrict__ normal, float* __restrict__ depth,
+                                                               float* __restrict__ opacity) {
+    const int lane = threadIdx.x & 31;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int nwarps = (gridDim.x * blockDim.x) >> 5;
+    for (int r = warp; r < n_rays; r += nwarps) {
+        const int b = off[r], e = off[r + 1];
+        float c0 = 0.f, c1 = 0.f, c2 = 0.f;
+        for (int j = b + lane; j < e; j += 32) {
+            const float w = weight[j];
+            c0 += w * nrm[3 * j]; c1 += w * nrm[3 * j + 1]; c2 += w * nrm[3 * j + 2];
+        }
+        c0 = warp_sum(c0); c1 = warp_sum(c1); c2 = warp_sum(c2);
+        if (lane == 0) {
+            const float acc = acc_in[r];
+            normal[3 * r + 0] = c0; normal[3 * r + 1] = c1; normal[3 * r + 2] = c2;
+            depth[r] = ray_depth(wz_in[r], acc, rays_d[3 * r + 2], depth_bias);
             opacity[r] = acc;
         }
     }
@@ -362,6 +399,17 @@ extern "C" int jt_composite_fwd(const int* app_off, int n_rays, const int* aidx,
     composite_fwd_kernel<<<ray_grid(n_rays), 256, 0, stream>>>(app_off, n_rays, aidx, weight, rgb, acc, wz, rays_d,
                                                                white_bg, depth_bias, rgb_pre, rgb_map, depth, opacity,
                                                                app_cap > 0 ? app_cap : 2147483647);
+    JT_RETURN_LAUNCH();
+}
+
+extern "C" int jt_normal_composite(const int* ray_off, int n_rays, const float* weight, const float* normals,
+                                   const float* acc, const float* wz, const float* rays_d, float depth_bias,
+                                   float* normal_map, float* depth, float* opacity, cudaStream_t stream) {
+    JT_CHECK_ARG(ray_off && weight && normals && acc && wz && rays_d && normal_map && depth && opacity);
+    if (n_rays <= 0) return JT_OK;
+    g_launches += 1;
+    normal_composite_kernel<<<ray_grid(n_rays), 256, 0, stream>>>(ray_off, n_rays, weight, normals, acc, wz, rays_d,
+                                                                  depth_bias, normal_map, depth, opacity);
     JT_RETURN_LAUNCH();
 }
 

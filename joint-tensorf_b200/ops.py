@@ -537,6 +537,34 @@ def field_alpha(fs, geom, shift, act, length, xyz=None, lin=None, grid=None, mas
     return out
 
 
+def field_density_grad(fs, geom, shift, act, xyz=None, samp=None, slot=None, n_dev=None, n_max=None, mask=None,
+                       normals=False, want_sigma=True):
+    """sigma = feature2density(sigma_feature(p)) and grad = d sigma / d p (jt_field_density_grad, no autograd): at world
+    points xyz [n,3] (tested against the occupancy mask) -> (sigma [n], grad [n,3]), or at compacted samples samp
+    [cap,4] (normalised coordinates; element e reads samp[slot[e]] when slot is given; count n_dev on the device, at
+    most n_max; no mask). normals=True: the second
+    output holds the unit outward normals -grad/|grad| (0 where grad is 0 or not finite). want_sigma=False: sigma is
+    not written and None is returned in its place. fs: FactorSet of the fp32 density factors."""
+    mb, md, mg = (mask.bits, mask.h_dims, mask.h_geom) if mask is not None else (None, None, None)
+    if xyz is not None:
+        _need_cuda(xyz, "xyz")
+        xyz = xyz.reshape(-1, 3).contiguous().float()
+        n = xyz.shape[0]
+        dev = xyz.device
+        if n == 0:
+            return (torch.empty((0,), device=dev) if want_sigma else None), torch.empty((0, 3), device=dev)
+    else:
+        _need_cuda(samp, "samp")
+        n, dev = int(n_max), samp.device
+    sigma = torch.empty((n,), device=dev) if want_sigma else None
+    grad = torch.empty((n, 3), device=dev)
+    with TIMER.span("field_density_grad"):
+        check(_lib.lib().jt_field_density_grad(fs.ptrs, fs.dims, geom, _p(xyz), _p(samp), _p(slot), _p(n_dev), n,
+                                               _p(mb), md, mg, float(shift), int(act), int(bool(normals)),
+                                               _p(sigma), _p(grad), _stream()), "jt_field_density_grad")
+    return sigma, grad
+
+
 def alpha_mask_build(alpha_zyx, thres):
     """alpha [D,H,W] -> (vol [D,H,W] float {0,1}, bits int32 words, stats int32[7])."""
     _need_cuda(alpha_zyx, "alpha")

@@ -9,6 +9,8 @@ index, SURVEY.md section 2b):
               tcgen05, MLP_Fea head      jt_app_basis_fwd_tc -> jt_head_mlp_fwd_tc
               strict fp32 (any head)     jt_vm_gather_fwd(app) -> jt_gemm_nt(basis) -> jt_pe_encode / jt_gemm_nt / jt_sh_shade
             -> jt_composite_fwd
+  normals   jt_march_compact -> jt_vm_gather_fwd(density) -> jt_alpha_fwd -> jt_field_density_grad(samples)
+            -> jt_normal_composite   (render_normals: no grad, no appearance stage)
   backward  jt_render_bwd -> jt_ray_init -> head backward (jt_sh_bwd_tc | jt_head_bwd_tc | fp32 GEMM chain)
             -> jt_vm_scatter_rays(app) -> jt_vm_scatter_rays(density)
             (pose-path gradients accumulate inside the scatters; with a gradient synchroniser attached the
@@ -288,6 +290,45 @@ def shade_points(cfg, afs, xyz_norm, viewdirs, basis_w, params):
     count = torch.full((1,), n, device=dev, dtype=torch.int32)
     h = Head(cfg, afs, comp, comp.sidx, viewdirs.contiguous().float(), basis_w, params, count, max(n, 1))
     return h.forward(train=False, basis_grad=False)[:n, :3]
+
+
+def render_normals(cfg, dfs, dfs32, rays_o, rays_d, aux):
+    """Normal map of N rays (no grad): (normal_map [N,3], depth [N], opacity [N]). The samples, the density gather
+    (on `dfs`, the factors forward gathers from) and jt_alpha_fwd run exactly as in VMRender.forward, so depth and
+    opacity are the no-grad forward's bit for bit; jt_field_density_grad then gives every valid sample's unit outward
+    normal from the fp32 factors `dfs32`, and jt_normal_composite sums weight x normal per ray over all valid samples.
+    No appearance stage runs. cfg supplies n_samples, ndc, h_geom, mask, density_shift, act, distance_scale, thres and
+    depth_bias."""
+    lib = _lib.lib()
+    dev = rays_o.device
+    N, S = rays_o.shape[0], cfg.n_samples
+    comp = ops.march_compact(rays_o, rays_d, aux, cfg.ndc, S, cfg.h_geom, cfg.mask)
+    cap = comp.cap
+    sigfeat = torch.empty((cap,), device=dev)
+    ops.vm_gather_fwd(0, dfs, comp.samp, None, comp.count, cap, sigfeat)
+    weight = torch.empty((cap,), device=dev)
+    trans = torch.empty((cap,), device=dev)
+    acc = torch.empty((N,), device=dev)
+    wz = torch.empty((N,), device=dev)
+    app_cnt = torch.empty((N,), device=dev, dtype=torch.int32)
+    app_off = torch.zeros((N + 1,), device=dev, dtype=torch.int32)
+    aidx = torch.empty((1,), device=dev, dtype=torch.int32)       # appearance list capped at one entry: not used here
+    app_of = torch.empty((cap,), device=dev, dtype=torch.int32)
+    with TIMER.span("alpha_fwd"):
+        check(lib.jt_alpha_fwd(_p(comp.ray_off), N, _p(sigfeat), _p(comp.dist), _p(comp.samp),
+                               float(cfg.density_shift), cfg.act, float(cfg.distance_scale), float(cfg.thres),
+                               _p(weight), _p(trans), _p(acc), _p(wz), _p(app_cnt), _p(app_off), _p(aidx),
+                               _p(app_of), 1, None, _stream()), "jt_alpha_fwd")
+    _, nrm = ops.field_density_grad(dfs32, cfg.h_geom, cfg.density_shift, cfg.act, samp=comp.samp, n_dev=comp.count,
+                                    n_max=cap, normals=True, want_sigma=False)
+    normal_map = torch.empty((N, 3), device=dev)
+    depth = torch.empty((N,), device=dev)
+    opacity = torch.empty((N,), device=dev)
+    with TIMER.span("normal_composite"):
+        check(lib.jt_normal_composite(_p(comp.ray_off), N, _p(weight), _p(nrm), _p(acc), _p(wz), _p(rays_d),
+                                      float(cfg.depth_bias), _p(normal_map), _p(depth), _p(opacity), _stream()),
+              "jt_normal_composite")
+    return normal_map, depth, opacity
 
 
 # VMRender.apply's inputs as ctx.needs_input_grad indexes them: cfg, rays_o, rays_d, aux, then these groups

@@ -17,7 +17,7 @@ import torch.nn.functional as F
 from . import _lib, ops
 from ._lib import floats, ints
 from .ops import MAT_MODE, VEC_MODE
-from .render import RenderCfg, VMRender, shade_points, tc_head
+from .render import RenderCfg, VMRender, render_normals, shade_points, tc_head
 
 CL = torch.channels_last
 
@@ -591,6 +591,62 @@ class B200_VMSplit(torch.nn.Module):
                             mask=self.alphaMask)
         return a.view(shape)
 
+    @torch.no_grad()
+    def compute_density_grad(self, xyz_locs):
+        """Density and its gradient at points xyz_locs [..., 3] in the field's input coordinates (world, or NDC for an
+        NDC field): (sigma [...], grad [..., 3]), grad = d sigma / d xyz, the analytic derivative of the field
+        compute_alpha evaluates (jt_field_density_grad). Same field state as compute_alpha: the density factors
+        blurred with the kernel the last forward cached, the fp32 factors whatever factor_storage is, and the alpha
+        mask (rejected points give sigma 0, grad 0). At a cell boundary the derivative is the one-sided one of the
+        cell the tap rounding selects. No autograd; rows are independent of each other."""
+        shape = xyz_locs.shape[:-1]
+        sigma, grad = ops.field_density_grad(self._density_factorset(), self._h_geom(), self.density_shift,
+                                             0 if self.fea2denseAct == "softplus" else 1, xyz=xyz_locs,
+                                             mask=self.alphaMask)
+        return sigma.view(shape), grad.view(*shape, 3)
+
+    @torch.no_grad()
+    def compute_normals(self, xyz_locs):
+        """Unit outward surface normals at points xyz_locs [..., 3]: -grad / |grad| of compute_density_grad's
+        gradient, pointing toward decreasing density; (0, 0, 0) where the gradient is zero (masked points, empty
+        space, points outside the aabb) or not finite. Coordinates as compute_density_grad."""
+        shape = xyz_locs.shape[:-1]
+        _, nrm = ops.field_density_grad(self._density_factorset(), self._h_geom(), self.density_shift,
+                                        0 if self.fea2denseAct == "softplus" else 1, xyz=xyz_locs,
+                                        mask=self.alphaMask, normals=True, want_sigma=False)
+        return nrm.view(*shape, 3)
+
+    @torch.no_grad()
+    def render_normals(self, center, ray_dir, ndc_ray=False, N_samples=-1):
+        """Normal map of rays: (normal_map [N,3], depth [N], opacity [N]). normal_map = sum_k w_k n_k over every
+        valid sample of the ray, w_k the compositing weights (those whose sum is opacity) and n_k compute_normals at
+        the sample (field coordinates: world, or NDC with ndc_ray); it is not renormalised, |normal_map| <= opacity.
+        Samples, alpha mask rule (the mask only without a cached blur, batBase.py:76), blur and factor storage are
+        those of forward(..., is_train=False) with the same module state, so depth and opacity equal that forward's
+        bit for bit. No shading head or appearance stage runs. Each ray's result is independent of the batch."""
+        rays_o = center.reshape(-1, 3).detach().contiguous().float()
+        rays_d = ray_dir.reshape(-1, 3).detach().contiguous().float()
+        ops._need_cuda(rays_o, "center")
+        ops._need_cuda(rays_d, "ray_dir")
+        n = rays_o.shape[0]
+        if n == 0:
+            z = torch.zeros((0,), device=rays_o.device)
+            return torch.zeros((0, 3), device=rays_o.device), z, z.clone()
+        n_samples = N_samples if N_samples > 0 else self.nSamples
+        aux = self._ndc_table(n_samples, False).contiguous() if ndc_ray else None
+        blur_active = self.c2f_mode is not None
+        cfg = RenderCfg(
+            n_samples=int(n_samples), ndc=bool(ndc_ray), h_geom=self._h_geom(),
+            mask=(self.alphaMask if (self.alphaMask is not None and not blur_active) else None),   # batBase.py:76
+            density_shift=float(self.density_shift), act=(0 if self.fea2denseAct == "softplus" else 1),
+            distance_scale=float(self.distance_scale), thres=float(self.rayMarch_weight_thres),
+            depth_bias=-float(self.near_far[0]) + 0.05)
+        dfs = self._density_factorset()
+        gather_fs = dfs
+        if self._checked_storage() == "bf16":      # forward's density gather reads the bf16 copy
+            gather_fs = dfs.with_bf16_store(self._store_cache[0] if not blur_active else None)
+        return render_normals(cfg, gather_fs, dfs, rays_o, rays_d, aux)
+
     # ---------------------------------------------------------------- forward (batBase.py:44-165)
     def forward(self, opt, center, ray_dir, white_bg=True, is_train=False, ndc_ray=False, N_samples=-1,
                 c2f_parameter_density=None, c2f_parameter_color=None, c2f_mode=None, c2f_kernel_size=None,
@@ -735,30 +791,37 @@ class B200_VMSplit(torch.nn.Module):
         return self._dense_alpha_zyx(gridSize).permute(2, 1, 0), dense_xyz
 
     @torch.no_grad()
-    def extract_mesh(self, level=0.005, gridSize=None, colors=False):
+    def extract_mesh(self, level=0.005, gridSize=None, colors=False, normal_source="lattice"):
         """The field's geometry as a triangle mesh: marching cubes (ops.marching_cubes) on the dense alpha grid of
         getDenseAlpha(gridSize) at alpha `level` (0.005 is TensoRF's exporter level). Honours the alpha mask and a
         cached density blur exactly as getDenseAlpha does. Returns (verts [V,3] fp32 world coordinates, faces [F,3]
         int32) on the module's device; normals point out of the high-alpha region.
-        colors=True returns (verts, faces, normals, rgb) with the same verts and faces: normals [V,3] are the unit
-        gradients of the alpha volume the surface was extracted from (ops.marching_cubes(normals=True)), pointing out
-        of the high-alpha region, and rgb [V,3] = compute_rgb(verts, -normals), the colour seen looking at the surface
-        head-on (a vertex with a zero normal is shaded with a zero view direction). For an NDC (LLFF) field the
+        colors=True returns (verts, faces, normals, rgb) with the same verts and faces: normals [V,3] point out of the
+        high-alpha region, and rgb [V,3] = compute_rgb(verts, -normals), the colour seen looking at the surface
+        head-on (a vertex with a zero normal is shaded with a zero view direction). normal_source="lattice" (default):
+        the unit gradients of the alpha volume the surface was extracted from (ops.marching_cubes(normals=True));
+        "field": compute_normals(verts), the field's own density gradient at each vertex. For an NDC (LLFF) field the
         vertices, normals and view directions are all in the field's NDC coordinates."""
+        if normal_source not in ("lattice", "field"):
+            raise _lib.JtError(f"extract_mesh: normal_source {normal_source!r}: expected 'lattice' or 'field'")
         gridSize = self._grid if gridSize is None else [int(v) for v in gridSize]
         mesh = ops.marching_cubes(self._dense_alpha_zyx(gridSize), level, self._dense_tables(gridSize), self._h_aabb,
-                                  normals=colors)
+                                  normals=colors and normal_source == "lattice")
         if not colors:
             return mesh
-        verts, faces, normals = mesh
+        if normal_source == "field":
+            verts, faces = mesh
+            normals = self.compute_normals(verts)
+        else:
+            verts, faces, normals = mesh
         return verts, faces, normals, self.compute_rgb(verts, -normals)
 
-    def export_mesh(self, path, level=0.005, gridSize=None, colors=False):
+    def export_mesh(self, path, level=0.005, gridSize=None, colors=False, normal_source="lattice"):
         """extract_mesh written to `path` as a binary little-endian PLY (float x, y, z per vertex; `list uchar int
         vertex_indices` per face). colors=True adds `float nx, ny, nz` and `uchar red, green, blue` per vertex (the
         names MeshLab, Blender and Open3D read), colours quantised as floor(clamp(rgb, 0, 1) * 255 + 0.5) in fp32.
-        Returns (V, F)."""
-        mesh = self.extract_mesh(level, gridSize, colors=colors)
+        normal_source: as extract_mesh. Returns (V, F)."""
+        mesh = self.extract_mesh(level, gridSize, colors=colors, normal_source=normal_source)
         verts, faces = mesh[0], mesh[1]
         v = verts.cpu().numpy().astype("<f4")
         props = "property float x\nproperty float y\nproperty float z\n"
