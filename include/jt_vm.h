@@ -331,6 +331,24 @@ int jt_field_density_grad(const void* const* h_factors, const int* h_dims, const
                           const float* samp, const int* slot, const int* n_dev, long long n_max,
                           const uint32_t* mask_bits, const int* h_mask_dims, const float* h_mask_geom,
                           float density_shift, int act, int normals, float* sigma, float* grad, cudaStream_t stream);
+/* First hit of each ray on the level set extract_mesh contours. A point p is inside iff point_in_box (the marcher's
+ * aabb test) passes and jt_field_alpha's alpha at p, with `length`, the occupancy mask and the same taps, summation
+ * order and exp, is >= level (fp32). Candidates are the sample depths t_k of the no-grad forward for the same rays
+ * and n_samples: t_min + stepSize * k for metric rays (ztab NULL), ztab[k] for NDC rays; the points are the marcher's
+ * separately rounded o + d t. The hit sample k is the first inside one in ray order. For k > 0 the crossing is
+ * refined in [t_{k-1}, t_k]: each round evaluates the predicate at P equally spaced interior points lo + w j
+ * (w = (hi - lo) / (P + 1), j = 1..P, fp32; P = 15 with 16 channels on every plane, else 7) and keeps the first
+ * inside point as hi and the point before it as lo, until hi - lo <= 2^-20 (t_k - t_{k-1}) or no fp32 value lies
+ * strictly between them. k == 0 (the ray starts inside): no refinement.
+ * Outputs per ray [n_rays]: t = hi (inside; the ray parameter of xyz = o + t d, not the forward's depth_map), +inf on
+ * a miss; xyz [n][3] = the fp32 point whose predicate was evaluated at t, 0 on a miss; k = the hit sample, -1 on a
+ * miss; rounds (may be NULL) = refinement rounds. Each ray's result depends on nothing but the ray. work: one zeroed
+ * device int (rays are handed to warps through it), or NULL (static grid stride; the same results). Factors: fp32
+ * only (JT_ERR_UNSUPPORTED for bf16). 0 < level < 1 and n_samples > 0 are checked. */
+int jt_raycast(const void* const* h_factors, const int* h_dims, const float* h_geom, const uint32_t* mask_bits,
+               const int* h_mask_dims, const float* h_mask_geom, float density_shift, int act, float length,
+               float level, const float* rays_o, const float* rays_d, int n_rays, const float* ztab, int n_samples,
+               int* work, float* t, float* xyz, int* k, int* rounds, cudaStream_t stream);
 /* The rest of updateAlphaMask (tensorBase.py:639-657): clamp(alpha, 0, 1) -> max_pool3d(kernel 5, pad 2, stride 1)
  * -> >= thres, on alpha [D][H][W]. Outputs: vol [D][H][W] floats {0,1} (AlphaGridMask.alpha_volume), bits = the same
  * bit-packed ((W*H*D+31)/32 words, layout of MaskGeom), stats7 = {min_x, max_x, min_y, max_y, min_z, max_z, count}

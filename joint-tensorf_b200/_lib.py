@@ -42,6 +42,7 @@ SIGNATURES = {
     "jt_reg_grads": [_I, _P, _P, _P, _P, _P, _P, _P, _P],
     "jt_field_alpha": [_P, _P, _P, _P, ctypes.c_longlong, _P, _P, _P, _P, _P, _P, _P, _F, _I, _F, _P, _P],
     "jt_field_density_grad": [_P, _P, _P, _P, _P, _P, _P, ctypes.c_longlong, _P, _P, _P, _F, _I, _I, _P, _P, _P],
+    "jt_raycast": [_P, _P, _P, _P, _P, _P, _F, _I, _F, _F, _P, _P, _I, _P, _I, _P, _P, _P, _P, _P, _P],
     "jt_normal_composite": [_P, _I, _P, _P, _P, _P, _P, _F, _P, _P, _P, _P],
     "jt_alpha_mask_build": [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P],
     "jt_resize_bilinear_cl": [_P, _I, _I, _I, _P, _I, _I, _P],

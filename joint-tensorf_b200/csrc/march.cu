@@ -18,52 +18,7 @@
 
 namespace jt {
 
-struct RaySetup {
-    float o[3], d[3];
-    float tmin;      // metric rays only
-    float norm;      // |d| (NDC rays scale dists by it), 1 for metric rays
-};
-
-__device__ __forceinline__ RaySetup load_ray(const float* __restrict__ ro, const float* __restrict__ rd, int r,
-                                             const Geom& g, bool ndc) {
-    RaySetup s;
-#pragma unroll
-    for (int a = 0; a < 3; ++a) { s.o[a] = ro[3 * r + a]; s.d[a] = rd[3 * r + a]; }
-    s.tmin = 0.f;
-    s.norm = 1.f;
-    if (!ndc) {
-        float tm = -INFINITY;
-#pragma unroll
-        for (int a = 0; a < 3; ++a) {
-            float vec = (s.d[a] == 0.0f) ? 1e-6f : s.d[a];
-            float ra = __fdiv_rn(__fsub_rn(g.a1[a], s.o[a]), vec);
-            float rb = __fdiv_rn(__fsub_rn(g.a0[a], s.o[a]), vec);
-            tm = fmaxf(tm, fminf(ra, rb));
-        }
-        s.tmin = fminf(fmaxf(tm, g.near_), g.far_);
-    } else {
-        s.norm = sqrtf(s.d[0] * s.d[0] + s.d[1] * s.d[1] + s.d[2] * s.d[2]);
-    }
-    return s;
-}
-
-// depth of sample k. metric: t_min + stepSize * (k + jitter); NDC: table lookup.
-__device__ __forceinline__ float sample_depth(const RaySetup& s, const Geom& g, int k, float jit,
-                                              const float* __restrict__ ztab, bool ndc) {
-    if (ndc) return ztab[k];
-    float rng = __fadd_rn((float)k, jit);
-    return __fadd_rn(s.tmin, __fmul_rn(g.step, rng));
-}
-
-__device__ __forceinline__ bool point_in_box(const RaySetup& s, const Geom& g, float t, float p[3]) {
-    bool ok = true;
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        p[a] = __fadd_rn(s.o[a], __fmul_rn(s.d[a], t));
-        ok = ok && !((g.a0[a] > p[a]) || (p[a] > g.a1[a]));
-    }
-    return ok;
-}
+// RaySetup, load_ray, sample_depth and point_in_box live in vm_taps.cuh (the ray caster samples the same points).
 
 // ---------------------------------------------------------------- dense variant (API parity)
 __global__ void sample_dense_kernel(const float* __restrict__ ro, const float* __restrict__ rd,

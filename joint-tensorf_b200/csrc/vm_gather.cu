@@ -70,30 +70,7 @@ __global__ void __launch_bounds__(256, 4) vm_fwd_kernel(Factors F, const float4*
 // quads 2h and 2h + 1 (channels 8h .. 8h + 7), so a warp covers 16 samples for about the same setup work, and the
 // offsets are 32-bit (the host checks H W C < 2^31). The sum keeps vm_fwd_kernel's order -- per quad k,
 // a_k = ((0 + dot_0k) + dot_1k) + dot_2k over the planes, then (a_0 + a_1) + (a_2 + a_3) -- so the result is
-// bit-identical to it.
-template <bool B16>
-__device__ __forceinline__ void dens16_plane(const Factors& F, const int i, const float u[3], const int q,
-                                             float& a0, float& a1) {
-    const Tap tx = make_tap(u[mat0(i)], F.W[i]), ty = make_tap(u[mat1(i)], F.H[i]), tl = make_tap(u[vecm(i)], F.L[i]);
-    const unsigned W = (unsigned)F.W[i];
-    const unsigned r0 = (unsigned)ty.i0 * W, r1 = (unsigned)ty.i1 * W;
-    const unsigned o00 = (r0 + tx.i0) * 16u + q, o10 = (r0 + tx.i1) * 16u + q;
-    const unsigned o01 = (r1 + tx.i0) * 16u + q, o11 = (r1 + tx.i1) * 16u + q;
-    const unsigned ol0 = (unsigned)tl.i0 * 16u + q, ol1 = (unsigned)tl.i1 * 16u + q;
-    const float w00 = tx.w0 * ty.w0, w10 = tx.w1 * ty.w0, w01 = tx.w0 * ty.w1, w11 = tx.w1 * ty.w1;
-    const float* P = F.plane[i];
-    const float* Ln = F.line[i];
-    float4 a[2], b[2], c[2], d[2], la[2], lb[2];
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-        a[k] = ld_tap4<B16>(P, o00 + 4 * k); b[k] = ld_tap4<B16>(P, o10 + 4 * k);
-        c[k] = ld_tap4<B16>(P, o01 + 4 * k); d[k] = ld_tap4<B16>(P, o11 + 4 * k);
-        la[k] = ld_tap4<B16>(Ln, ol0 + 4 * k); lb[k] = ld_tap4<B16>(Ln, ol1 + 4 * k);
-    }
-    a0 += f4_dot(f4_bilin(a[0], w00, b[0], w10, c[0], w01, d[0], w11), f4_lerp2(la[0], tl.w0, lb[0], tl.w1));
-    a1 += f4_dot(f4_bilin(a[1], w00, b[1], w10, c[1], w01, d[1], w11), f4_lerp2(la[1], tl.w0, lb[1], tl.w1));
-}
-
+// bit-identical to it. The per-plane step is dens16_plane (vm_taps.cuh).
 template <bool B16>
 __global__ void __launch_bounds__(256, 4) vm_density16_fwd_kernel(Factors F, const float4* __restrict__ samp,
                                                                 const int* __restrict__ slot, const int* __restrict__ n_dev,

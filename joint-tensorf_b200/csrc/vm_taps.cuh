@@ -1,6 +1,7 @@
 // Device helpers shared by the kernels that evaluate the VM field at a point: bilinear / linear tap setup on the
-// channel-last factors (vm_gather.cu, field_maint.cu), the density activation (composite.cu, field_maint.cu) and
-// the occupancy-mask test (march.cu, field_maint.cu).
+// channel-last factors (vm_gather.cu, field_maint.cu, field_grad.cu, raycast.cu), the ray sample points (march.cu,
+// raycast.cu), the density activation (composite.cu, field_maint.cu) and the occupancy-mask test (march.cu,
+// field_maint.cu).
 #pragma once
 #include "jt_common.cuh"
 
@@ -40,6 +41,80 @@ __device__ __forceinline__ PlaneTaps plane_taps(const Factors& F, int i, const f
     t.w00 = t.tx.w0 * t.ty.w0; t.w10 = t.tx.w1 * t.ty.w0;     // nw, ne
     t.w01 = t.tx.w0 * t.ty.w1; t.w11 = t.tx.w1 * t.ty.w1;     // sw, se
     return t;
+}
+
+// One channel-quad pair of a 16-channel plane / line pair i at normalised coordinate u: lane half q (0 or 8) adds
+// quads q/4 and q/4 + 1 of the plane's dot product into a0 and a1, with 32-bit element offsets (the host checks
+// H W 16 < 2^31). The density gather's 2-lanes-per-sample layout (vm_density16_fwd_kernel) and the ray caster's.
+template <bool B16>
+__device__ __forceinline__ void dens16_plane(const Factors& F, const int i, const float u[3], const int q,
+                                             float& a0, float& a1) {
+    const Tap tx = make_tap(u[mat0(i)], F.W[i]), ty = make_tap(u[mat1(i)], F.H[i]), tl = make_tap(u[vecm(i)], F.L[i]);
+    const unsigned W = (unsigned)F.W[i];
+    const unsigned r0 = (unsigned)ty.i0 * W, r1 = (unsigned)ty.i1 * W;
+    const unsigned o00 = (r0 + tx.i0) * 16u + q, o10 = (r0 + tx.i1) * 16u + q;
+    const unsigned o01 = (r1 + tx.i0) * 16u + q, o11 = (r1 + tx.i1) * 16u + q;
+    const unsigned ol0 = (unsigned)tl.i0 * 16u + q, ol1 = (unsigned)tl.i1 * 16u + q;
+    const float w00 = tx.w0 * ty.w0, w10 = tx.w1 * ty.w0, w01 = tx.w0 * ty.w1, w11 = tx.w1 * ty.w1;
+    const float* P = F.plane[i];
+    const float* Ln = F.line[i];
+    float4 a[2], b[2], c[2], d[2], la[2], lb[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+        a[k] = ld_tap4<B16>(P, o00 + 4 * k); b[k] = ld_tap4<B16>(P, o10 + 4 * k);
+        c[k] = ld_tap4<B16>(P, o01 + 4 * k); d[k] = ld_tap4<B16>(P, o11 + 4 * k);
+        la[k] = ld_tap4<B16>(Ln, ol0 + 4 * k); lb[k] = ld_tap4<B16>(Ln, ol1 + 4 * k);
+    }
+    a0 += f4_dot(f4_bilin(a[0], w00, b[0], w10, c[0], w01, d[0], w11), f4_lerp2(la[0], tl.w0, lb[0], tl.w1));
+    a1 += f4_dot(f4_bilin(a[1], w00, b[1], w10, c[1], w01, d[1], w11), f4_lerp2(la[1], tl.w0, lb[1], tl.w1));
+}
+
+// ---- ray sampling (march.cu's marcher and raycast.cu's caster: the same points bit for bit)
+struct RaySetup {
+    float o[3], d[3];
+    float tmin;      // metric rays only
+    float norm;      // |d| (NDC rays scale dists by it), 1 for metric rays
+};
+
+__device__ __forceinline__ RaySetup load_ray(const float* __restrict__ ro, const float* __restrict__ rd, int r,
+                                             const Geom& g, bool ndc) {
+    RaySetup s;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) { s.o[a] = ro[3 * r + a]; s.d[a] = rd[3 * r + a]; }
+    s.tmin = 0.f;
+    s.norm = 1.f;
+    if (!ndc) {
+        float tm = -INFINITY;
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            float vec = (s.d[a] == 0.0f) ? 1e-6f : s.d[a];
+            float ra = __fdiv_rn(__fsub_rn(g.a1[a], s.o[a]), vec);
+            float rb = __fdiv_rn(__fsub_rn(g.a0[a], s.o[a]), vec);
+            tm = fmaxf(tm, fminf(ra, rb));
+        }
+        s.tmin = fminf(fmaxf(tm, g.near_), g.far_);
+    } else {
+        s.norm = sqrtf(s.d[0] * s.d[0] + s.d[1] * s.d[1] + s.d[2] * s.d[2]);
+    }
+    return s;
+}
+
+// depth of sample k. metric: t_min + stepSize * (k + jitter); NDC: table lookup.
+__device__ __forceinline__ float sample_depth(const RaySetup& s, const Geom& g, int k, float jit,
+                                              const float* __restrict__ ztab, bool ndc) {
+    if (ndc) return ztab[k];
+    float rng = __fadd_rn((float)k, jit);
+    return __fadd_rn(s.tmin, __fmul_rn(g.step, rng));
+}
+
+__device__ __forceinline__ bool point_in_box(const RaySetup& s, const Geom& g, float t, float p[3]) {
+    bool ok = true;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        p[a] = __fadd_rn(s.o[a], __fmul_rn(s.d[a], t));
+        ok = ok && !((g.a0[a] > p[a]) || (p[a] > g.a1[a]));
+    }
+    return ok;
 }
 
 // exp(x) for x <= 0 as the reference's alpha = 1 - exp(-sigma*dist) needs it (tensorBase.py:59): for a thin

@@ -565,6 +565,34 @@ def field_density_grad(fs, geom, shift, act, xyz=None, samp=None, slot=None, n_d
     return sigma, grad
 
 
+def raycast(fs, geom, shift, act, length, level, rays_o, rays_d, n_samples, ztab=None, mask=None, rounds=False,
+            counter=True):
+    """First hit of rays_o / rays_d [n,3] on {compute_alpha(p, length) >= level} (jt_raycast, no autograd), on the
+    no-grad forward's sample depths (metric rays, or the NDC depth table ztab [n_samples]) refined to the first
+    crossing -> (t [n] (+inf: miss), xyz [n,3] (0: miss), k [n] int32 hit sample (-1: miss)), plus the refinement
+    rounds per ray [n] int32 with rounds=True. counter=False hands rays to warps by a static grid stride instead of an
+    atomic counter (the same results; for timing the two schedules). fs: FactorSet of the fp32 density factors."""
+    if not 0.0 < float(level) < 1.0:
+        raise _lib.JtError(f"raycast: level {level} must lie in (0, 1)")
+    _need_cuda(rays_o, "rays_o")
+    _need_cuda(rays_d, "rays_d")
+    rays_o = rays_o.reshape(-1, 3).contiguous().float()
+    rays_d = rays_d.reshape(-1, 3).contiguous().float()
+    n, dev = rays_o.shape[0], rays_o.device
+    t = torch.empty((n,), device=dev)
+    xyz = torch.empty((n, 3), device=dev)
+    k = torch.empty((n,), device=dev, dtype=torch.int32)
+    rnd = torch.empty((n,), device=dev, dtype=torch.int32) if rounds else None
+    if n > 0:
+        mb, md, mg = (mask.bits, mask.h_dims, mask.h_geom) if mask is not None else (None, None, None)
+        work = torch.zeros((1,), device=dev, dtype=torch.int32) if counter else None
+        with TIMER.span("raycast"):
+            check(_lib.lib().jt_raycast(fs.ptrs, fs.dims, geom, _p(mb), md, mg, float(shift), int(act), float(length),
+                                        float(level), _p(rays_o), _p(rays_d), n, _p(ztab), int(n_samples), _p(work),
+                                        _p(t), _p(xyz), _p(k), _p(rnd), _stream()), "jt_raycast")
+    return (t, xyz, k, rnd) if rounds else (t, xyz, k)
+
+
 def alpha_mask_build(alpha_zyx, thres):
     """alpha [D,H,W] -> (vol [D,H,W] float {0,1}, bits int32 words, stats int32[7])."""
     _need_cuda(alpha_zyx, "alpha")

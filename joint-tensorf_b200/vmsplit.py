@@ -647,6 +647,32 @@ class B200_VMSplit(torch.nn.Module):
             gather_fs = dfs.with_bf16_store(self._store_cache[0] if not blur_active else None)
         return render_normals(cfg, gather_fs, dfs, rays_o, rays_d, aux)
 
+    @torch.no_grad()
+    def raycast(self, center, ray_dir, level=0.005, ndc_ray=False, N_samples=-1, colors=False):
+        """First hit of each ray on the surface extract_mesh(level) contours, {compute_alpha(p, stepSize) >= level}
+        inside the aabb (jt_raycast): (hit [N] bool, t [N], xyz [N,3], normal [N,3]), plus rgb [N,3] with colors=True.
+        The candidates are the sample depths of forward(..., is_train=False) with the same ndc_ray / N_samples; the
+        first inside sample is refined to the first crossing between it and the sample before it. t is the ray
+        parameter of xyz = center + t * ray_dir (+inf on a miss; not forward's depth_map), xyz the fp32 point known to
+        be inside (0 on a miss). normal = compute_normals(xyz) and rgb = compute_rgb(xyz, viewdir) on the hits, 0 on
+        misses; viewdir is ray_dir as forward's head sees it (normalised for NDC rays, as given otherwise). Same field
+        state as compute_alpha: the density factors blurred with the kernel the last forward cached, the fp32 factors
+        whatever factor_storage is, and the alpha mask. Each ray's result is independent of the batch."""
+        rays_o = center.reshape(-1, 3).detach().contiguous().float()
+        rays_d = ray_dir.reshape(-1, 3).detach().contiguous().float()
+        n_samples = N_samples if N_samples > 0 else self.nSamples
+        ztab = self._ndc_table(n_samples, False).contiguous() if ndc_ray else None
+        t, xyz, _ = ops.raycast(self._density_factorset(), self._h_geom(), self.density_shift,
+                                0 if self.fea2denseAct == "softplus" else 1, float(self._h_step), level, rays_o,
+                                rays_d, n_samples, ztab=ztab, mask=self.alphaMask)
+        hit = torch.isfinite(t)
+        # rows are independent in both point queries: evaluate every row (no host sync), keep the hits' rows
+        normal = torch.where(hit[:, None], self.compute_normals(xyz), 0.0)
+        if not colors:
+            return hit, t, xyz, normal
+        dirs = rays_d / torch.linalg.vector_norm(rays_d, dim=-1, keepdim=True) if ndc_ray else rays_d
+        return hit, t, xyz, normal, torch.where(hit[:, None], self.compute_rgb(xyz, dirs), 0.0)
+
     # ---------------------------------------------------------------- forward (batBase.py:44-165)
     def forward(self, opt, center, ray_dir, white_bg=True, is_train=False, ndc_ray=False, N_samples=-1,
                 c2f_parameter_density=None, c2f_parameter_color=None, c2f_mode=None, c2f_kernel_size=None,
